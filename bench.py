@@ -3,6 +3,7 @@
 
   python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
   python bench.py --impl reference [--gpus N] ...                # the reference algorithm on host cores
+  python bench.py ... --dump-outputs DIR                         # also save the last timed frame as DIR/framebuffer.npy
 
 Workload (config.workload): the 1 002 528-triangle displaced sphere of BASELINE config 5 (the scene
 the north star's 70 % target is quoted on) seen by the config-2 camera, traced with config 4's ray
@@ -42,6 +43,7 @@ for _p in (ROOT, os.path.join(ROOT, "bih-gpu-raytracer_b200")):
 METRIC = "Mrays/s"
 L2_FLUSH_BYTES = 256 << 20          # > 126 MB L2
 NODE_BYTES = 64                     # one node record: the BIH pair of clip planes + child references (16 B) and the two children boxes (48 B)
+DUMP_BYTES = 64 << 20               # --dump-outputs: at most this much in all
 
 
 def log(*a):
@@ -106,6 +108,27 @@ def ncu_counters(workload_key):
         return e
     except Exception as ex:       # noqa
         return {"stale": "no capture: %r" % (ex,)}
+
+
+def dump_outputs(path, **arrays):
+    """--dump-outputs: the arrays the timed path returned in its last step, one <path>/<name>.npy each, so that two
+    builds of the project can be compared output for output.  Values are stored as float32 (the framebuffer's packed
+    r | g<<8 | b<<16 pixels are below 2**24 and therefore exact).  The files take at most DUMP_BYTES in all: each array
+    gets an equal share, and one larger than its share is replaced by a fixed, seeded sample of its elements,
+    <name>_sample.npy, with their flat indices in <name>_sample_index.npy."""
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays) - 2 * 4096          # (room for the .npy headers)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        assert np.all(np.asarray(a, np.float32) == a), name + " is not exact in float32"
+        a = a.astype(np.float32)
+        if a.nbytes <= share:
+            np.save(os.path.join(path, name + ".npy"), a)
+            continue
+        idx = np.sort(np.random.default_rng(1984).choice(a.size, share // 12, replace=False))
+        np.save(os.path.join(path, name + "_sample.npy"), a.ravel()[idx])
+        np.save(os.path.join(path, name + "_sample_index.npy"), idx.astype(np.float64))
+    log("outputs of the last timed step written to %s: %s" % (path, ", ".join(sorted(os.listdir(path)))))
 
 
 def oracle_tile_check(fb, tri_or_bih, cam, W, H, spp, tiles=12, seed=1984):
@@ -398,6 +421,8 @@ def run_ours(args, rank, world, local_rank):
     if rank == 0:
         frame = frame_from_device(0)
         frame_crc = crc32(frame)
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, framebuffer=frame)
         try:
             tile_check = oracle_tile_check(frame, tri, cam, W, H, spp)
         except Exception as ex:       # noqa
@@ -970,7 +995,13 @@ def main():
     ap.add_argument("--spp", type=int, default=16)
     ap.add_argument("--no-extras", action="store_true")
     ap.add_argument("--no-config4", action="store_true", help="N > 1: skip the 10 M-triangle config-4 section")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the framebuffer of the last timed step to DIR/framebuffer.npy (float32, packed r | g<<8 | b<<16)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs applies to --impl b200")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

@@ -8,9 +8,8 @@
 //   __device__ TraverseTree     R/src/CUDAKernels.cu:227-368   (through a 10-line wrapper kernel)
 // and restates only the five thrust calls of Renderer::Render (R/src/Renderer.cpp:422-472) and the
 // sentinel initialisation of GPUArrayManager::AllocateBIHTree (R/src/GPUArrayManager.cpp:58-91), which
-// live in translation units that need a GL context.  Built by oracle/Makefile into oracle/_ref/ (git-
-// ignored, travels to the GPU box); used by tests/test_gpu_reference_kernels.py to pin the CPU oracle
-// against the real reference, and by bench.py --impl refcuda as the "reference kernels on B200" baseline.
+// live in translation units that need a GL context.  Built by `make -C oracle ref REF=<reference src dir>`
+// into oracle/_ref/ (git-ignored); bench.py reports it as the "reference kernels on B200" baseline.
 #define STR2(x) #x
 #define STR(x) STR2(x)
 #include STR(REF_SRC_DIR/CUDAKernels.cu)
