@@ -28,7 +28,8 @@
 //
 // Logical per-ray algorithm = oracle/bih_oracle.c:traverse_box (pruned traversal + children boxes that returns what
 // the reference's TraverseTree returns, including on axis-aligned flat geometry where the reference's
-// strict comparisons decide).  Everything that decides a hit is IEEE binary32 without FMA contraction (explicit __f*_rn)
+// strict comparisons decide); framebuffer renders (MODE 1) end a sample at its first accepted triangle, which
+// tests/coverage_oracle.c restates as mode "first" (TRACE_COVERAGE_EXIT below).  Everything that decides a hit is IEEE binary32 without FMA contraction (explicit __f*_rn)
 // so t is bit-identical to the oracle's; the box distances are explicit FMAs, mirrored with fmaf in the oracle.
 #include "bihrt_internal.cuh"
 #include <float.h>
@@ -73,6 +74,16 @@
 #ifndef TRACE_LDG256
 #define TRACE_LDG256 1
 #endif
+// Framebuffer renders (MODE 1) as coverage queries: a pixel's colour depends only on WHETHER each sample hits, so a sample
+// ends at the first triangle it accepts -- inside the leaf and for the whole walk -- instead of searching on for the
+// closest one.  Until that first hit the walk is the closest-hit walk step for step (h.t is FLT_MAX in both: same strict
+// test, same far-leaf-first order, same flat-geometry misses), so a sample hits exactly when the closest-hit search hits and
+// the image is the same bit for bit.  While a sample is alive every stacked item is still valid (pMin <= pMax <= FLT_MAX
+// held when it was pushed), so the pop needs no compare-and-drop loop.  MODE 0 and 2 keep the closest hit.
+// 1 = on; 0 = every mode searches for the closest hit (A/B builds: make variant EXTRA="-DTRACE_COVERAGE_EXIT=0").
+#ifndef TRACE_COVERAGE_EXIT
+#define TRACE_COVERAGE_EXIT 1
+#endif
 #define TOP_FLAG 0x40000000u
 #define BOX_EPS 2.384185791015625e-07f      /* 2^-22: the box tests' margin is this times (largest finite |o/d| + larger end of the ray's scene interval), one constant per ray */
 
@@ -95,7 +106,8 @@ __device__ __forceinline__ uint32_t pack_colour(uint32_t hits, int samples) {
     return ((uint32_t)(int)cb << 16) | ((uint32_t)(int)cr << 8) | (uint32_t)(int)cr;
 }
 
-template <bool COUNTED>
+// FIRST: stop at the first accepted triangle (coverage queries)
+template <bool COUNTED, bool FIRST>
 __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, float ox, float oy, float oz,
                                           float dx, float dy, float dz, Hit& h, uint32_t& ntris, uint32_t& wleaf) {
     const float4* p = reinterpret_cast<const float4*>(first_tri);
@@ -119,7 +131,10 @@ __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, fl
                 const float v = __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(dx, qx), __fmul_rn(dy, qy)), __fmul_rn(dz, qz)), inv);
                 if (!(v < 0.f || __fadd_rn(u, v) > 1.f)) {
                     const float t = __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(e2x, qx), __fmul_rn(e2y, qy)), __fmul_rn(e2z, qz)), inv);
-                    if (t > 0.f && t < h.t) { h.t = t; h.slot = (int)__float_as_uint(q2.w); }   // :218-221, slot = sorted index
+                    if (t > 0.f && t < h.t) {                                                   // :218-221, slot = sorted index
+                        h.t = t; h.slot = (int)__float_as_uint(q2.w);
+                        if (FIRST) break;
+                    }
                 }
             }
         }
@@ -140,6 +155,7 @@ __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, fl
 template <int MODE, bool COUNTED, int WALK, bool Q>
 __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(TraceArgs a) {
     constexpr int STACK_DEPTH = Q ? STACK_DEPTH_QUALITY : STACK_DEPTH_PARITY;
+    constexpr bool COVER = MODE == 1 && TRACE_COVERAGE_EXIT != 0;     // a sample ends at its first hit
     // per-axis ray constants (origin, 1/dir), one row of 3 float2 per thread: 24-byte stride keeps a
     // half-warp's 64-bit accesses on distinct banks when the lanes agree on the axis
     // per-thread ray record in shared memory, 10 words: (ox, 1/dx) (oy, 1/dy) (oz, 1/dz) dx dy dz -.  The node step picks
@@ -449,7 +465,8 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                     // plane logic of the BIH proper keeps the reference's infinity (it reads 1 / d from shared memory).
                     const float qnan = __uint_as_float(0x7fc00000u);
                     ix = fabsf(ix) <= FLT_MAX ? ix : qnan; iy = fabsf(iy) <= FLT_MAX ? iy : qnan; iz = fabsf(iz) <= FLT_MAX ? iz : qnan;
-                    rMin = tMin; pMin = fmaxf(tMin, 0.f); pMax = (MODE == 0 && a.any_hit) ? fminf(tMax, h.t) : tMax;
+                    // (coverage: cut at h.t = FLT_MAX too, so that every item's pMax is finite and never needs the pop's check)
+                    rMin = tMin; pMin = fmaxf(tMin, 0.f); pMax = ((MODE == 0 && a.any_hit) || COVER) ? fminf(tMax, h.t) : tMax;
                     // Nu == 1: no internal node; the single leaf starts at slot 0 (and must not be
                     // interval-pruned: the reference tests it unconditionally once the box is hit)
                     if (nu == 1) { cur = BIH_REF_LEAFREF(0); pMin = -FLT_MAX; pMax = FLT_MAX; }
@@ -487,7 +504,13 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
 #define POP_VALID()                                                                                         \
         do {                                                                                                \
             cur = NONE;                                                                                     \
-            while (sp > 0) {                                                                                \
+            if (COVER) {                       /* h.t is still FLT_MAX: the top item is valid */            \
+                if (sp > 0) {                                                                               \
+                    uint4 e;                                                                                \
+                    STACK_POP(e);                                                                           \
+                    cur = e.x; rMin = __uint_as_float(e.y); pMin = __uint_as_float(e.z); pMax = __uint_as_float(e.w); \
+                }                                                                                           \
+            } else while (sp > 0) {                                                                         \
                 uint4 e;                                                                                    \
                 STACK_POP(e);                                                                               \
                 const float m = fminf(__uint_as_float(e.w), h.t);                                           \
@@ -581,8 +604,9 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
             const char* tp;
             asm("mad.wide.u32 %0, %1, 12, %2;" : "=l"(tp) : "r"(cur & 0x7FFFFFFCu), "l"(tris_b));
             const float2 dxy = *reinterpret_cast<const float2*>(my_ray + 6);
-            test_leaf<COUNTED>(tp, my_ray[0], my_ray[2], my_ray[4], dxy.x, dxy.y, my_ray[8], h, ntris, wleaf);
-            if (MODE == 0 && a.any_hit && h.slot >= 0) { STACK_RESET(); cur = NONE; }      // occluded: nothing else to learn
+            test_leaf<COUNTED, COVER>(tp, my_ray[0], my_ray[2], my_ray[4], dxy.x, dxy.y, my_ray[8], h, ntris, wleaf);
+            // occluded / covered: nothing else to learn
+            if (((MODE == 0 && a.any_hit) || COVER) && h.slot >= 0) { STACK_RESET(); cur = NONE; }
             else POP_VALID();
         }
 #undef POP_VALID
