@@ -60,11 +60,38 @@ class BuildInfo(C.Structure):
                 ("last_build_ms", C.c_float), ("sort_passes", C.c_int32), ("reserved", C.c_int32 * 6)]
 
 
+class Hits(C.Structure):
+    """bihrt_hits: where bihrt_intersect writes each part of the hit record (NULL = not wanted)."""
+    _fields_ = [("t", C.c_void_p), ("u", C.c_void_p), ("v", C.c_void_p), ("slot", C.c_void_p), ("prim", C.c_void_p),
+                ("ng", C.c_void_p)]
+
+
+INTERSECT_ANY = 1
+HIT_OUTPUTS = ("t", "u", "v", "slot", "prim", "ng")
+
+
+def interval_rays(rays6, tmin=0.0, tmax=np.inf):
+    """(N,8) float32 rays o.xyz tmin d.xyz tmax for Renderer.intersect, from (N,6) rays o.xyz d.xyz and a scalar or per-ray
+    (N,) tmin / tmax.  numpy in -> numpy out; torch in -> torch out on the same device."""
+    if isinstance(rays6, np.ndarray):
+        r = np.asarray(rays6, np.float32).reshape(-1, 6)
+        out = np.empty((r.shape[0], 8), np.float32)
+    else:
+        import torch
+        r = rays6.reshape(-1, 6).to(torch.float32)
+        out = torch.empty((r.shape[0], 8), dtype=torch.float32, device=r.device)
+    out[:, 0:3] = r[:, 0:3]
+    out[:, 4:7] = r[:, 3:6]
+    out[:, 3] = tmin
+    out[:, 7] = tmax
+    return out
+
+
 # every symbol include/bihrt.h declares (tests check that the library exports all of them)
 ABI_SYMBOLS = [
     "bihrt_version", "bihrt_create", "bihrt_destroy", "bihrt_last_error", "bihrt_set_stream", "bihrt_get_stream", "bihrt_sync",
     "bihrt_set_option", "bihrt_get_stat", "bihrt_scene_load_triangles", "bihrt_scene_update_vertices", "bihrt_scene_load_obj",
-    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_trace_counted",
+    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_trace_counted",
     "bihrt_render", "bihrt_render_counted", "bihrt_render_shard", "bihrt_render_samples", "bihrt_render_interleaved", "bihrt_render_interleaved_to", "bihrt_framebuffer_ipc_export", "bihrt_framebuffer_ipc_open", "bihrt_framebuffer_ipc_close", "bihrt_framebuffer_ipc_unexport", "bihrt_bih_region", "bihrt_bih_adopt", "bihrt_bih_copy", "bihrt_framebuffer_resolve", "bihrt_render_hits", "bihrt_secondary_rays", "bihrt_framebuffer", "bihrt_framebuffer_read",
     "bihrt_bih_blob_bytes", "bihrt_bih_export", "bihrt_bih_import",
     "bihrt_create_multi", "bihrt_destroy_multi", "bihrt_multi_size", "bihrt_multi_nccl_version", "bihrt_multi_broadcast",
@@ -304,6 +331,36 @@ class Renderer:
         if on_dev:
             self.torch_wait()
         return blocker
+
+    def intersect(self, rays8, any_hit=False, outputs=HIT_OUTPUTS):
+        """Ray queries with per-ray intervals (bihrt_intersect).  rays8: (N,8) float32 o.xyz tmin d.xyz tmax (numpy or torch,
+        host or device; interval_rays builds it).  A triangle counts when max(tmin,0) < t < min(tmax,FLT_MAX); any_hit ends a
+        ray at the first one (occlusion).  Returns {name: array} for the requested outputs of
+        t (N,), u (N,), v (N,), slot (N,), prim (N,), ng (N,3): numpy for numpy input, torch tensors on the rays' device for
+        torch input.  A miss reads t = FLT_MAX, slot = prim = -1, u = v = ng = 0."""
+        unknown = set(outputs) - set(HIT_OUTPUTS)
+        if unknown:
+            raise ValueError("unknown outputs %s (known: %s)" % (sorted(unknown), ", ".join(HIT_OUTPUTS)))
+        shapes = {"t": (), "u": (), "v": (), "slot": (), "prim": (), "ng": (3,)}
+        if isinstance(rays8, np.ndarray):
+            rays8 = np.ascontiguousarray(rays8, dtype=np.float32)
+            n = rays8.size // 8
+            res = {k: np.empty((n,) + shapes[k], np.int32 if k in ("slot", "prim") else np.float32) for k in outputs}
+        else:
+            import torch
+            rays8 = rays8.contiguous()
+            n = rays8.numel() // 8
+            res = {k: torch.empty((n,) + shapes[k], dtype=torch.int32 if k in ("slot", "prim") else torch.float32, device=rays8.device)
+                   for k in outputs}
+        hits = Hits(**{k: _ptr(res[k]) for k in res})
+        on_dev = getattr(rays8, "is_cuda", False)
+        if on_dev:
+            self.wait_torch()            # rays (and recycled output blocks) were last touched on torch's current stream
+        self._check(self._lib.bihrt_intersect(self._ctx, _ptr(rays8), C.c_int64(n), C.c_uint32(INTERSECT_ANY if any_hit else 0),
+                                              C.byref(hits)))
+        if on_dev:
+            self.torch_wait()            # device outputs are written asynchronously on the context's stream
+        return res
 
     def render(self, camera, w, h, spp=1, seed=1984, jitter=False, shard=(0, 1)):
         cam = camera if isinstance(camera, Camera) else Camera.from_array(camera)

@@ -505,34 +505,50 @@ static void base_args(bihrt_ctx* c, TraceArgs& a) {
     a.queues = c->opt_sm_queues;      // resolved per launch in bihrt_trace_launch (-1 = by ray count)
 }
 
-// outputs may individually be host or device; host ones are staged through d_io
-struct OutStage { float* t; int32_t* slot; int32_t* prim; float* ht; int32_t* hslot; int32_t* hprim; };
+// outputs may individually be host or device; host ones are staged through d_io.  t, slot, prim (4 bytes per ray) for every
+// trace; u, v (4 bytes) and ng (12 bytes) for bihrt_intersect's hit records.  dev[k] is what the kernel writes (the caller's
+// device array, a staging block, or NULL), host[k] the caller's host array it is copied back to (NULL: none).
+enum { OUT_T, OUT_SLOT, OUT_PRIM, OUT_U, OUT_V, OUT_NG, OUT_COUNT };
+static const size_t out_bytes_per_ray[OUT_COUNT] = { 4, 4, 4, 4, 4, 12 };
+struct OutStage {
+    void* dev[OUT_COUNT]; void* host[OUT_COUNT];
+    float* t() const { return (float*)dev[OUT_T]; }
+    int32_t* slot() const { return (int32_t*)dev[OUT_SLOT]; }
+    int32_t* prim() const { return (int32_t*)dev[OUT_PRIM]; }
+};
 
-static int stage_outputs(bihrt_ctx* c, int64_t n, size_t front_bytes, float* t, int32_t* slot, int32_t* prim, OutStage& o, uint8_t** front) {
-    const bool dt = t && !is_device_ptr(t), ds = slot && !is_device_ptr(slot), dp = prim && !is_device_ptr(prim);
-    size_t need = front_bytes + ((dt ? 1 : 0) + (ds ? 1 : 0) + (dp ? 1 : 0)) * (size_t)n * 4 + 256;
+static int stage_outputs(bihrt_ctx* c, int64_t n, size_t front_bytes, float* t, int32_t* slot, int32_t* prim, OutStage& o, uint8_t** front,
+                         float* u = nullptr, float* v = nullptr, float* ng = nullptr) {
+    void* const want[OUT_COUNT] = { t, slot, prim, u, v, ng };
+    bool staged[OUT_COUNT];
+    size_t need = front_bytes + 256;
+    for (int k = 0; k < OUT_COUNT; k++) {
+        staged[k] = want[k] && !is_device_ptr(want[k]);
+        if (staged[k]) need += (size_t)n * out_bytes_per_ray[k] + 16;    // (+16: every staged array starts 16-byte aligned)
+    }
     int rc = ensure_io(c, need);
     if (rc) return rc;
     uint8_t* p = (uint8_t*)c->d_io;
     *front = p;
     p += (front_bytes + 255) / 256 * 256;
-    o = OutStage{ t, slot, prim, nullptr, nullptr, nullptr };
-    if (dt) { o.ht = t; o.t = (float*)p; p += (size_t)n * 4; }
-    if (ds) { o.hslot = slot; o.slot = (int32_t*)p; p += (size_t)n * 4; }
-    if (dp) { o.hprim = prim; o.prim = (int32_t*)p; p += (size_t)n * 4; }
+    for (int k = 0; k < OUT_COUNT; k++) {
+        o.dev[k] = want[k]; o.host[k] = nullptr;
+        if (staged[k]) { o.host[k] = want[k]; o.dev[k] = p; p += ((size_t)n * out_bytes_per_ray[k] + 15) / 16 * 16; }
+    }
     return BIHRT_OK;
 }
 
 static int unstage_outputs(bihrt_ctx* c, int64_t n, const OutStage& o) {
-    if (!o.ht && !o.hslot && !o.hprim) return BIHRT_OK;
+    bool any = false;
+    for (int k = 0; k < OUT_COUNT; k++) any |= o.host[k] != nullptr;
+    if (!any) return BIHRT_OK;
     // host outputs: the call is synchronous anyway -- learn first whether the BIH that was traced is valid (a tripped
     // build watchdog makes the kernel trace nothing), and leave the caller's arrays untouched if it is not
     BIHRT_CUDA(c, cudaStreamSynchronize(c->stream));
     int rc = check_status(c);
     if (rc) return rc;
-    if (o.ht) BIHRT_CUDA(c, cudaMemcpyAsync(o.ht, o.t, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-    if (o.hslot) BIHRT_CUDA(c, cudaMemcpyAsync(o.hslot, o.slot, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
-    if (o.hprim) BIHRT_CUDA(c, cudaMemcpyAsync(o.hprim, o.prim, (size_t)n * 4, cudaMemcpyDeviceToHost, c->stream));
+    for (int k = 0; k < OUT_COUNT; k++)
+        if (o.host[k]) BIHRT_CUDA(c, cudaMemcpyAsync(o.host[k], o.dev[k], (size_t)n * out_bytes_per_ray[k], cudaMemcpyDeviceToHost, c->stream));
     BIHRT_CUDA(c, cudaStreamSynchronize(c->stream));
     return BIHRT_OK;
 }
@@ -553,7 +569,7 @@ static int trace_impl(bihrt_ctx* c, const bihrt_ray* rays, int64_t n, float* t, 
         TraceArgs a; base_args(c, a);
         if (rays_dev) a.rays = rays;
         else { BIHRT_CUDA(c, cudaMemcpyAsync(front, rays, (size_t)n * sizeof(bihrt_ray), cudaMemcpyHostToDevice, c->stream)); a.rays = (const bihrt_ray*)front; }
-        a.nrays = n; a.out_t = o.t; a.out_slot = o.slot; a.out_prim = o.prim;
+        a.nrays = n; a.out_t = o.t(); a.out_slot = o.slot(); a.out_prim = o.prim();
         a.any_hit = any_hit ? 1 : 0; a.tmax = tmax;
         // incoherent batches (option trace_sort_rays): trace through a permutation that groups the rays by origin cell and
         // direction octant; results still land in list order
@@ -585,6 +601,35 @@ int bihrt_trace_any(bihrt_ctx* c, const bihrt_ray* rays, int64_t n, float tmax, 
     if (!c) return BIHRT_ERR_INVALID;
     if (!(tmax > 0.f)) return bihrt_fail(c, BIHRT_ERR_INVALID, "tmax must be positive");
     return trace_impl(c, rays, n, nullptr, blocker, nullptr, nullptr, true, tmax);
+}
+
+// Ray queries with per-ray intervals and hit records (include/bihrt.h): k_trace MODE 3.
+int bihrt_intersect(bihrt_ctx* c, const bihrt_ray_interval* rays, int64_t n, uint32_t flags, const bihrt_hits* out) {
+    ENTER(c);
+    if (flags & ~BIHRT_INTERSECT_ANY) return bihrt_fail(c, BIHRT_ERR_INVALID, "unknown flags 0x%x", flags & ~BIHRT_INTERSECT_ANY);
+    if (!out) return bihrt_fail(c, BIHRT_ERR_INVALID, "no output record");
+    if (n < 0 || (n > 0 && !rays)) return bihrt_fail(c, BIHRT_ERR_INVALID, "bad ray array");
+    if (n >= (1ll << 32) - (1ll << 24)) return bihrt_fail(c, BIHRT_ERR_INVALID, "too many rays in one call (32-bit work counter)");
+    if (!c->built) return bihrt_fail(c, BIHRT_ERR_STATE, "BIH not built");
+    { int st = check_status(c); if (st) return st; }
+    if (n == 0) return BIHRT_OK;
+    const bool rays_dev = is_device_ptr(rays);
+    if (rays_dev && ((uintptr_t)rays & 15u)) return bihrt_fail(c, BIHRT_ERR_INVALID, "device rays must be 16-byte aligned (two 128-bit loads per ray)");
+    OutStage o; uint8_t* front;
+    int rc = stage_outputs(c, n, rays_dev ? 0 : (size_t)n * sizeof(bihrt_ray_interval), out->t, out->slot, out->prim, o, &front,
+                           out->u, out->v, out->ng);
+    if (rc) return rc;
+    TraceArgs a; base_args(c, a);
+    if (rays_dev) a.rays_iv = rays;
+    else {
+        BIHRT_CUDA(c, cudaMemcpyAsync(front, rays, (size_t)n * sizeof(bihrt_ray_interval), cudaMemcpyHostToDevice, c->stream));
+        a.rays_iv = (const bihrt_ray_interval*)front;
+    }
+    a.nrays = n; a.any_hit = (flags & BIHRT_INTERSECT_ANY) ? 1 : 0;
+    a.out_t = o.t(); a.out_slot = o.slot(); a.out_prim = o.prim();
+    a.out_u = (float*)o.dev[OUT_U]; a.out_v = (float*)o.dev[OUT_V]; a.out_ng = (float*)o.dev[OUT_NG];
+    if ((rc = bihrt_trace_launch(c, a, 3, false))) return rc;
+    return unstage_outputs(c, n, o);
 }
 
 static int render_check(bihrt_ctx* c, const bihrt_camera* cam, int w, int h, int spp, int si, int sc) {
@@ -783,7 +828,7 @@ int bihrt_render_hits(bihrt_ctx* c, const bihrt_camera* cam, int32_t w, int32_t 
     TraceArgs a; base_args(c, a);
     a.cam = *cam; a.w = w; a.h = h; a.spp = spp; a.seed = seed; a.flags = flags;
     a.s_begin = 0; a.s_end = spp; a.gshift = fit_gshift(w, h, 1, pick_gshift(c, spp));
-    a.out_t = o.t; a.out_slot = o.slot; a.out_prim = o.prim;
+    a.out_t = o.t(); a.out_slot = o.slot(); a.out_prim = o.prim();
     if ((rc = bihrt_trace_launch(c, a, 2, false))) return rc;
     return unstage_outputs(c, n, o);
 }

@@ -154,6 +154,45 @@ BIHRT_API int bihrt_trace(bihrt_ctx* ctx, const bihrt_ray* rays, int64_t n, floa
  * hit bihrt_trace reports has t < tmax; which blocker is found is unspecified.  With the shadow rays of
  * bihrt_secondary_rays (direction = light - origin) tmax = 1 asks "is the light hidden". */
 BIHRT_API int bihrt_trace_any(bihrt_ctx* ctx, const bihrt_ray* rays, int64_t n, float tmax, int32_t* blocker);
+/* ---- ray queries: rays with their own parametric interval, full hit records.
+ *      A triangle is ACCEPTED when max(tmin, 0) < t < min(tmax, FLT_MAX), both comparisons strict (like bihrt_trace's
+ *      0 < t < best): a negative tmin acts as 0, a tmax of FLT_MAX or more (+inf included) as FLT_MAX.  A ray with
+ *      !(max(tmin, 0) < tmax) -- a NaN in either bound included -- misses without being traced.
+ *      flags 0 (closest hit): the accepted triangle with the smallest t that bihrt_trace's walk reaches.  The walk is
+ *        bihrt_trace's (the reference's strict plane test with the scene-box entry, far-leaf-first order, and its misses on
+ *        axis-aligned flat geometry); the interval only narrows it.  So with tmin = 0 and tmax >= FLT_MAX, t / slot / prim
+ *        are bihrt_trace's bit for bit, and with tmin = 0 a ray hits exactly when bihrt_trace's t < tmax, with the same
+ *        triangle.  Peeling (next query with tmin = the last t) visits a ray's distinct hit distances front to back.
+ *      BIHRT_INTERSECT_ANY (occlusion): the walk ends with the leaf in which a triangle is first accepted.  A ray hits exactly when the
+ *        closest-hit query with the same interval hits; the record describes the triangle found (which one: unspecified).
+ *      Record per ray (every output pointer of bihrt_hits may be NULL; each one host or device):
+ *        t     Moller-Trumbore t, bit-identical to what bihrt_trace reports for that triangle;
+ *        u, v  the reference's Moller-Trumbore u, v (R/src/CUDAKernels.cu:35,42, same IEEE binary32 operations): the hit
+ *              point is ~ (1-u-v) v0 + u v1 + v v2 in the triangle's input vertex order;
+ *        slot, prim  as bihrt_trace;
+ *        ng    geometric normal e1 x e2, e1 = v1 - v0, e2 = v2 - v0, NOT normalised, binary32 with every product rounded and
+ *              no FMA: (e1y*e2z - e1z*e2y, e1z*e2x - e1x*e2z, e1x*e2y - e1y*e2x), 3 floats per ray.  Hits are front faces
+ *              only (det >= 1e-6, as in the reference), so dot(d, ng) < 0.
+ *        miss: t = FLT_MAX, slot = prim = -1, u = v = 0, ng = (0, 0, 0).
+ *      Quality-mode trees (morton_bits 63): same contract without the reference's quirks; hits equal brute force over the
+ *      interval.  The option trace_sort_rays does not apply (rays are traced in list order).  rays: host or device; device
+ *      rays must be 16-byte aligned (a ray is read as two 128-bit loads).  Host outputs: the call synchronises and leaves them
+ *      untouched if the build's watchdog tripped; device outputs are written asynchronously on the context's stream.
+ *      Errors: BIHRT_ERR_INVALID for unknown flag bits, rays == NULL with n > 0, out == NULL, n < 0, n >= 2^32 - 2^24 or
+ *      misaligned device rays; BIHRT_ERR_STATE without a built BIH. ------------------------------------------------------ */
+/* ray with its own parametric interval: 32 B, two 128-bit loads */
+typedef struct bihrt_ray_interval { float o[3]; float tmin; float d[3]; float tmax; } bihrt_ray_interval;
+/* outputs of bihrt_intersect: any pointer may be NULL; each one host or device */
+typedef struct bihrt_hits {
+    float*   t;     /* [n] */
+    float*   u;     /* [n] barycentric weight of v1 */
+    float*   v;     /* [n] barycentric weight of v2 */
+    int32_t* slot;  /* [n] */
+    int32_t* prim;  /* [n] */
+    float*   ng;    /* [3n] geometric normal, xyz per ray */
+} bihrt_hits;
+#define BIHRT_INTERSECT_ANY 1u   /* occlusion: end at the first accepted triangle of the interval */
+BIHRT_API int bihrt_intersect(bihrt_ctx* ctx, const bihrt_ray_interval* rays, int64_t n, uint32_t flags, const bihrt_hits* out);
 /* instrumented trace: counters[0]=internal nodes visited, [1]=triangle tests, [2]=max stack depth,
  * [3]=rays; same results as bihrt_trace (outputs may be NULL). */
 BIHRT_API int bihrt_trace_counted(bihrt_ctx* ctx, const bihrt_ray* rays, int64_t n, float* t, int32_t* slot,
