@@ -68,7 +68,7 @@ static int ensure_capacity(bihrt_ctx* c, int64_t n, bool with_build_scratch) {
         c->blob_cap = blob_capacity(cap);
         dev_free(&c->d_tri_in);
         for (int i = 0; i < 2; i++) { dev_free(&c->d_keys[i]); dev_free(&c->d_vals[i]); }
-        dev_free(&c->d_umc); dev_free(&c->d_first); dev_free(&c->d_lookback); dev_free(&c->d_heaps); dev_free(&c->d_xctl); dev_free(&c->d_xbox);
+        dev_free(&c->d_umc); dev_free(&c->d_first); dev_free(&c->d_lookback); dev_free(&c->d_heaps);
         dev_free(&c->d_keys64[0]); dev_free(&c->d_keys64[1]); dev_free(&c->d_lookback_q); c->lookback_q_words = 0;
         c->cap_n = cap;
         c->have_scene = false; c->built = false;
@@ -136,9 +136,9 @@ void bihrt_destroy(bihrt_ctx* c) {
     dev_free(&c->d_tri_in); dev_free(&c->d_blob);
     for (int i = 0; i < 2; i++) { dev_free(&c->d_keys[i]); dev_free(&c->d_vals[i]); }
     dev_free(&c->d_umc); dev_free(&c->d_first); dev_free(&c->d_hist); dev_free(&c->d_lookback);
-    dev_free(&c->d_heaps); dev_free(&c->d_scenebox_enc); dev_free(&c->d_xctl); dev_free(&c->d_xbox);
+    dev_free(&c->d_heaps); dev_free(&c->d_scenebox_enc);
     dev_free(&c->d_keys64[0]); dev_free(&c->d_keys64[1]); dev_free(&c->d_lookback_q);
-    dev_free(&c->d_fb); dev_free(&c->d_counters); dev_free(&c->d_work); dev_free(&c->d_top);
+    dev_free(&c->d_fb); dev_free(&c->d_counters); dev_free(&c->d_work);
     for (auto& ts : c->tile_slots) { dev_free(&ts.cost); dev_free(&ts.order); }
     if (c->d_io) { cudaFree(c->d_io); c->d_io = nullptr; }
     for (int i = 0; i < 2; i++) { dev_free(&c->d_rs_keys[i]); dev_free(&c->d_rs_vals[i]); }
@@ -190,10 +190,6 @@ int bihrt_set_option(bihrt_ctx* c, const char* name, int64_t v) {
     if (!strcmp(name, "trace_blocks_per_sm")) c->opt_trace_blocks_per_sm = (int)v;
     else if (!strcmp(name, "trace_refill_threshold")) c->opt_refill_threshold = (int)std::max<int64_t>(1, std::min<int64_t>(32, v));
     else if (!strcmp(name, "build_graph")) c->opt_build_graph = (int)v;
-    else if (!strcmp(name, "build_tree")) {
-        c->opt_build_tree = (int)v;
-        if (c->build_graph_exec) { cudaGraphExecDestroy(c->build_graph_exec); c->build_graph_exec = nullptr; }
-    }
     else if (!strcmp(name, "morton_bits")) {
         // 30: the reference's 10-bit grid (parity path).  63: quality mode (non-parity): 21 bits per axis, ties broken by position,
         // subtrees of at most leaf_cap triangles collapsed into leaves.  Takes effect at the next bihrt_build / bihrt_bih_adopt.
@@ -332,18 +328,6 @@ int bihrt_scene_load_obj(bihrt_ctx* c, const char* path) {
 }
 
 // ---- build -------------------------------------------------------------------------------------
-// option build_tree: exchange words of the bottom-up k_tree, allocated on first use.  They are never cleared between builds
-// (every launch has its own tag), so they start from zero.
-static int ensure_tree_scratch(bihrt_ctx* c) {
-    if (!c->opt_build_tree || c->d_xctl) return BIHRT_OK;
-    int rc;
-    const size_t cap = (size_t)c->cap_n;
-    if ((rc = dev_alloc(c, &c->d_xctl, cap + 8))) return rc;
-    if ((rc = dev_alloc(c, &c->d_xbox, 2 * (cap + 8)))) return rc;
-    BIHRT_CUDA(c, cudaMemsetAsync(c->d_xctl, 0, (cap + 8) * sizeof(unsigned long long), c->stream));
-    BIHRT_CUDA(c, cudaMemsetAsync(c->d_xbox, 0, 2 * (cap + 8) * sizeof(float4), c->stream));
-    return BIHRT_OK;
-}
 // quality mode: 63-bit keys (two buffers) and the look-back words of 8 sort passes over 2048-key tiles, allocated on first use
 static int ensure_quality_scratch(bihrt_ctx* c) {
     int rc;
@@ -362,7 +346,6 @@ int bihrt_build(bihrt_ctx* c) {
     if (!c->have_scene || !c->d_tri_in) return bihrt_fail(c, BIHRT_ERR_STATE, "no scene loaded");
     const bool quality = c->opt_morton_bits == 63;
     if (quality) { int rq = ensure_quality_scratch(c); if (rq) return rq; }
-    { int rt = ensure_tree_scratch(c); if (rt) return rt; }
     auto build_launch = [&]() { return quality ? bihrt_build_launch_q(c) : bihrt_build_launch(c); };
     BIHRT_CUDA(c, cudaEventRecord(c->ev0, c->stream));
     if (c->n == 0) {
@@ -404,7 +387,6 @@ int bihrt_refit(bihrt_ctx* c) {
     if (!c->have_scene || !c->d_tri_in) return bihrt_fail(c, BIHRT_ERR_STATE, "no scene loaded");
     if (c->built_quality || c->opt_morton_bits == 63) return bihrt_fail(c, BIHRT_ERR_STATE, "bihrt_refit is not available in quality mode (morton_bits = 63)");
     if (!c->topology_valid) return bihrt_fail(c, BIHRT_ERR_STATE, "refit needs a full bihrt_build of the same triangle count first");
-    { int rt = ensure_tree_scratch(c); if (rt) return rt; }
     BIHRT_CUDA(c, cudaEventRecord(c->ev0, c->stream));
     int rc = bihrt_refit_launch(c);
     if (rc) return rc;

@@ -104,8 +104,6 @@ struct bihrt_ctx {
     uint32_t *d_lookback = nullptr;   // onesweep / RLE decoupled look-back words
     size_t    lookback_words = 0;
     float4   *d_heaps = nullptr;      // implicit min/max heap over the slot boxes: entry e = (lo.xyz, -), (hi.xyz, -) at [2e], [2e+1]; 2P entries
-    unsigned long long *d_xctl = nullptr;  // k_tree: per node, the 64-bit word its two children meet in (tag | far bound of the first to arrive)
-    float4   *d_xbox = nullptr;       // k_tree: per node, the box the first child to arrive leaves for the second (2 x 16 B, tagged)
     uint32_t *d_scenebox_enc = nullptr; // 6 order-preserving encoded floats
 
     // trace
@@ -115,7 +113,6 @@ struct bihrt_ctx {
     uint32_t* d_status_map = nullptr;                  // its device alias
     void*     d_io = nullptr; size_t io_cap = 0;      // staging for host ray lists / results
     unsigned long long* d_counters = nullptr;
-    BihNode*  d_top = nullptr;                         // TRACE_TOP_NODES experiment
     // ray sorting scratch (raysort.cu)
     uint32_t *d_rs_keys[2] = {nullptr, nullptr}, *d_rs_vals[2] = {nullptr, nullptr}, *d_rs_hist = nullptr, *d_rs_lookback = nullptr;
     BihHeader* d_rs_hdr = nullptr; size_t rs_cap = 0;
@@ -153,7 +150,6 @@ struct bihrt_ctx {
     int opt_sm_queues = -1; // 1: per-SM work queues (tile locality in L1), 0: one global counter, -1: by launch size
     int64_t kernel_launches = 0;
     int opt_build_graph = 1;            // replay the build as a captured CUDA graph
-    int opt_build_tree = 0;             // 0: upper heap levels + top-down k_nodes; 1: bottom-up k_tree (topology + children boxes in one pass; measured 2.5x slower, DESIGN.md)
     cudaGraphExec_t build_graph_exec = nullptr; int64_t build_graph_n = -1, build_graph_launches = 0;
     int opt_morton_bits = 30;   // 30: the reference's grid (parity path); 63: quality mode (SURVEY.md 8(f) f4, non-parity)
     int opt_leaf_cap = 4;       // quality mode: a subtree of at most this many triangles becomes one leaf
@@ -197,7 +193,6 @@ struct TraceArgs {
     int gshift;             // the samples of a pixel are spread over 2^gshift consecutive lanes (camera modes)
     uint32_t* fb;
     unsigned long long* counters; uint32_t* work;
-    const BihNode* top;     // TRACE_TOP_NODES experiment: breadth-first copy of the top levels (NULL = not staged)
     uint32_t* status_map;   // mapped host word for device-detected errors (tree of the wrong kind for this kernel)
     int refill_threshold;   // lanes whose ray ended wait until this many are idle (or nobody is busy)
     int refill_incoherent;  // threshold used instead for ray-list packets with mixed direction signs

@@ -243,7 +243,6 @@ __global__ void __launch_bounds__(256) k_morton(const float* __restrict__ tri, u
 // At 1 M triangles: 4 + 11 + 14 us of three launches -> one launch.
 // ------------------------------------------------------------------------------------------
 #define H_BAR    3000      // d_hist words [H_BAR] = arrivals, [H_BAR + 1] = generation of the grid barrier (self-resetting)
-#define H_TREE_TAG 3003     // launches of k_tree so far (bumped by the k_reorder in front of it): the tag of its exchange words
 #define H_EPOCH  3002      // builds started on this context: selects the scene-box accumulator enc[(epoch & 1) * 6 ..]
 #define FRONT_THREADS 256
 #define FRONT_STAGE_BYTES (8 * 288 * 16)              // load_quads_warp staging, one 4608-byte buffer per warp
@@ -734,11 +733,10 @@ template <bool RLE, bool QUALITY>
 __global__ void __launch_bounds__(256) k_reorder(const float* __restrict__ tri_in, const uint32_t* __restrict__ idx_sorted,
                                                  const uint32_t* __restrict__ keys_sorted, uint32_t n, BihTri* __restrict__ tris,
                                                  float4* __restrict__ heaps, uint32_t P, const uint32_t* __restrict__ tile_off,
-                                                 uint32_t* __restrict__ umc, uint32_t* __restrict__ first, uint32_t* __restrict__ hist) {
+                                                 uint32_t* __restrict__ umc, uint32_t* __restrict__ first) {
     __shared__ float s[6][8];
     __shared__ uint32_t s_w[8];
     const uint32_t j = blockIdx.x * 256u + threadIdx.x;
-    if (j == 0 && hist) hist[H_TREE_TAG] += 1u;      // a fresh tag for the exchange words of the k_tree that follows
     float mn[3] = { INFINITY, INFINITY, INFINITY }, mx[3] = { -INFINITY, -INFINITY, -INFINITY };
     uint32_t key = 0, head = 0;
     if (j < n) {
@@ -804,6 +802,18 @@ __global__ void __launch_bounds__(256) k_heap_up(float4* __restrict__ heaps, uin
     }
     __syncthreads();
     heap_reduce_block(r, s, heaps, P, base2, 0u);
+}
+
+// The heap levels above the 8 that k_reorder builds, for n slots in heaps padded to P: returns the number of k_heap_up launches
+static int heap_levels_launch(bihrt_ctx* c, uint32_t n, uint32_t P) {
+    int launches = 0;
+    for (uint32_t lvl = P >> 8, used = (n + 255) / 256; lvl > 1; lvl >>= 8, used = (used + 255) / 256) {   // level with `lvl` elements
+        const uint32_t hb = (used + 255) / 256;
+        k_heap_up<<<hb, 256, 0, c->stream>>>(c->d_heaps, P, lvl, used, c->d_hist + H_HEAPCTR);
+        if (hb <= 256 && (lvl >> 8) > 1) { lvl >>= 8; used = hb; }       // its last block has done the next 8 levels as well
+        launches++;
+    }
+    return launches;
 }
 
 // Boxes of the slot ranges [l0, r0) and [l1, r1) (heap indices at the bottom level), both walked in one loop so that up to
@@ -880,129 +890,6 @@ __global__ void __launch_bounds__(NODES_BLOCK, NODES_MINB) k_nodes(const uint32_
     heap_range_boxes(heaps, sa + P, sm + P, sm + P, sb + P, bl, br);
     node_store(nodes + idx, axis, ref_l, ref_r, bl, br);
     if (idx == 0) hdr->root_axis = (uint32_t)axis;
-}
-
-// ------------------------------------------------------------------------------------------
-// k_tree: topology + children boxes in ONE bottom-up pass, thread per leaf (replaces the upper heap levels and k_nodes on the
-// parity path and in the refit; k_nodes stays as the reference-shaped top-down variant, option build_tree = 0).
-//
-// Why: k_nodes spends ~log(range) dependent loads per node in three searches and two heap range queries, and 32 consecutive
-// nodes always contain one long one -- 14 of 32 lanes busy, 65 us at 1 M triangles.  Bottom-up every node costs O(1):
-//   a thread owns a finished subtree [a, b] of leaves (at first one leaf).  Its parent splits at p = b if the subtree has the
-//   longer common prefix with its right neighbour (delta(b) > delta(a-1); the subtree is then the LEFT child), else at p = a-1.
-//   The two children of p meet in one 64-bit atomic exchange on ctl[p]: the first to arrive leaves its far bound there, deposits
-//   its box in xbox[p] and ends; the second reads both, writes the node record (it knows both children's ranges and boxes) and
-//   climbs on with the union.  No fence anywhere: the bound rides in the atomic itself and every 16-byte half of the deposited
-//   box carries the tag of this launch, so the reader simply waits until both halves show it (aligned 16-byte accesses are
-//   single transactions).  Nothing is cleared between launches either: a stale word never carries the current tag.
-// Node numbering is the reference's (Karras): a LEFT child is the node of its LAST leaf, a right child that of its first leaf,
-// the root is node 0 -- because node i of BuildTree grows away from the neighbour it shares the SHORTER prefix with
-// (R/src/CUDAKernels.cu:616-651).  So the finished subtree [a, b] is node b if delta(b) > delta(a-1), else node a: the same
-// comparison that finds its parent.  Boxes are unions of the same per-slot boxes as the heap queries: bit-identical nodes.
-// ------------------------------------------------------------------------------------------
-
-__device__ __forceinline__ float4 ld_volatile_f4(const float4* p) {
-    float4 v; asm volatile("ld.volatile.global.v4.f32 {%0,%1,%2,%3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "l"(p) : "memory"); return v;
-}
-__device__ __forceinline__ void st_volatile_f4(float4* p, float4 v) {
-    asm volatile("st.volatile.global.v4.f32 [%0], {%1,%2,%3,%4};" :: "l"(p), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
-}
-
-// box of the slots [l, r) (bottom-level heap indices): levels 0..8 exist below a k_reorder block, above them walk level 8
-__device__ __forceinline__ void leaf_box(const float4* __restrict__ heaps, uint32_t l, uint32_t r, float b[6]) {
-#pragma unroll
-    for (int k = 0; k < 3; k++) { b[k] = INFINITY; b[3 + k] = -INFINITY; }
-    int level = 0;
-    while (l < r && level < 8) {
-        if (l & 1u) heap_merge(heaps, l++, b);
-        if (r & 1u) heap_merge(heaps, --r, b);
-        l >>= 1; r >>= 1; level++;
-    }
-    for (; l < r; l++) heap_merge(heaps, l, b);
-}
-
-#define TREE_BLOCK 128
-__global__ void __launch_bounds__(TREE_BLOCK) k_tree(const uint32_t* __restrict__ umc, const uint32_t* __restrict__ first,
-                                                     BihHeader* hdr, const float4* __restrict__ heaps, uint32_t P,
-                                                     BihNode* __restrict__ nodes, unsigned long long* __restrict__ ctl,
-                                                     float4* __restrict__ xbox, const uint32_t* __restrict__ hist,
-                                                     uint32_t* __restrict__ status_map) {
-    const int i = blockIdx.x * blockDim.x + threadIdx.x;
-    const int nu = (int)hdr->nu;
-    if (i == 0) *status_map = hdr->status;      // last kernel of the build: the watchdog word, mirrored into mapped host memory
-    const uint32_t tag = hist[H_TREE_TAG];
-    const float ftag = __uint_as_float(tag);
-    bool alive = i < nu && nu >= 2;
-    int a = i, b = i;
-    uint32_t ka = 0, kb = 0, kl = 0, kr = 0;    // umc[a], umc[b], umc[a-1], umc[b+1]
-    uint32_t ref = 0;                           // reference to the finished subtree [a, b]
-    bool left = false;                          // ... which is the left child of its parent,
-    int p = 0;                                  // ... the node that splits between leaves p and p+1
-    float box[6] = { 0.f, 0.f, 0.f, 0.f, 0.f, 0.f };
-    if (alive) {
-        ka = kb = __ldg(umc + i);
-        int dl = -1, dr = -1;
-        if (i > 0)      { kl = __ldg(umc + i - 1); dl = __clz(kl ^ ka); }
-        if (i < nu - 1) { kr = __ldg(umc + i + 1); dr = __clz(kb ^ kr); }
-        left = dr > dl; p = left ? b : a - 1;
-        const uint32_t s0 = __ldg(first + i), s1 = __ldg(first + i + 1);
-        ref = BIH_REF_LEAFREF(s0);
-        leaf_box(heaps, s0 + P, s1 + P, box);
-    }
-    while (__any_sync(FULL, alive)) {
-        bool second = false;
-        unsigned long long old = 0;
-        if (alive) {
-            old = atomicExch(ctl + p, ((unsigned long long)tag << 32) | (uint32_t)(left ? a : b));
-            second = (uint32_t)(old >> 32) == tag;
-            if (!second) {                      // first to arrive: leave the box and end
-                st_volatile_f4(xbox + 2 * (size_t)p, make_float4(box[0], box[1], box[2], ftag));
-                st_volatile_f4(xbox + 2 * (size_t)p + 1, make_float4(box[3], box[4], box[5], ftag));
-                alive = false;
-            }
-        }
-        __syncwarp();                           // a sibling in this warp has issued its deposit before anyone waits for one
-        if (second) {
-            float4 h0, h1;
-            do { h0 = ld_volatile_f4(xbox + 2 * (size_t)p); } while (__float_as_uint(h0.w) != tag);
-            do { h1 = ld_volatile_f4(xbox + 2 * (size_t)p + 1); } while (__float_as_uint(h1.w) != tag);
-            const float sib[6] = { h0.x, h0.y, h0.z, h1.x, h1.y, h1.z };
-            const int far = (int)(uint32_t)old;
-            const uint32_t ms = left ? kb : kl, ms1 = left ? kr : ka;    // umc[p], umc[p+1]
-            const int axis = (__clz(ms ^ ms1) + 1) % 3;                  // R/src/CUDAKernels.cu:702-706
-            uint32_t ref_l, ref_r;
-            float bl[6], br[6];
-            if (left) {                         // this subtree = [a, p], sibling = [p+1, far]
-                ref_l = ref;
-                b = far; kb = __ldg(umc + b);
-                ref_r = (p + 1 == b) ? BIH_REF_LEAFREF(__ldg(first + p + 1)) : BIH_REF_NODE(p + 1, (__clz(ms1 ^ kb) + 1) % 3);
-#pragma unroll
-                for (int k = 0; k < 6; k++) { bl[k] = box[k]; br[k] = sib[k]; }
-            } else {                            // sibling = [far, p], this subtree = [p+1, b]
-                ref_r = ref;
-                a = far; ka = __ldg(umc + a);
-                ref_l = (a == p) ? BIH_REF_LEAFREF(__ldg(first + a)) : BIH_REF_NODE(p, (__clz(ka ^ ms) + 1) % 3);
-#pragma unroll
-                for (int k = 0; k < 6; k++) { bl[k] = sib[k]; br[k] = box[k]; }
-            }
-            // the node's own index (root = 0, else the end it does not grow from) and its parent, from the same comparison
-            int id = 0;
-            if (a == 0 && b == nu - 1) {
-                hdr->root_axis = (uint32_t)axis;
-                alive = false;
-            } else {
-                int dl = -1, dr = -1;
-                if (a > 0)      { kl = __ldg(umc + a - 1); dl = __clz(kl ^ ka); }
-                if (b < nu - 1) { kr = __ldg(umc + b + 1); dr = __clz(kb ^ kr); }
-                left = dr > dl;
-                id = left ? b : a; p = left ? b : a - 1;
-            }
-            node_store(nodes + id, axis, ref_l, ref_r, bl, br);
-            ref = BIH_REF_NODE(id, axis);
-#pragma unroll
-            for (int k = 0; k < 3; k++) { box[k] = fminf(bl[k], br[k]); box[3 + k] = fmaxf(bl[3 + k], br[3 + k]); }
-        }
-    }
 }
 
 // ==========================================================================================
@@ -1146,14 +1033,8 @@ int bihrt_build_launch_q(bihrt_ctx* c) {
     }
     uint32_t P = 256;
     while (P < n) P <<= 1;
-    k_reorder<false, true><<<(n + 255) / 256, 256, 0, st>>>(c->d_tri_in, c->d_vals[cur], nullptr, n, c->d_tris, c->d_heaps, P, nullptr, nullptr, nullptr, nullptr);
-    int launches = 0;
-    for (uint32_t lvl = P >> 8, used = (n + 255) / 256; lvl > 1; lvl >>= 8, used = (used + 255) / 256) {   // level with `lvl` elements
-        const uint32_t hb = (used + 255) / 256;
-        k_heap_up<<<hb, 256, 0, st>>>(c->d_heaps, P, lvl, used, c->d_hist + H_HEAPCTR);
-        if (hb <= 256 && (lvl >> 8) > 1) { lvl >>= 8; used = hb; }       // its last block has done the next 8 levels as well
-        launches++;
-    }
+    k_reorder<false, true><<<(n + 255) / 256, 256, 0, st>>>(c->d_tri_in, c->d_vals[cur], nullptr, n, c->d_tris, c->d_heaps, P, nullptr, nullptr, nullptr);
+    const int launches = heap_levels_launch(c, n, P);
     k_nodes_q<<<(n + 127) / 128, 128, 0, st>>>(c->d_keys64[cur], n, (uint32_t)c->opt_leaf_cap, c->d_hdr, c->d_heaps, P, c->d_nodes, c->d_tris, c->d_status_map);
     c->kernel_launches += 13 + launches;
     BIHRT_CUDA(c, cudaGetLastError());
@@ -1197,26 +1078,15 @@ int bihrt_build_launch(bihrt_ctx* c) {
     // heaps are padded to a power of two >= n (Nu <= n is only known on the device)
     uint32_t P = 256;
     while (P < n) P <<= 1;
-    k_reorder<true, false><<<(n + 255) / 256, 256, 0, st>>>(c->d_tri_in, c->d_vals[cur], c->d_keys[cur], n, c->d_tris, c->d_heaps, P, tile_cnt, c->d_umc, c->d_first, c->d_hist);
+    k_reorder<true, false><<<(n + 255) / 256, 256, 0, st>>>(c->d_tri_in, c->d_vals[cur], c->d_keys[cur], n, c->d_tris, c->d_heaps, P, tile_cnt, c->d_umc, c->d_first);
     PROF_MARK();   // 9: after reorder + slot boxes + leaves
-    int launches = 0;
-    if (c->opt_build_tree) {
-        PROF_MARK();   // 10
-        k_tree<<<(n + TREE_BLOCK - 1) / TREE_BLOCK, TREE_BLOCK, 0, st>>>(c->d_umc, c->d_first, c->d_hdr, c->d_heaps, P, c->d_nodes, c->d_xctl, c->d_xbox, c->d_hist, c->d_status_map);
-    } else {
-        for (uint32_t lvl = P >> 8, used = (n + 255) / 256; lvl > 1; lvl >>= 8, used = (used + 255) / 256) {   // level with `lvl` elements
-            const uint32_t hb = (used + 255) / 256;
-            k_heap_up<<<hb, 256, 0, st>>>(c->d_heaps, P, lvl, used, c->d_hist + H_HEAPCTR);
-            if (hb <= 256 && (lvl >> 8) > 1) { lvl >>= 8; used = hb; }       // its last block has done the next 8 levels as well
-            launches++;
-        }
-        PROF_MARK();   // 10: after upper heap levels
-        k_nodes<<<(n + NODES_BLOCK - 1) / NODES_BLOCK, NODES_BLOCK, 0, st>>>(c->d_umc, c->d_first, c->d_hdr, c->d_heaps, P, c->d_nodes, c->d_status_map);
-    }
+    const int launches = heap_levels_launch(c, n, P);
+    PROF_MARK();   // 10: after upper heap levels
+    k_nodes<<<(n + NODES_BLOCK - 1) / NODES_BLOCK, NODES_BLOCK, 0, st>>>(c->d_umc, c->d_first, c->d_hdr, c->d_heaps, P, c->d_nodes, c->d_status_map);
     PROF_MARK();   // 11: after nodes
     PROF_MARK();   // 12: after reorder
     c->prof_count = pe;
-    c->kernel_launches += 9 + launches;    // k_front, 4 x k_onesweep, k_rle_count, k_rle_scan, k_reorder, k_heap_up.., k_nodes (or k_tree)
+    c->kernel_launches += 9 + launches;    // k_front, 4 x k_onesweep, k_rle_count, k_rle_scan, k_reorder, k_heap_up.., k_nodes
     BIHRT_CUDA(c, cudaGetLastError());
     return BIHRT_OK;
 }
@@ -1244,19 +1114,9 @@ int bihrt_refit_launch(bihrt_ctx* c) {
     k_refit_init<<<1, 32, 0, st>>>(c->d_scenebox_enc + ENC_AUX);
     k_scene_box<<<stream_grid, 256, 0, st>>>(c->d_tri_in, n, c->d_scenebox_enc + ENC_AUX);
     k_refit_box<<<1, 32, 0, st>>>(c->d_scenebox_enc + ENC_AUX, c->d_hdr);
-    k_reorder<false, false><<<(n + 255) / 256, 256, 0, st>>>(c->d_tri_in, c->d_vals[0], c->d_keys[0], n, c->d_tris, c->d_heaps, P, nullptr, nullptr, nullptr, c->d_hist);
-    int launches = 0;
-    if (c->opt_build_tree) {
-        k_tree<<<(n + TREE_BLOCK - 1) / TREE_BLOCK, TREE_BLOCK, 0, st>>>(c->d_umc, c->d_first, c->d_hdr, c->d_heaps, P, c->d_nodes, c->d_xctl, c->d_xbox, c->d_hist, c->d_status_map);
-    } else {
-        for (uint32_t lvl = P >> 8, used = (n + 255) / 256; lvl > 1; lvl >>= 8, used = (used + 255) / 256) {   // level with `lvl` elements
-            const uint32_t hb = (used + 255) / 256;
-            k_heap_up<<<hb, 256, 0, st>>>(c->d_heaps, P, lvl, used, c->d_hist + H_HEAPCTR);
-            if (hb <= 256 && (lvl >> 8) > 1) { lvl >>= 8; used = hb; }       // its last block has done the next 8 levels as well
-            launches++;
-        }
-        k_nodes<<<(n + NODES_BLOCK - 1) / NODES_BLOCK, NODES_BLOCK, 0, st>>>(c->d_umc, c->d_first, c->d_hdr, c->d_heaps, P, c->d_nodes, c->d_status_map);
-    }
+    k_reorder<false, false><<<(n + 255) / 256, 256, 0, st>>>(c->d_tri_in, c->d_vals[0], c->d_keys[0], n, c->d_tris, c->d_heaps, P, nullptr, nullptr, nullptr);
+    const int launches = heap_levels_launch(c, n, P);
+    k_nodes<<<(n + NODES_BLOCK - 1) / NODES_BLOCK, NODES_BLOCK, 0, st>>>(c->d_umc, c->d_first, c->d_hdr, c->d_heaps, P, c->d_nodes, c->d_status_map);
     c->kernel_launches += 5 + launches;
     BIHRT_CUDA(c, cudaGetLastError());
     return BIHRT_OK;

@@ -45,35 +45,6 @@
 #define TRACE_MIN_BLOCKS 8        // <= 64 registers per thread
 #endif
 
-// The newest TRACE_SSTACK items of every lane's stack live in SHARED memory (slot i & (TRACE_SSTACK-1) of a per-thread column:
-// 16-byte accesses of consecutive threads are conflict-free whatever row each lane is on); older items spill to the
-// local-memory array, which a root-to-leaf path of a shallow tree never reaches.  Local memory is cached in L1 like the nodes
-// and triangles that stream through it, so a popped item is often an L2 round trip away (the pop was the top stall of the
-// 1 spp profile next to the node fetch itself); shared memory is never evicted.  0 = everything in local memory.
-// MEASURED (round 2, B200, 1 M triangles; Mrays/s with 0 / 4 / 8 shared items): 1080p x 1 spp 2887 / 2661 / 2901, x 4 spp
-// 3805 / 3506 / 3634, x 16 spp 5015 / 4594 / 4694, 4K x 16 spp 5983 / 5446 / 5519; 10 M triangles and the atrium lose 2-7 %
-// too.  The ring bookkeeping costs more issue slots than the pops save, and 16 KB x items of shared memory per SM come out
-// of the L1 the nodes live in.  Shipped: 0.
-#ifndef TRACE_SSTACK
-#define TRACE_SSTACK 0
-#endif
-
-// Shared-memory staging of the top levels of the tree (named in the north star), as a compile-time experiment: the first
-// TRACE_TOP_NODES nodes in breadth-first order (127 = 7 levels, 8 KB) are copied into every block's shared memory when the
-// kernel starts; references between them carry TOP_FLAG and index the table, so the top of every ray's walk never leaves
-// the SM.  0 = off (every node comes through L1).
-// MEASURED (round 2, B200, same results bit for bit; Mrays/s with 0 / 31 / 127 / 255 staged nodes): 1 M triangles 1080p x 1 spp
-// 5786 / 5429 / 5458 / 5127, 1080p x 16 spp 10029 / 9297 / 9297 / 9050, 4K x 16 spp 11759 / - / 10879 / -; atrium 1080p x 1 spp
-// 6009 / 5371 / 5302 / 5287, x 16 spp 7231 / 6581 / 6572 / 6549: 6-12 % slower everywhere -- the top levels are the
-// hottest lines of L1 anyway (every warp of every SM reads them all the time), a shared-memory copy replaces an L1 hit by a
-// 4 x LDS.128 that conflicts whenever the lanes of a warp disagree on the node, costs a compare-and-branch per step in an
-// issue-bound loop, and its 8 KB x 8 blocks come out of the L1 the deep levels need.  Shipped: 0.
-#ifndef TRACE_TOP_NODES
-#define TRACE_TOP_NODES 0
-#endif
-#ifndef TRACE_LDG256
-#define TRACE_LDG256 1
-#endif
 // Framebuffer renders (MODE 1) as coverage queries: a pixel's colour depends only on WHETHER each sample hits, so a sample
 // ends at the first triangle it accepts -- inside the leaf and for the whole walk -- instead of searching on for the
 // closest one.  Until that first hit the walk is the closest-hit walk step for step (h.t is FLT_MAX in both: same strict
@@ -84,7 +55,6 @@
 #ifndef TRACE_COVERAGE_EXIT
 #define TRACE_COVERAGE_EXIT 1
 #endif
-#define TOP_FLAG 0x40000000u
 #define BOX_EPS 2.384185791015625e-07f      /* 2^-22: the box tests' margin is this times (largest finite |o/d| + larger end of the ray's scene interval), one constant per ray */
 
 // (double)det < 0.000001 (R/src/CUDAKernels.cu:28)  <=>  det < 0x358637be as binary32
@@ -205,13 +175,6 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
         if (blockIdx.x == 0 && threadIdx.x == 0 && a.status_map) *a.status_map = 0x100u;
         return;
     }
-#if TRACE_TOP_NODES > 0
-    __shared__ float4 s_top[TRACE_TOP_NODES * 4];
-    if (a.top) {
-        for (int i = threadIdx.x; i < TRACE_TOP_NODES * 4; i += TRACE_THREADS) s_top[i] = __ldg(reinterpret_cast<const float4*>(a.top) + i);
-        __syncthreads();
-    }
-#endif
     const float blo[3] = { a.hdr->lo[0], a.hdr->lo[1], a.hdr->lo[2] }, bhi[3] = { a.hdr->hi[0], a.hdr->hi[1], a.hdr->hi[2] };
     uint32_t nnodes = 0, ntris = 0, maxsp = 0;
     uint32_t wnode = 0, wleaf = 0;              // COUNTED: warp-level executions of the node step / the triangle test (SIMD efficiency = lane steps / 32 / these)
@@ -252,33 +215,10 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
     bool tracing = false;                      // a ray is in flight (its result has not been recorded)
     uint4 stack[STACK_DEPTH];
     int sp = 0;
-#if TRACE_SSTACK > 0
-    __shared__ uint4 s_stack[TRACE_SSTACK * TRACE_THREADS];
-    uint4* const my_stack = s_stack + threadIdx.x;
-    int lo = 0;                                // items [0, lo) are in local memory, [lo, sp) in shared memory; sp - lo <= TRACE_SSTACK
-#define STACK_RESET() do { sp = 0; lo = 0; } while (0)
-#define STACK_PUSH(item)                                                                                    \
-        do {                                                                                                \
-            if (sp - lo == TRACE_SSTACK) { stack[lo] = my_stack[(lo & (TRACE_SSTACK - 1)) * TRACE_THREADS]; lo++; }   \
-            my_stack[(sp & (TRACE_SSTACK - 1)) * TRACE_THREADS] = (item);                                   \
-            sp++;                                                                                           \
-        } while (0)
-#define STACK_POP(e)                                                                                        \
-        do {                                                                                                \
-            sp--;                                                                                           \
-            (e) = my_stack[(sp & (TRACE_SSTACK - 1)) * TRACE_THREADS];                                      \
-            if (sp == lo && lo > 0) { lo--; my_stack[(lo & (TRACE_SSTACK - 1)) * TRACE_THREADS] = stack[lo]; }  \
-        } while (0)
-#else
 #define STACK_RESET() do { sp = 0; } while (0)
 #define STACK_PUSH(item) do { stack[sp] = (item); sp++; } while (0)
 #define STACK_POP(e) do { sp--; (e) = stack[sp]; } while (0)
-#endif
-#if TRACE_TOP_NODES > 0
-    const uint32_t root_ref = BIH_REF_NODE(0, a.hdr->root_axis) | (a.top ? TOP_FLAG : 0u);
-#else
     const uint32_t root_ref = BIH_REF_NODE(0, a.hdr->root_axis);
-#endif
     const bool vote = WALK > 0 || a.vote_wait != 0;
     int thresh = a.refill_threshold;          // lanes that must be idle before a partial refill (warp-uniform)
     // colours with a pixel's samples in several lanes: the warp moves from sample to sample in lock step, so the lanes
@@ -604,12 +544,6 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 // node address = base + index * 64, as one 32x32->64 multiply-add on the base pointer
                 const float4* np;
                 asm("mad.wide.u32 %0, %1, 64, %2;" : "=l"(np) : "r"(cur >> 2), "l"(nodes_b));
-#if TRACE_TOP_NODES > 0
-                float4 nd, b0, b1, b2;
-                if (cur & TOP_FLAG) { const float4* tp4 = s_top + ((cur & ~TOP_FLAG) >> 2) * 4; nd = tp4[0]; b0 = tp4[1]; b1 = tp4[2]; b2 = tp4[3]; }
-                else { nd = __ldg(np); b0 = __ldg(np + 1); b1 = __ldg(np + 2); b2 = __ldg(np + 3); }
-#else
-#if TRACE_LDG256
                 // Ray lists (MODE 0 and 3) fetch the 64-byte node as TWO 256-bit read-only loads (LDG.E.256, new on sm_100) instead of
                 // four 128-bit ones.  Measured (B200, Mrays/s, 128-bit -> 256-bit): diffuse bounce list on the atrium 2157 -> 2304
                 // (there every lane fetches its own node and the L1 tag stage is the busiest unit, 88 %), 1 M triangles 1080p x 1
@@ -623,10 +557,6 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                     asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
                         : "=f"(b1.x), "=f"(b1.y), "=f"(b1.z), "=f"(b1.w), "=f"(b2.x), "=f"(b2.y), "=f"(b2.z), "=f"(b2.w) : "l"(np + 2));
                 } else { nd = __ldg(np); b0 = __ldg(np + 1); b1 = __ldg(np + 2); b2 = __ldg(np + 3); }
-#else
-                const float4 nd = __ldg(np), b0 = __ldg(np + 1), b1 = __ldg(np + 2), b2 = __ldg(np + 3);
-#endif
-#endif
                 if (COUNTED) { nnodes++; const uint32_t am = __activemask(); wnode += (lane == __ffs(am) - 1); }
                 const uint32_t rl = __float_as_uint(nd.z), rr = __float_as_uint(nd.w);
                 const bool neg = oi.y < 0.f;                           // near = sign[axis], :286
@@ -811,37 +741,6 @@ int bihrt_resolve_launch(bihrt_ctx* c, uint32_t* fb, int npix, int spp) {
     return BIHRT_OK;
 }
 
-#if TRACE_TOP_NODES > 0
-// breadth-first copy of the first TRACE_TOP_NODES nodes with the references between them rewritten to table references
-__global__ void __launch_bounds__(128) k_top(const BihNode* __restrict__ nodes, const BihHeader* __restrict__ hdr, BihNode* __restrict__ top) {
-    __shared__ uint32_t s_src[TRACE_TOP_NODES];
-    __shared__ int s_cnt;
-    if (hdr->nu < 2) return;
-    if (threadIdx.x == 0) { s_src[0] = 0; s_cnt = 1; }
-    __syncthreads();
-    int lo = 0, hi = 1;
-    while (lo < hi) {
-        for (int e = lo + threadIdx.x; e < hi; e += blockDim.x) {
-            BihNode nd = nodes[s_src[e]];
-            uint32_t* refs[2] = { &nd.ref_l, &nd.ref_r };
-            for (int k = 0; k < 2; k++) {
-                const uint32_t r = *refs[k];
-                if (!(r & BIH_REF_LEAF)) {
-                    const int slot = atomicAdd(&s_cnt, 1);
-                    if (slot < TRACE_TOP_NODES) { s_src[slot] = r >> 2; *refs[k] = TOP_FLAG | ((uint32_t)slot << 2) | (r & 3u); }
-                }
-            }
-            top[e] = nd;
-        }
-        __syncthreads();
-        lo = hi; hi = min(s_cnt, TRACE_TOP_NODES);
-        __syncthreads();
-        if (threadIdx.x == 0) s_cnt = hi;
-        __syncthreads();
-    }
-}
-#endif
-
 #ifndef TRACE_WALK
 #define TRACE_WALK 4
 #endif
@@ -924,13 +823,6 @@ int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a_in, int mode, bool count
     const bool shipped = a.vote_wait != 0 && a.vote_walk == TRACE_WALK;    // the unrolled instantiation
     int rc = BIHRT_ERR_INVALID;
     a.status_map = c->d_status_map;
-#if TRACE_TOP_NODES > 0
-    if (c->n < (1ll << 28) && !counted) {
-        if (!c->d_top) BIHRT_CUDA(c, cudaMalloc((void**)&c->d_top, sizeof(BihNode) * TRACE_TOP_NODES));
-        k_top<<<1, 128, 0, c->stream>>>(c->d_nodes, c->d_hdr, c->d_top);       // (experiment: rebuilt per launch, ~3 us)
-        a.top = c->d_top;
-    }
-#endif
     if (c->built_quality) {
         // quality-mode tree: the shipped schedule only (TRACE_WALK node steps per vote); the instrumented build walks one step per vote
         TraceArgs q = a; q.vote_wait = 1; q.vote_walk = 1;

@@ -144,10 +144,9 @@ def test_refit_keeps_hits_correct(renderer, scenes, oracle):
 
 
 @pytest.mark.parametrize("name", ["cornell", "sphere187", "atrium", "duplicates", "flat", "soup8193", "single", "two"])
-def test_bottom_up_tree_option_is_bit_exact(renderer, scenes, oracle, name):
-    """Option build_tree = 1: topology + children boxes in one bottom-up pass (k_tree; measured slower and left off, DESIGN.md).
-    Same node numbering, references, clip planes and children boxes as the top-down path, rebuilt twice (the exchange words are
-    never cleared between launches) and through a refit."""
+def test_rebuild_and_refit_reproduce_the_blob(renderer, scenes, oracle, name):
+    """The whole blob (header, 64-byte nodes with the children boxes, triangle records) is a function of the triangles alone:
+    a second build over the scratch of the first and a refit of unmoved vertices rewrite it byte for byte."""
     tri = {
         "cornell": lambda: scenes.cornell_box(),
         "sphere187": lambda: scenes.displaced_sphere(187),
@@ -167,17 +166,13 @@ def test_bottom_up_tree_option_is_bit_exact(renderer, scenes, oracle, name):
         return torch.as_tensor(multi._CudaView(ptr, (nbytes,), "|u1"), device="cuda:%d" % renderer.device).cpu().numpy()
 
     renderer.load_models(tri).build()
+    assert_view_equals_oracle(renderer.reference_view(), oracle.Bih(tri))
     blob_ref = blob()
-    renderer.set_option("build_tree", 1)
-    try:
-        for _ in range(2):
-            renderer.build()
-            assert_view_equals_oracle(renderer.reference_view(), oracle.Bih(tri))
-            assert np.array_equal(blob(), blob_ref)          # header, 64-byte nodes (children boxes), triangle records
-        renderer.refit()
-        assert np.array_equal(blob(), blob_ref)
-    finally:
-        renderer.set_option("build_tree", 0)
+    renderer.build()
+    assert_view_equals_oracle(renderer.reference_view(), oracle.Bih(tri))
+    assert np.array_equal(blob(), blob_ref)
+    renderer.refit()
+    assert np.array_equal(blob(), blob_ref)
 
 
 def test_builds_alternate_cleanly_between_parity_quality_and_refit(renderer, scenes, oracle):
