@@ -67,6 +67,7 @@ class Hits(C.Structure):
 
 
 INTERSECT_ANY = 1
+INTERSECT_TWO_SIDED = 4
 HIT_OUTPUTS = ("t", "u", "v", "slot", "prim", "ng")
 
 
@@ -332,10 +333,11 @@ class Renderer:
             self.torch_wait()
         return blocker
 
-    def intersect(self, rays8, any_hit=False, outputs=HIT_OUTPUTS):
+    def intersect(self, rays8, any_hit=False, two_sided=False, outputs=HIT_OUTPUTS):
         """Ray queries with per-ray intervals (bihrt_intersect).  rays8: (N,8) float32 o.xyz tmin d.xyz tmax (numpy or torch,
         host or device; interval_rays builds it).  A triangle counts when max(tmin,0) < t < min(tmax,FLT_MAX); any_hit ends a
-        ray at the first one (occlusion).  Returns {name: array} for the requested outputs of
+        ray at the first one (occlusion).  two_sided accepts back faces too (BIHRT_INTERSECT_TWO_SIDED): dot(d, ng) > 0 marks
+        a back-face hit.  Returns {name: array} for the requested outputs of
         t (N,), u (N,), v (N,), slot (N,), prim (N,), ng (N,3): numpy for numpy input, torch tensors on the rays' device for
         torch input.  A miss reads t = FLT_MAX, slot = prim = -1, u = v = ng = 0."""
         unknown = set(outputs) - set(HIT_OUTPUTS)
@@ -353,11 +355,11 @@ class Renderer:
             res = {k: torch.empty((n,) + shapes[k], dtype=torch.int32 if k in ("slot", "prim") else torch.float32, device=rays8.device)
                    for k in outputs}
         hits = Hits(**{k: _ptr(res[k]) for k in res})
+        flags = (INTERSECT_ANY if any_hit else 0) | (INTERSECT_TWO_SIDED if two_sided else 0)
         on_dev = getattr(rays8, "is_cuda", False)
         if on_dev:
             self.wait_torch()            # rays (and recycled output blocks) were last touched on torch's current stream
-        self._check(self._lib.bihrt_intersect(self._ctx, _ptr(rays8), C.c_int64(n), C.c_uint32(INTERSECT_ANY if any_hit else 0),
-                                              C.byref(hits)))
+        self._check(self._lib.bihrt_intersect(self._ctx, _ptr(rays8), C.c_int64(n), C.c_uint32(flags), C.byref(hits)))
         if on_dev:
             self.torch_wait()            # device outputs are written asynchronously on the context's stream
         return res

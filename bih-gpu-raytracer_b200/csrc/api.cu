@@ -585,10 +585,11 @@ int bihrt_trace_any(bihrt_ctx* c, const bihrt_ray* rays, int64_t n, float tmax, 
     return trace_impl(c, rays, n, nullptr, blocker, nullptr, nullptr, true, tmax);
 }
 
-// Ray queries with per-ray intervals and hit records (include/bihrt.h): k_trace MODE 3.
+// Ray queries with per-ray intervals and hit records (include/bihrt.h): k_trace MODE 3, MODE 4 with two-sided triangles.
 int bihrt_intersect(bihrt_ctx* c, const bihrt_ray_interval* rays, int64_t n, uint32_t flags, const bihrt_hits* out) {
     ENTER(c);
-    if (flags & ~BIHRT_INTERSECT_ANY) return bihrt_fail(c, BIHRT_ERR_INVALID, "unknown flags 0x%x", flags & ~BIHRT_INTERSECT_ANY);
+    const uint32_t known = BIHRT_INTERSECT_ANY | BIHRT_INTERSECT_TWO_SIDED;
+    if (flags & ~known) return bihrt_fail(c, BIHRT_ERR_INVALID, "unknown flags 0x%x", flags & ~known);
     if (!out) return bihrt_fail(c, BIHRT_ERR_INVALID, "no output record");
     if (n < 0 || (n > 0 && !rays)) return bihrt_fail(c, BIHRT_ERR_INVALID, "bad ray array");
     if (n >= (1ll << 32) - (1ll << 24)) return bihrt_fail(c, BIHRT_ERR_INVALID, "too many rays in one call (32-bit work counter)");
@@ -610,7 +611,7 @@ int bihrt_intersect(bihrt_ctx* c, const bihrt_ray_interval* rays, int64_t n, uin
     a.nrays = n; a.any_hit = (flags & BIHRT_INTERSECT_ANY) ? 1 : 0;
     a.out_t = o.t(); a.out_slot = o.slot(); a.out_prim = o.prim();
     a.out_u = (float*)o.dev[OUT_U]; a.out_v = (float*)o.dev[OUT_V]; a.out_ng = (float*)o.dev[OUT_NG];
-    if ((rc = bihrt_trace_launch(c, a, 3, false))) return rc;
+    if ((rc = bihrt_trace_launch(c, a, (flags & BIHRT_INTERSECT_TWO_SIDED) ? 4 : 3, false))) return rc;
     return unstage_outputs(c, n, o);
 }
 

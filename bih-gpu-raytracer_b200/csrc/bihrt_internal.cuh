@@ -200,12 +200,12 @@ struct TraceArgs {
     int queues;             // > 1: one work queue per SM (tile t -> queue t % queues) with stealing
     int vote_wait, vote_walk;   // vote_wait != 0: the node phase also ends when the waiting lanes outnumber the walking ones;
                                 // vote_walk: node steps a lane may take between two votes
-    // MODE 3 (bihrt_intersect): rays with intervals instead of `rays`, and the hit record's other outputs (NULL = not wanted);
+    // MODE 3 and 4 (bihrt_intersect): rays with intervals instead of `rays`, and the hit record's other outputs (NULL = not wanted);
     // any_hit = BIHRT_INTERSECT_ANY (tmax comes with every ray)
     const bihrt_ray_interval* rays_iv;
     float* out_u; float* out_v; float* out_ng;
 };
-int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a, int mode /*0 rays,1 render fb,2 render hits,3 ray queries*/, bool counted);
+int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a, int mode /*0 rays,1 render fb,2 render hits,3 ray queries,4 two-sided ray queries*/, bool counted);
 int bihrt_resolve_launch(bihrt_ctx* c, uint32_t* fb, int npix, int spp);
 int bihrt_tile_order_launch(bihrt_ctx* c, uint32_t* cost, uint32_t* order, uint32_t ntiles, bool full_sort);
 // raysort.cu: permutation that groups a ray list by origin cell and direction octant (perm[i] = index of the i-th ray to trace)

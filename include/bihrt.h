@@ -171,9 +171,24 @@ BIHRT_API int bihrt_trace_any(bihrt_ctx* ctx, const bihrt_ray* rays, int64_t n, 
  *              point is ~ (1-u-v) v0 + u v1 + v v2 in the triangle's input vertex order;
  *        slot, prim  as bihrt_trace;
  *        ng    geometric normal e1 x e2, e1 = v1 - v0, e2 = v2 - v0, NOT normalised, binary32 with every product rounded and
- *              no FMA: (e1y*e2z - e1z*e2y, e1z*e2x - e1x*e2z, e1x*e2y - e1y*e2x), 3 floats per ray.  Hits are front faces
- *              only (det >= 1e-6, as in the reference), so dot(d, ng) < 0.
+ *              no FMA: (e1y*e2z - e1z*e2y, e1z*e2x - e1x*e2z, e1x*e2y - e1y*e2x), 3 floats per ray.  ng keeps the input
+ *              winding, so it tells the side that was hit: dot(d, ng) < 0 on a front face, > 0 on a back face (the
+ *              convention Embree uses).  Without BIHRT_INTERSECT_TWO_SIDED hits are front faces only (det >= 1e-6, as in
+ *              the reference), so dot(d, ng) < 0.
  *        miss: t = FLT_MAX, slot = prim = -1, u = v = 0, ng = (0, 0, 0).
+ *      BIHRT_INTERSECT_TWO_SIDED (combines with BIHRT_INTERSECT_ANY): back faces count too.  A triangle is a candidate when
+ *        !(|det| < 1e-6) instead of !(det < 1e-6) -- Moller-Trumbore's non-culling branch -- and everything after that test is
+ *        the same arithmetic (1 / det rounds symmetrically), so u, v, t of a front face are computed bit for bit as without the
+ *        flag.  The walk is unchanged (strict plane test, far-leaf-first order, the flat-geometry misses of the parity tree,
+ *        the quality tree's rules); only more triangles are accepted.  Hence:
+ *          - every ray the one-sided query hits, the two-sided query hits, with t <= the one-sided t;
+ *          - where the two-sided record's triangle is front-facing, the record equals the one-sided one (slot and prim
+ *            may differ only between triangles at exactly the same t);
+ *          - on quality-mode trees, hits equal two-sided brute force over the interval, except where triangles of
+ *            different leaves lie in one plane (coincident surfaces, such as the bottom face of a box resting on a floor,
+ *            which only a two-sided query can hit from above): their t differ only by rounding, and the walk may report
+ *            the one whose t is an ulp larger.
+ *        A ray from inside a closed mesh sees its inner (back) faces; peeling visits entry and exit hits in order.
  *      Quality-mode trees (morton_bits 63): same contract without the reference's quirks; hits equal brute force over the
  *      interval.  The option trace_sort_rays does not apply (rays are traced in list order).  rays: host or device; device
  *      rays must be 16-byte aligned (a ray is read as two 128-bit loads).  Host outputs: the call synchronises and leaves them
@@ -192,6 +207,7 @@ typedef struct bihrt_hits {
     float*   ng;    /* [3n] geometric normal, xyz per ray */
 } bihrt_hits;
 #define BIHRT_INTERSECT_ANY 1u   /* occlusion: end at the first accepted triangle of the interval */
+#define BIHRT_INTERSECT_TWO_SIDED 4u   /* back faces count too (|det| >= 1e-6); flag values 0, 1, 4 and 5 are valid */
 BIHRT_API int bihrt_intersect(bihrt_ctx* ctx, const bihrt_ray_interval* rays, int64_t n, uint32_t flags, const bihrt_hits* out);
 /* instrumented trace: counters[0]=internal nodes visited, [1]=triangle tests, [2]=max stack depth,
  * [3]=rays; same results as bihrt_trace (outputs may be NULL). */

@@ -12,6 +12,13 @@ Workloads:
                      bihrt_trace_any(tmax = 1)  |  bihrt_intersect ANY with per-ray (0, 1), slot only
   atrium_diffuse     diffuse bounce list of the atrium at 1920x1080:
                      bihrt_trace  |  bihrt_intersect(0, inf) with all outputs
+Two-sided queries (BIHRT_INTERSECT_TWO_SIDED) against the one-sided query on the same list; their results differ by
+design, so these report each arm's hit fraction and check that every one-sided hit is a two-sided hit with t <= its t:
+  sphere_1m_primary_two_sided  the sphere_1m_primary list, all outputs: one-sided | two-sided
+  atrium_diffuse_two_sided     the atrium_diffuse list, all outputs: one-sided | two-sided
+  atrium_shadow_two_sided      the atrium_shadow list, ANY with per-ray (0, 1), slot only: one-sided | two-sided
+  sphere_1m_inside_two_sided   1 M-triangle sphere, 1920x1080 camera inside it, all outputs: two-sided only (a one-sided
+                               query sees nothing from there)
 
     python tools/bench_intersect.py --runs 5 --out bench_intersect.json
 """
@@ -86,12 +93,44 @@ def workloads(r):
         "trace": lambda x=diffuse: r.trace(x),
         "intersect_all": lambda x=bihrt.interval_rays(diffuse): r.intersect(x, outputs=ALL),
     }
+    yield "atrium_diffuse_two_sided", diffuse, {
+        "intersect_all": lambda x=bihrt.interval_rays(diffuse): r.intersect(x, outputs=ALL),
+        "intersect_all_two_sided": lambda x=bihrt.interval_rays(diffuse): r.intersect(x, two_sided=True, outputs=ALL),
+    }
+    yield "atrium_shadow_two_sided", shadow, {
+        "intersect_any_0_1_slot": lambda x=bihrt.interval_rays(shadow, 0.0, 1.0): r.intersect(x, any_hit=True, outputs=("slot",)),
+        "intersect_any_0_1_slot_two_sided": lambda x=bihrt.interval_rays(shadow, 0.0, 1.0):
+            r.intersect(x, any_hit=True, two_sided=True, outputs=("slot",)),
+    }
+
+    r.load_models(sphere).build()
+    yield "sphere_1m_primary_two_sided", prim6, {
+        "intersect_all": lambda x=bihrt.interval_rays(prim6): r.intersect(x, outputs=ALL),
+        "intersect_all_two_sided": lambda x=bihrt.interval_rays(prim6): r.intersect(x, two_sided=True, outputs=ALL),
+    }
+    inside = torch.from_numpy(scenes.camera_rays(scenes.pinhole_camera(origin=(0.03, -0.02, 0.05), half=0.9, aspect=w / h), w, h)).cuda()
+    yield "sphere_1m_inside_two_sided", inside, {
+        "intersect_all_two_sided": lambda x=bihrt.interval_rays(inside): r.intersect(x, two_sided=True, outputs=ALL),
+    }
+
+
+def hit_frac(v):
+    s = v["slot"] if isinstance(v, dict) else v[1] if isinstance(v, tuple) else v
+    return (s >= 0).float().mean().item()
 
 
 def agree(name, res):
-    """The arms report the same hits: closest-hit arms the same (t, slot, prim), occlusion arms the same hit / miss."""
+    """The arms report the same hits: closest-hit arms the same (t, slot, prim), occlusion arms the same hit / miss.
+    Two-sided workloads: every hit of the one-sided arm is a hit of the two-sided arm, with t <= (closest hit)."""
     import torch
     vals = list(res.values())
+    if name.endswith("_two_sided"):
+        if len(vals) == 1:
+            return True
+        one, two = vals
+        h1 = one["slot"] >= 0
+        ok = bool((two["slot"][h1] >= 0).all())
+        return ok and ("t" not in one or bool((two["t"][h1] <= one["t"][h1]).all()))
     if name == "atrium_shadow":
         a, b = vals
         return bool(torch.equal(a >= 0, b["slot"] >= 0))
@@ -125,12 +164,14 @@ def main():
                 ms[arm].append(time_ms(arms[arm], a.reps, a.warmup))
         results = {arm: arms[arm]() for arm in order}
         torch.cuda.synchronize()
-        s = {arm: {"ms": summary(ms[arm]), "mrays_s_median": n / (summary(ms[arm])["median"] * 1e-3) / 1e6} for arm in order}
+        s = {arm: {"ms": summary(ms[arm]), "mrays_s_median": n / (summary(ms[arm])["median"] * 1e-3) / 1e6,
+                   "hit_frac": hit_frac(results[arm])} for arm in order}
         base = s[order[0]]["ms"]["median"]
         for arm in order:
             s[arm]["time_vs_" + order[0]] = s[arm]["ms"]["median"] / base - 1.0
         res["workloads"][name] = {"rays": int(n), "arms": s, "same_hits": agree(name, results)}
-        print(name, json.dumps({k: (round(v["ms"]["median"], 4), round(v["ms"]["spread_frac"], 4), round(v["time_vs_" + order[0]], 4))
+        print(name, json.dumps({k: (round(v["ms"]["median"], 4), round(v["ms"]["spread_frac"], 4), round(v["time_vs_" + order[0]], 4),
+                                    round(v["mrays_s_median"], 1), round(v["hit_frac"], 4))
                                 for k, v in s.items()}), "same_hits", res["workloads"][name]["same_hits"], flush=True)
     r.close()
     txt = json.dumps(res, indent=1)
