@@ -55,6 +55,18 @@
 #ifndef TRACE_COVERAGE_EXIT
 #define TRACE_COVERAGE_EXIT 1
 #endif
+// Framebuffer renders (MODE 1) with lane groups (spp > 1) walk in one of nine copies of the node phase, chosen per warp after
+// every refill: one per ray octant, where every live lane's 1/d has the same sign on each axis, and the generic copy for a warp that mixes signs.  In
+// an octant copy a box's near and far distances are taken by compile-time sign, one FMNMX3 each, instead of the per-axis
+// min / max of the plane pair.  Exact: with lo <= hi (every child box) and a finite nonzero 1/d, round-to-nearest FMA is
+// monotone in the plane, so the sign selects the very distance min / max returns; a NaN 1/d (zero direction component)
+// gives two NaN distances, which the three-input min / max drop as the nested calls do, and 1/d == 0 gives two equal
+// ones.  Same intervals, same visits, same counters, same pixels.
+// 1 = on; 0 = the generic copy only (A/B builds: make variant EXTRA="-DTRACE_OCTANT_WALK=0").
+#ifndef TRACE_OCTANT_WALK
+#define TRACE_OCTANT_WALK 1
+#endif
+#define OCT_MIXED 8                         // the generic copy: lanes disagree on the sign of some axis
 #define BOX_EPS 2.384185791015625e-07f      /* 2^-22: the box tests' margin is this times (largest finite |o/d| + larger end of the ray's scene interval), one constant per ray */
 
 // (double)det < 0.000001 (R/src/CUDAKernels.cu:28)  <=>  det < 0x358637be as binary32; two-sided ray queries (MODE 4) test
@@ -160,12 +172,14 @@ template <int MODE, bool COUNTED, int WALK, bool Q>
 __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(TraceArgs a) {
     constexpr int STACK_DEPTH = Q ? STACK_DEPTH_QUALITY : STACK_DEPTH_PARITY;
     constexpr bool COVER = MODE == 1 && TRACE_COVERAGE_EXIT != 0;     // a sample ends at its first hit
+    constexpr bool OCTS = MODE == 1 && TRACE_OCTANT_WALK != 0;        // node phase specialised on the warp's ray octant
     constexpr bool LIST = MODE == 0 || MODE == 3 || MODE == 4;         // work items are rays of a list
     constexpr bool RANGE = MODE == 3 || MODE == 4;                     // rays carry [tmin, tmax]; hit records out
     constexpr bool TWO_SIDED = MODE == 4;                              // back faces accepted too
     // per-axis ray constants (origin, 1/dir), one row of 3 float2 per thread: 24-byte stride keeps a
     // half-warp's 64-bit accesses on distinct banks when the lanes agree on the axis
-    // per-thread ray record in shared memory, 10 words: (ox, 1/dx) (oy, 1/dy) (oz, 1/dz) dx dy dz tlo (MODE 3 and 4 only).  The node step picks
+    // per-thread ray record in shared memory, 10 words: (ox, 1/dx) (oy, 1/dy) (oz, 1/dz) dx dy dz, and word 9: tlo (MODE 3 and 4) or
+    // the warp's ray octant (MODE 1, TRACE_OCTANT_WALK: read once per node phase, so no register holds it through the walk).  The node step picks
     // (origin, 1/dir) of the node's axis with one 64-bit LDS (40-byte stride: a half-warp's accesses fall on distinct banks
     // when the lanes agree on the axis); the direction is only needed by the triangle test, so it lives here, not in registers.
     __shared__ __align__(16) float s_ray[TRACE_THREADS * 10];
@@ -499,6 +513,21 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 const uint32_t upd = __ballot_sync(FULL, new_thresh >= 0);
                 if (upd) thresh = __shfl_sync(FULL, new_thresh, __ffs(upd) - 1);
             }
+            if (OCTS) {
+                // the octant of the lanes with an item to walk, after every refill; a NaN or zero 1/d fits either sign.  Only
+                // warps of pixel sample groups (gshift > 0: at 16 spp a warp holds 2 pixels) take the octant copies: a 1 spp
+                // warp spans 8x4 pixels and is refilled lane by lane, and with the copies 1080p x 1 spp lost 11 % (1 M
+                // triangles) and 21 % (atrium) against the generic walk alone
+                int oct = OCT_MIXED;
+                if (gshift > 0) {
+                    const bool w = cur != NONE;
+                    const uint32_t xn = __ballot_sync(FULL, w && ix < 0.f), xp = __ballot_sync(FULL, w && ix > 0.f);
+                    const uint32_t yn = __ballot_sync(FULL, w && iy < 0.f), yp = __ballot_sync(FULL, w && iy > 0.f);
+                    const uint32_t zn = __ballot_sync(FULL, w && iz < 0.f), zp = __ballot_sync(FULL, w && iz > 0.f);
+                    if (!((xn && xp) || (yn && yp) || (zn && zp))) oct = (xn != 0) | (yn != 0) << 1 | (zn != 0) << 2;
+                }
+                my_ray[9] = __int_as_float(oct);
+            }
             if (__ballot_sync(FULL, cur != NONE || tracing) == 0 && exhausted &&
                 __ballot_sync(FULL, item != ~0ull) == 0) break;
         }
@@ -518,8 +547,14 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
             const float ax0 = __fmaf_rn((lx), ix, nx), ax1 = __fmaf_rn((hx), ix, nx);                       \
             const float ay0 = __fmaf_rn((ly), iy, ny), ay1 = __fmaf_rn((hy), iy, ny);                       \
             const float az0 = __fmaf_rn((lz), iz, nz), az1 = __fmaf_rn((hz), iz, nz);                       \
-            const float n_ = fmaxf(fmaxf(fminf(ax0, ax1), fminf(ay0, ay1)), fminf(az0, az1));               \
-            const float f_ = fminf(fminf(fmaxf(ax0, ax1), fmaxf(ay0, ay1)), fmaxf(az0, az1));               \
+            float n_, f_;                                                                                   \
+            if (OCT == OCT_MIXED) {                                                                         \
+                n_ = fmaxf(fmaxf(fminf(ax0, ax1), fminf(ay0, ay1)), fminf(az0, az1));                       \
+                f_ = fminf(fminf(fmaxf(ax0, ax1), fmaxf(ay0, ay1)), fmaxf(az0, az1));                       \
+            } else {                           /* 1/d < 0: the hi plane is the near one */                  \
+                n_ = fmax3((OCT & 1) ? ax1 : ax0, (OCT & 2) ? ay1 : ay0, (OCT & 4) ? az1 : az0);            \
+                f_ = fmin3((OCT & 1) ? ax0 : ax1, (OCT & 2) ? ay0 : ay1, (OCT & 4) ? az0 : az1);            \
+            }                                                                                               \
             (bn) = __fsub_rn(n_, bpad);                                                                     \
             (bf) = __fadd_rn(f_, bpad);                                                                     \
         } while (0)
@@ -539,77 +574,99 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 if (__uint_as_float(e.z) <= m) { cur = e.x; rMin = __uint_as_float(e.y); pMin = __uint_as_float(e.z); pMax = m; break; } \
             }                                                                                               \
         } while (0)
-        for (;;) {
-#pragma unroll (WALK > 0 ? WALK : 1)
-            for (int rep = 0; rep < steps_per_vote && (int)cur >= 0; rep++) {
-                // (origin, 1/dir) on this node's axis: one 64-bit LDS at ray_smem + axis * 8
-                float2 oi;
-                uint32_t ra;
-                asm("mad.lo.u32 %0, %1, 8, %2;" : "=r"(ra) : "r"(cur & 3u), "r"(ray_smem));
-                asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(oi.x), "=f"(oi.y) : "r"(ra));
-                // node address = base + index * 64, as one 32x32->64 multiply-add on the base pointer
-                const float4* np;
-                asm("mad.wide.u32 %0, %1, 64, %2;" : "=l"(np) : "r"(cur >> 2), "l"(nodes_b));
-                // Ray lists (MODE 0 and 3) fetch the 64-byte node as TWO 256-bit read-only loads (LDG.E.256, new on sm_100) instead of
-                // four 128-bit ones.  Measured (B200, Mrays/s, 128-bit -> 256-bit): diffuse bounce list on the atrium 2157 -> 2304
-                // (there every lane fetches its own node and the L1 tag stage is the busiest unit, 88 %), 1 M triangles 1080p x 1
-                // spp 6045 -> 6230, 10 M 3282 -> 3403; but coherent packets lose -- 4K x 16 spp 12014 -> 11833, atrium x 4 spp
-                // 6613 -> 6475 (the 8-register alignment of the destination costs two spills in a 64-register kernel).  So the
-                // camera modes keep the 128-bit loads.
-                float4 nd, b0, b1, b2;
-                if (LIST) {
-                    asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                        : "=f"(nd.x), "=f"(nd.y), "=f"(nd.z), "=f"(nd.w), "=f"(b0.x), "=f"(b0.y), "=f"(b0.z), "=f"(b0.w) : "l"(np));
-                    asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"
-                        : "=f"(b1.x), "=f"(b1.y), "=f"(b1.z), "=f"(b1.w), "=f"(b2.x), "=f"(b2.y), "=f"(b2.z), "=f"(b2.w) : "l"(np + 2));
-                } else { nd = __ldg(np); b0 = __ldg(np + 1); b1 = __ldg(np + 2); b2 = __ldg(np + 3); }
-                if (COUNTED) { nnodes++; const uint32_t am = __activemask(); wnode += (lane == __ffs(am) - 1); }
-                const uint32_t rl = __float_as_uint(nd.z), rr = __float_as_uint(nd.w);
-                const bool neg = oi.y < 0.f;                           // near = sign[axis], :286
-                const float t0 = __fmul_rn(__fsub_rn(nd.x, oi.x), oi.y);   // :288-289
-                const float t1 = __fmul_rn(__fsub_rn(nd.y, oi.x), oi.y);
-                const float tn = neg ? t1 : t0, tf = neg ? t0 : t1;
-                const uint32_t refn = neg ? rr : rl, reff = neg ? rl : rr;
-                // the children's boxes: parametric interval of the ray inside each (slab test on all three axes; min / max of
-                // the two plane distances per axis orders them whatever the sign of the direction, and drops the NaN of a
-                // zero direction component), widened by the ray's margin (bpad) so that rounding never culls a box the
-                // exact ray touches.  A child the ray misses is never fetched; a child that is entered gets the tighter interval.
-                float bnL, bfL, bnR, bfR;
-                BOX_SLAB(b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, bnL, bfL);
-                BOX_SLAB(b1.z, b1.w, b2.x, b2.y, b2.z, b2.w, bnR, bfR);
-                // (three-input min / max, FMNMX3: same NaN and signed-zero behaviour as the nested two-input calls they replace)
-                const float nLo = fmaxf(pMin, neg ? bnR : bnL), nHi = fmin3(pMax, tn, neg ? bfR : bfL);
-                const float fLo = fmax3(pMin, tf, neg ? bnL : bnR), fHi = fminf(pMax, neg ? bfL : bfR);
-                const bool go_near = (Q || rMin < tn) && (nLo <= nHi);   // reference's strict test (:292) + closed tight interval
-                const bool go_far = (fLo <= fHi);
-                // (the four cases as SELECTS instead of branch targets were measured: 4K x 16 spp 11997 -> 11259 Mrays/s, atrium -9 %:
-                // coherent lanes mostly agree on the case, and the selects cost every lane every time)
-                if (go_near && go_far) {
-                    // near before far, except a far LEAF next to a near NODE is tested first (:344-349)
-                    if ((int)refn >= 0 && (int)reff < 0) {
-                        STACK_PUSH(make_uint4(refn, __float_as_uint(rMin), __float_as_uint(nLo), __float_as_uint(nHi)));
-                        cur = reff; rMin = tf; pMin = fLo; pMax = fHi;
-                    } else {
-                        STACK_PUSH(make_uint4(reff, __float_as_uint(tf), __float_as_uint(fLo), __float_as_uint(fHi)));
-                        cur = refn; pMin = nLo; pMax = nHi;
-                    }
-                    // depth: a root-to-leaf path pushes at most one item per Morton bit, so sp <= 30 < STACK_DEPTH by
-                    // construction; the instrumented build reports the deepest stack (counters[2]) and refuses to run past
-                    // the array, -DBIHRT_DEBUG_STACK traps in every build
-                    if (COUNTED) { maxsp = max(maxsp, (uint32_t)sp); if (sp >= STACK_DEPTH) { maxsp = 0x7fffffffu; sp = STACK_DEPTH - 1; } }
 #ifdef BIHRT_DEBUG_STACK
-                    if (sp >= STACK_DEPTH) __trap();
+#define DEBUG_STACK_TRAP() do { if (sp >= STACK_DEPTH) __trap(); } while (0)
+#else
+#define DEBUG_STACK_TRAP() do { } while (0)
 #endif
-                } else if (go_near) { cur = refn; pMin = nLo; pMax = nHi; }
-                else if (go_far) { cur = reff; rMin = tf; pMin = fLo; pMax = fHi; }
-                else POP_VALID();
-            }
-            const uint32_t m_walk = __ballot_sync(FULL, (int)cur >= 0);
-            if (m_walk == 0) break;
-            if (vote) {
-                const uint32_t m_wait = __ballot_sync(FULL, cur + 1u > 0x80000000u);  // a leaf (negative, not NONE)
-                if (__popc(m_wait) > __popc(m_walk)) break;
-            }
+        // The node phase, expanded once per ray octant (OCT = its sign bits) and once generic (OCT_MIXED), see
+        // TRACE_OCTANT_WALK.  A macro rather than a function or lambda: the other modes then compile to the code they had.
+#define NODE_PHASE(OCT_)                                                                                           \
+        do {                                                                                                        \
+            constexpr int OCT = (OCT_);                                                                             \
+            for (;;) {                                                                                              \
+                _Pragma("unroll (WALK > 0 ? WALK : 1)")                                                             \
+                for (int rep = 0; rep < steps_per_vote && (int)cur >= 0; rep++) {                                   \
+                    /* (origin, 1/dir) on this node's axis: one 64-bit LDS at ray_smem + axis * 8 */                \
+                    float2 oi;                                                                                      \
+                    uint32_t ra;                                                                                    \
+                    asm("mad.lo.u32 %0, %1, 8, %2;" : "=r"(ra) : "r"(cur & 3u), "r"(ray_smem));                     \
+                    asm volatile("ld.shared.v2.f32 {%0, %1}, [%2];" : "=f"(oi.x), "=f"(oi.y) : "r"(ra));            \
+                    /* node address = base + index * 64, as one 32x32->64 multiply-add on the base pointer */       \
+                    const float4* np;                                                                               \
+                    asm("mad.wide.u32 %0, %1, 64, %2;" : "=l"(np) : "r"(cur >> 2), "l"(nodes_b));                   \
+                    /* Ray lists (MODE 0 and 3) fetch the 64-byte node as TWO 256-bit read-only loads (LDG.E.256, new on sm_100) instead of */ \
+                    /* four 128-bit ones.  Measured (B200, Mrays/s, 128-bit -> 256-bit): diffuse bounce list on the atrium 2157 -> 2304 */ \
+                    /* (there every lane fetches its own node and the L1 tag stage is the busiest unit, 88 %), 1 M triangles 1080p x 1 */ \
+                    /* spp 6045 -> 6230, 10 M 3282 -> 3403; but coherent packets lose -- 4K x 16 spp 12014 -> 11833, atrium x 4 spp */ \
+                    /* 6613 -> 6475 (the 8-register alignment of the destination costs two spills in a 64-register kernel).  So the */ \
+                    /* camera modes keep the 128-bit loads. */                                                      \
+                    float4 nd, b0, b1, b2;                                                                          \
+                    if (LIST) {                                                                                     \
+                        asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"                                  \
+                            : "=f"(nd.x), "=f"(nd.y), "=f"(nd.z), "=f"(nd.w), "=f"(b0.x), "=f"(b0.y), "=f"(b0.z), "=f"(b0.w) : "l"(np)); \
+                        asm("ld.global.nc.v8.f32 {%0,%1,%2,%3,%4,%5,%6,%7}, [%8];"                                  \
+                            : "=f"(b1.x), "=f"(b1.y), "=f"(b1.z), "=f"(b1.w), "=f"(b2.x), "=f"(b2.y), "=f"(b2.z), "=f"(b2.w) : "l"(np + 2)); \
+                    } else { nd = __ldg(np); b0 = __ldg(np + 1); b1 = __ldg(np + 2); b2 = __ldg(np + 3); }          \
+                    if (COUNTED) { nnodes++; const uint32_t am = __activemask(); wnode += (lane == __ffs(am) - 1); } \
+                    const uint32_t rl = __float_as_uint(nd.z), rr = __float_as_uint(nd.w);                          \
+                    const bool neg = oi.y < 0.f;                           /* near = sign[axis], :286 */            \
+                    const float t0 = __fmul_rn(__fsub_rn(nd.x, oi.x), oi.y);   /* :288-289 */                       \
+                    const float t1 = __fmul_rn(__fsub_rn(nd.y, oi.x), oi.y);                                        \
+                    const float tn = neg ? t1 : t0, tf = neg ? t0 : t1;                                             \
+                    const uint32_t refn = neg ? rr : rl, reff = neg ? rl : rr;                                      \
+                    /* the children's boxes: parametric interval of the ray inside each (slab test on all three axes; min / max of */ \
+                    /* the two plane distances per axis orders them whatever the sign of the direction -- an octant copy orders */ \
+                    /* them by the sign it knows -- and drops the NaN of a zero direction component), widened by the ray's margin */ \
+                    /* (bpad) so that rounding never culls a box the exact ray touches.  A child the ray misses is never fetched; a */ \
+                    /* child that is entered gets the tighter interval. */                                          \
+                    float bnL, bfL, bnR, bfR;                                                                       \
+                    BOX_SLAB(b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, bnL, bfL);                                         \
+                    BOX_SLAB(b1.z, b1.w, b2.x, b2.y, b2.z, b2.w, bnR, bfR);                                         \
+                    /* (three-input min / max, FMNMX3: same NaN and signed-zero behaviour as the nested two-input calls they replace) */ \
+                    const float nLo = fmaxf(pMin, neg ? bnR : bnL), nHi = fmin3(pMax, tn, neg ? bfR : bfL);         \
+                    const float fLo = fmax3(pMin, tf, neg ? bnL : bnR), fHi = fminf(pMax, neg ? bfL : bfR);         \
+                    const bool go_near = (Q || rMin < tn) && (nLo <= nHi);   /* reference's strict test (:292) + closed tight interval */ \
+                    const bool go_far = (fLo <= fHi);                                                               \
+                    /* (the four cases as SELECTS instead of branch targets were measured: 4K x 16 spp 11997 -> 11259 Mrays/s, atrium -9 %: */ \
+                    /* coherent lanes mostly agree on the case, and the selects cost every lane every time) */      \
+                    if (go_near && go_far) {                                                                        \
+                        /* near before far, except a far LEAF next to a near NODE is tested first (:344-349) */     \
+                        if ((int)refn >= 0 && (int)reff < 0) {                                                      \
+                            STACK_PUSH(make_uint4(refn, __float_as_uint(rMin), __float_as_uint(nLo), __float_as_uint(nHi))); \
+                            cur = reff; rMin = tf; pMin = fLo; pMax = fHi;                                          \
+                        } else {                                                                                    \
+                            STACK_PUSH(make_uint4(reff, __float_as_uint(tf), __float_as_uint(fLo), __float_as_uint(fHi))); \
+                            cur = refn; pMin = nLo; pMax = nHi;                                                     \
+                        }                                                                                           \
+                        /* depth: a root-to-leaf path pushes at most one item per Morton bit, so sp <= 30 < STACK_DEPTH by */ \
+                        /* construction; the instrumented build reports the deepest stack (counters[2]) and refuses to run past */ \
+                        /* the array, -DBIHRT_DEBUG_STACK traps in every build */                                   \
+                        if (COUNTED) { maxsp = max(maxsp, (uint32_t)sp); if (sp >= STACK_DEPTH) { maxsp = 0x7fffffffu; sp = STACK_DEPTH - 1; } } \
+                        DEBUG_STACK_TRAP();                                                                         \
+                    } else if (go_near) { cur = refn; pMin = nLo; pMax = nHi; }                                     \
+                    else if (go_far) { cur = reff; rMin = tf; pMin = fLo; pMax = fHi; }                             \
+                    else POP_VALID();                                                                               \
+                }                                                                                                   \
+                const uint32_t m_walk = __ballot_sync(FULL, (int)cur >= 0);                                         \
+                if (m_walk == 0) break;                                                                             \
+                if (vote) {                                                                                         \
+                    const uint32_t m_wait = __ballot_sync(FULL, cur + 1u > 0x80000000u);  /* a leaf (negative, not NONE) */ \
+                    if (__popc(m_wait) > __popc(m_walk)) break;                                                     \
+                }                                                                                                   \
+            }                                                                                                       \
+        } while (0)
+        if constexpr (!OCTS) NODE_PHASE(OCT_MIXED);       // (not instantiated in the other modes: their code stays as it was)
+        else switch (__float_as_int(my_ray[9])) {        // warp-uniform
+            case 0: NODE_PHASE(0); break;
+            case 1: NODE_PHASE(1); break;
+            case 2: NODE_PHASE(2); break;
+            case 3: NODE_PHASE(3); break;
+            case 4: NODE_PHASE(4); break;
+            case 5: NODE_PHASE(5); break;
+            case 6: NODE_PHASE(6); break;
+            case 7: NODE_PHASE(7); break;
+            default: NODE_PHASE(OCT_MIXED); break;
         }
         // ================= phase 2: the leaf this lane holds ===========================================
         if (cur + 1u > 0x80000000u) {
@@ -621,6 +678,8 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
             if (((LIST && a.any_hit) || COVER) && h.slot >= 0) { STACK_RESET(); cur = NONE; }
             else POP_VALID();
         }
+#undef NODE_PHASE
+#undef DEBUG_STACK_TRAP
 #undef POP_VALID
 #undef BOX_SLAB
 #undef STACK_RESET
