@@ -188,7 +188,6 @@ int bihrt_sync(bihrt_ctx* c) {
 int bihrt_set_option(bihrt_ctx* c, const char* name, int64_t v) {
     if (!c || !name) return BIHRT_ERR_INVALID;
     if (!strcmp(name, "trace_blocks_per_sm")) c->opt_trace_blocks_per_sm = (int)v;
-    else if (!strcmp(name, "trace_refill_threshold")) c->opt_refill_threshold = (int)std::max<int64_t>(1, std::min<int64_t>(32, v));
     else if (!strcmp(name, "build_graph")) c->opt_build_graph = (int)v;
     else if (!strcmp(name, "morton_bits")) {
         // 30: the reference's 10-bit grid (parity path).  63: quality mode (non-parity): 21 bits per axis, ties broken by position,
@@ -217,10 +216,6 @@ int bihrt_set_option(bihrt_ctx* c, const char* name, int64_t v) {
     else if (!strcmp(name, "trace_tile_sort_below")) c->opt_tile_sort_below = v;
     else if (!strcmp(name, "trace_tile_order")) { c->opt_tile_order = (int)v; for (auto& ts : c->tile_slots) ts.valid = false; }
     else if (!strcmp(name, "interleave_chunk")) c->opt_interleave_chunk = (int)std::max<int64_t>(1, std::min<int64_t>(1024, v));
-    else if (!strcmp(name, "trace_vote_wait")) c->opt_vote_wait = (int)v;
-    else if (!strcmp(name, "trace_vote_walk")) c->opt_vote_walk = (int)v;
-    else if (!strcmp(name, "trace_refill_incoherent")) c->opt_refill_incoherent = (int)std::max<int64_t>(1, std::min<int64_t>(32, v));
-    else if (!strcmp(name, "trace_chunk_items")) c->opt_chunk_items = (int)std::max<int64_t>(32, (v + 31) / 32 * 32);
     else return bihrt_fail(c, BIHRT_ERR_INVALID, "unknown option '%s'", name);
     return BIHRT_OK;
 }
@@ -481,9 +476,6 @@ static void base_args(bihrt_ctx* c, TraceArgs& a) {
     a.hdr = c->d_hdr; a.nodes = c->d_nodes; a.tris = c->d_tris;
     a.counters = c->d_counters; a.work = c->d_work;
     a.shard_index = 0; a.shard_count = 1; a.il_index = 0; a.il_count = 1;
-    a.refill_threshold = c->opt_refill_threshold; a.chunk_items = c->opt_chunk_items;
-    a.refill_incoherent = c->opt_refill_incoherent;
-    a.vote_wait = c->opt_vote_wait; a.vote_walk = c->opt_vote_walk;
     a.queues = c->opt_sm_queues;      // resolved per launch in bihrt_trace_launch (-1 = by ray count)
 }
 

@@ -139,10 +139,6 @@ struct bihrt_ctx {
 
     // options
     int opt_trace_blocks_per_sm = 0;   // 0 = occupancy query
-    int opt_refill_threshold = 32;
-    int opt_refill_incoherent = 32;   // (8 paid with the 16-byte nodes; with the children boxes an early refill of incoherent packets costs 5-10 %)
-    int opt_chunk_items = 32;
-    int opt_vote_wait = 1, opt_vote_walk = 4;
     int opt_lane_groups = -1; // samples of a pixel across lanes: -1 auto (as many as divide the sample count, <= 32), else 2^k
     int opt_interleave_chunk = 8;  // multi-GPU unit interleave: consecutive units per run (power of two; reduced until it divides a tile)
     int opt_tile_order = 1; // camera modes: start the tiles that were expensive in the previous frame first (1: launches of 64 k .. 48 M rays on scenes of >= 10 k triangles, 2: always, 0: never)
@@ -194,12 +190,7 @@ struct TraceArgs {
     uint32_t* fb;
     unsigned long long* counters; uint32_t* work;
     uint32_t* status_map;   // mapped host word for device-detected errors (tree of the wrong kind for this kernel)
-    int refill_threshold;   // lanes whose ray ended wait until this many are idle (or nobody is busy)
-    int refill_incoherent;  // threshold used instead for ray-list packets with mixed direction signs
-    int chunk_items;        // work items (rays / pixels) a warp takes from the global counter at once (queues == 1)
     int queues;             // > 1: one work queue per SM (tile t -> queue t % queues) with stealing
-    int vote_wait, vote_walk;   // vote_wait != 0: the node phase also ends when the waiting lanes outnumber the walking ones;
-                                // vote_walk: node steps a lane may take between two votes
     // MODE 3 and 4 (bihrt_intersect): rays with intervals instead of `rays`, and the hit record's other outputs (NULL = not wanted);
     // any_hit = BIHRT_INTERSECT_ANY (tmax comes with every ray)
     const bihrt_ray_interval* rays_iv;

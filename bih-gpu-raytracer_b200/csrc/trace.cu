@@ -7,8 +7,9 @@
 //     global atomic counter (or from per-SM queues, 1 spp launches of >= 16 M rays).  Camera modes: an item is a
 //     pixel's sample group -- the samples of a pixel sit in CONSECUTIVE LANES, the warp moves from sample to sample
 //     in lock step and a pixel is written once, as its final colour, by the lane that completes it (possibly into
-//     another GPU's framebuffer: bihrt_render_interleaved_to).  Ray lists: lanes whose ray ended are refilled once
-//     `refill_threshold` of them are idle; an option traces the list through a sort permutation (csrc/raysort.cu);
+//     another GPU's framebuffer: bihrt_render_interleaved_to).  A warp is refilled once every lane's ray has ended: each
+//     lane starts its item's next sample or takes a new item.  An option traces a ray list through a sort permutation
+//     (csrc/raysort.cu);
 //   * the tiles of a camera frame are traced in the order k_tile_order derived from the PREVIOUS launch of the same
 //     frame geometry (longest unit per tile, expensive tiles first): the launch is as long as its longest unit;
 //   * every lane walks its own ray with a short stack of 16-byte items (child reference + the three
@@ -29,7 +30,7 @@
 // Logical per-ray algorithm = oracle/bih_oracle.c:traverse_box (pruned traversal + children boxes that returns what
 // the reference's TraverseTree returns, including on axis-aligned flat geometry where the reference's
 // strict comparisons decide); framebuffer renders (MODE 1) end a sample at its first accepted triangle, which
-// tests/coverage_oracle.c restates as mode "first" (TRACE_COVERAGE_EXIT below).  Everything that decides a hit is IEEE binary32 without FMA contraction (explicit __f*_rn)
+// tests/coverage_oracle.c restates as mode "first" (COVER below).  Everything that decides a hit is IEEE binary32 without FMA contraction (explicit __f*_rn)
 // so t is bit-identical to the oracle's; the box distances are explicit FMAs, mirrored with fmaf in the oracle.
 #include "bihrt_internal.cuh"
 #include <float.h>
@@ -38,12 +39,10 @@
 #define STACK_DEPTH_PARITY  32  // <= 31 items: one per Morton bit on a root-to-leaf path, plus one
 #define STACK_DEPTH_QUALITY 96  // quality mode: 63 key bits + up to 29 position bits of tie-breaking
 #define NONE 0xFFFFFFFFu        // "no item": leaf bit set, never a valid slot
-#ifndef TRACE_THREADS
 #define TRACE_THREADS 128
-#endif
-#ifndef TRACE_MIN_BLOCKS
 #define TRACE_MIN_BLOCKS 8        // <= 64 registers per thread
-#endif
+// node steps a lane takes between two votes of the node phase (DESIGN §4: 2 / 3 / 6 steps measured -2 / -2 / 0 %)
+constexpr int NODE_STEPS = 4;
 
 // Framebuffer renders (MODE 1) as coverage queries: a pixel's colour depends only on WHETHER each sample hits, so a sample
 // ends at the first triangle it accepts -- inside the leaf and for the whole walk -- instead of searching on for the
@@ -51,10 +50,6 @@
 // test, same far-leaf-first order, same flat-geometry misses), so a sample hits exactly when the closest-hit search hits and
 // the image is the same bit for bit.  While a sample is alive every stacked item is still valid (pMin <= pMax <= FLT_MAX
 // held when it was pushed), so the pop needs no compare-and-drop loop.  MODE 0 and 2 keep the closest hit.
-// 1 = on; 0 = every mode searches for the closest hit (A/B builds: make variant EXTRA="-DTRACE_COVERAGE_EXIT=0").
-#ifndef TRACE_COVERAGE_EXIT
-#define TRACE_COVERAGE_EXIT 1
-#endif
 // Framebuffer renders (MODE 1) with lane groups (spp > 1) walk in one of nine copies of the node phase, chosen per warp after
 // every refill: one per ray octant, where every live lane's 1/d has the same sign on each axis, and the generic copy for a warp that mixes signs.  In
 // an octant copy a box's near and far distances are taken by compile-time sign, one FMNMX3 each, instead of the per-axis
@@ -62,10 +57,6 @@
 // monotone in the plane, so the sign selects the very distance min / max returns; a NaN 1/d (zero direction component)
 // gives two NaN distances, which the three-input min / max drop as the nested calls do, and 1/d == 0 gives two equal
 // ones.  Same intervals, same visits, same counters, same pixels.
-// 1 = on; 0 = the generic copy only (A/B builds: make variant EXTRA="-DTRACE_OCTANT_WALK=0").
-#ifndef TRACE_OCTANT_WALK
-#define TRACE_OCTANT_WALK 1
-#endif
 #define OCT_MIXED 8                         // the generic copy: lanes disagree on the sign of some axis
 #define BOX_EPS 2.384185791015625e-07f      /* 2^-22: the box tests' margin is this times (largest finite |o/d| + larger end of the ray's scene interval), one constant per ray */
 
@@ -163,23 +154,21 @@ __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, fl
 // at its register cap): when a hitting ray ends, its triangle is fetched again and u, v recomputed with the walk's own
 // arithmetic (mt_det / mt_u / mt_v).
 // ------------------------------------------------------------------------------------------
-// WALK > 0: the node phase takes exactly WALK steps between two votes and always votes (the shipped setting,
-// unrolled); WALK == 0: both come from the launch arguments (tuning / tests).
 // Q: the BIH is a quality-mode tree (63-bit keys, capped leaves; csrc/build.cu): long stack, and the closed tight-interval
 // tests alone decide -- the reference's extra strict test (rMin < t[near], :292), which the parity path reproduces together
 // with the hits it loses on axis-aligned geometry, is dropped.
-template <int MODE, bool COUNTED, int WALK, bool Q>
+template <int MODE, bool COUNTED, bool Q>
 __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(TraceArgs a) {
     constexpr int STACK_DEPTH = Q ? STACK_DEPTH_QUALITY : STACK_DEPTH_PARITY;
-    constexpr bool COVER = MODE == 1 && TRACE_COVERAGE_EXIT != 0;     // a sample ends at its first hit
-    constexpr bool OCTS = MODE == 1 && TRACE_OCTANT_WALK != 0;        // node phase specialised on the warp's ray octant
+    constexpr bool COVER = MODE == 1;                                  // a sample ends at its first hit
+    constexpr bool OCTS = MODE == 1;                                   // node phase specialised on the warp's ray octant
     constexpr bool LIST = MODE == 0 || MODE == 3 || MODE == 4;         // work items are rays of a list
     constexpr bool RANGE = MODE == 3 || MODE == 4;                     // rays carry [tmin, tmax]; hit records out
     constexpr bool TWO_SIDED = MODE == 4;                              // back faces accepted too
     // per-axis ray constants (origin, 1/dir), one row of 3 float2 per thread: 24-byte stride keeps a
     // half-warp's 64-bit accesses on distinct banks when the lanes agree on the axis
     // per-thread ray record in shared memory, 10 words: (ox, 1/dx) (oy, 1/dy) (oz, 1/dz) dx dy dz, and word 9: tlo (MODE 3 and 4) or
-    // the warp's ray octant (MODE 1, TRACE_OCTANT_WALK: read once per node phase, so no register holds it through the walk).  The node step picks
+    // the warp's ray octant (MODE 1: read once per node phase, so no register holds it through the walk).  The node step picks
     // (origin, 1/dir) of the node's axis with one 64-bit LDS (40-byte stride: a half-warp's accesses fall on distinct banks
     // when the lanes agree on the axis); the direction is only needed by the triangle test, so it lives here, not in registers.
     __shared__ __align__(16) float s_ray[TRACE_THREADS * 10];
@@ -239,27 +228,18 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
 #define STACK_PUSH(item) do { stack[sp] = (item); sp++; } while (0)
 #define STACK_POP(e) do { sp--; (e) = stack[sp]; } while (0)
     const uint32_t root_ref = BIH_REF_NODE(0, a.hdr->root_axis);
-    const bool vote = WALK > 0 || a.vote_wait != 0;
-    int thresh = a.refill_threshold;          // lanes that must be idle before a partial refill (warp-uniform)
     // colours with a pixel's samples in several lanes: the warp moves from sample to sample in lock step, so the lanes
     // of a pixel hold its complete hit count when they finish and the pixel is written once, without atomics
     const bool direct = MODE == 1 && gshift > 0 && !(a.flags & BIHRT_RENDER_COUNTS);
-    if (direct) thresh = 32;
-    const int steps_per_vote = WALK > 0 ? WALK : (a.vote_walk > 0 ? a.vote_walk : 1);
     const uint32_t ray_smem = (uint32_t)__cvta_generic_to_shared(my_ray);
 
     for (;;) {
-        // ================= refill: lanes whose ray has ended record it and get the next one ========
-        // A lane whose ray ended moves on to the next SAMPLE of its own pixel as soon as `refill_threshold`
-        // lanes can (same pixel, so the warp stays coherent); new ITEMS are only handed out when the whole
-        // warp has drained (MODE 0 ray lists: items are single rays, so those are handed out at the
-        // threshold too).  Lanes that have nothing left park until then.
-        const uint32_t idle = __ballot_sync(FULL, cur == NONE);
-        const uint32_t busy = ~idle;
-        // (the count of lanes that could go on is only needed for a partial refill; every term before it is warp-uniform)
-        if (idle && (busy == 0 || (thresh < 32 && __popc(__ballot_sync(FULL, cur == NONE && (tracing || item != ~0ull || LIST))) >= thresh))) {
-            const bool fresh = (busy == 0);          // the warp starts a new packet together
-            int new_thresh = -1;
+        // ================= refill: once the whole warp has drained, every lane records its ray and gets the next one ========
+        // A lane moves on to the next SAMPLE of its own item, or takes a new ITEM when its item is done, so the warp starts
+        // each packet together.  (Refilling the idle lanes of a warp that is still walking was measured as a loss with the
+        // children boxes: DESIGN §4.)  Lanes that have nothing left park until the launch ends.
+        const uint32_t busy = ~__ballot_sync(FULL, cur == NONE);
+        if (busy == 0) {
             bool want_item = false, finishing = false;
             if (cur == NONE) {
                 if (tracing) {                                   // record the ray that just ended
@@ -330,20 +310,19 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 }
             }
             // the packet that just drained: its duration is the cost of its tile for the next frame's order
-            if (!LIST && fresh && a.tile_cost && unit_tile != 0xFFFFFFFFu) {
+            if (!LIST && a.tile_cost && unit_tile != 0xFFFFFFFFu) {
                 if (lane == 0) atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
                 unit_tile = 0xFFFFFFFFu;
             }
             // hand out new items (warp-uniform control flow)
             uint32_t want = __ballot_sync(FULL, want_item);
-            if (!LIST && busy != 0) want = 0;                 // pixels: wait for the whole warp
             while (want && !exhausted) {
                 if (pool_next >= pool_end) {
                     // Work comes in units of 32 items, grouped in tiles of 32 units (a 32x32-pixel tile / 1024
                     // rays).  With per-SM queues (a.queues > 1) tile t belongs to queue t % queues and every
                     // warp of an SM drains its own SM's queue first, so the warps resident on one SM walk the
                     // same one or two tiles and share nodes and triangles in L1; an SM that runs dry steals
-                    // from the others.  a.queues == 1 is one global counter (chunk_items per fetch).
+                    // from the others.  a.queues == 1 is one global counter (one unit per fetch).
                     uint64_t base = ~0ull;
                     uint32_t got = 0;
                     if (lane == 0) {
@@ -352,8 +331,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                         // pixel keeps all its samples -- and their lane grouping -- on one GPU
                         const uint32_t ilc = (uint32_t)a.il_count, ili = (uint32_t)a.il_index, ics = (uint32_t)a.il_cshift;
                         if (a.queues <= 1) {
-                            const uint32_t chunk = ilc > 1 ? 32u : (uint32_t)a.chunk_items;
-                            const uint64_t fetched = atomicAdd(a.work, chunk); got = chunk;
+                            const uint64_t fetched = atomicAdd(a.work, 32u); got = 32;
                             const uint64_t lu = fetched >> 5;          // this rank's unit -> the frame's unit (runs of 2^il_cshift units)
                             base = ilc > 1 ? ((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u))) << 5 : fetched;
                             if (base >= total) base = ~0ull;
@@ -456,15 +434,6 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 nx = -__fmul_rn(ox, ix); ny = -__fmul_rn(oy, iy); nz = -__fmul_rn(oz, iz);
                 bpad = __fmul_rn(BOX_EPS, fmaxf(fmaxf(fabsf(nx) <= FLT_MAX ? fabsf(nx) : 0.f, fabsf(ny) <= FLT_MAX ? fabsf(ny) : 0.f),
                                                 fabsf(nz) <= FLT_MAX ? fabsf(nz) : 0.f));
-                if (LIST && fresh) {
-                    // ray lists: a packet whose directions disagree in sign is incoherent (diffuse bounces);
-                    // there, lanes that finish early are worth refilling before the whole packet has drained
-                    const uint32_t m = __activemask();
-                    const uint32_t bx = __ballot_sync(m, ix < 0.f), by = __ballot_sync(m, iy < 0.f), bz = __ballot_sync(m, iz < 0.f);
-                    // (one mixed axis is common in coherent packets that straddle a sign boundary; two are not)
-                    const bool mixed = ((bx != 0 && bx != m) + (by != 0 && by != m) + (bz != 0 && bz != m)) >= 2;
-                    new_thresh = mixed ? min(a.refill_threshold, a.refill_incoherent) : a.refill_threshold;
-                }
                 *reinterpret_cast<float2*>(my_ray) = make_float2(ox, ix); *reinterpret_cast<float2*>(my_ray + 2) = make_float2(oy, iy);
                 *reinterpret_cast<float2*>(my_ray + 4) = make_float2(oz, iz); *reinterpret_cast<float2*>(my_ray + 6) = make_float2(dx, dy);
                 my_ray[8] = dz;
@@ -508,10 +477,6 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                     if (nu == 1) { cur = BIH_REF_LEAFREF(0); pMin = -FLT_MAX; pMax = FLT_MAX; }
                     else if (pMin <= pMax) cur = root_ref;          // box behind the origin: nothing to walk
                 }
-            }
-            if (LIST) {
-                const uint32_t upd = __ballot_sync(FULL, new_thresh >= 0);
-                if (upd) thresh = __shfl_sync(FULL, new_thresh, __ffs(upd) - 1);
             }
             if (OCTS) {
                 // the octant of the lanes with an item to walk, after every refill; a NaN or zero 1/d fits either sign.  Only
@@ -579,14 +544,14 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
 #else
 #define DEBUG_STACK_TRAP() do { } while (0)
 #endif
-        // The node phase, expanded once per ray octant (OCT = its sign bits) and once generic (OCT_MIXED), see
-        // TRACE_OCTANT_WALK.  A macro rather than a function or lambda: the other modes then compile to the code they had.
+        // The node phase, expanded once per ray octant (OCT = its sign bits) and once generic (OCT_MIXED), see the
+        // octant copies at the head of this file.  A macro rather than a function or lambda: the other modes then compile to the code they had.
 #define NODE_PHASE(OCT_)                                                                                           \
         do {                                                                                                        \
             constexpr int OCT = (OCT_);                                                                             \
             for (;;) {                                                                                              \
-                _Pragma("unroll (WALK > 0 ? WALK : 1)")                                                             \
-                for (int rep = 0; rep < steps_per_vote && (int)cur >= 0; rep++) {                                   \
+                _Pragma("unroll (NODE_STEPS)")                                                                      \
+                for (int rep = 0; rep < NODE_STEPS && (int)cur >= 0; rep++) {                                       \
                     /* (origin, 1/dir) on this node's axis: one 64-bit LDS at ray_smem + axis * 8 */                \
                     float2 oi;                                                                                      \
                     uint32_t ra;                                                                                    \
@@ -650,10 +615,8 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 }                                                                                                   \
                 const uint32_t m_walk = __ballot_sync(FULL, (int)cur >= 0);                                         \
                 if (m_walk == 0) break;                                                                             \
-                if (vote) {                                                                                         \
-                    const uint32_t m_wait = __ballot_sync(FULL, cur + 1u > 0x80000000u);  /* a leaf (negative, not NONE) */ \
-                    if (__popc(m_wait) > __popc(m_walk)) break;                                                     \
-                }                                                                                                   \
+                const uint32_t m_wait = __ballot_sync(FULL, cur + 1u > 0x80000000u);  /* a leaf (negative, not NONE) */ \
+                if (__popc(m_wait) > __popc(m_walk)) break;                                                         \
             }                                                                                                       \
         } while (0)
         if constexpr (!OCTS) NODE_PHASE(OCT_MIXED);       // (not instantiated in the other modes: their code stays as it was)
@@ -806,21 +769,33 @@ int bihrt_resolve_launch(bihrt_ctx* c, uint32_t* fb, int npix, int spp) {
     return BIHRT_OK;
 }
 
-#ifndef TRACE_WALK
-#define TRACE_WALK 4
-#endif
-template <int MODE, bool COUNTED, int WALK, bool Q = false>
+template <int MODE, bool COUNTED, bool Q>
 static int launch(bihrt_ctx* c, const TraceArgs& a) {
     int per_sm = c->opt_trace_blocks_per_sm;
     if (per_sm <= 0) {
-        BIHRT_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_trace<MODE, COUNTED, WALK, Q>, TRACE_THREADS, 0));
+        BIHRT_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_trace<MODE, COUNTED, Q>, TRACE_THREADS, 0));
         if (per_sm < 1) per_sm = 1;
     }
     BIHRT_CUDA(c, cudaMemsetAsync(a.work, 0, 4 * 1024, c->stream));
-    k_trace<MODE, COUNTED, WALK, Q><<<c->sm_count * per_sm, TRACE_THREADS, 0, c->stream>>>(a);
+    k_trace<MODE, COUNTED, Q><<<c->sm_count * per_sm, TRACE_THREADS, 0, c->stream>>>(a);
     c->kernel_launches += 1;
     BIHRT_CUDA(c, cudaGetLastError());
     return BIHRT_OK;
+}
+
+template <bool Q>
+static int launch_mode(bihrt_ctx* c, const TraceArgs& a, int mode, bool counted) {
+    switch (mode * 2 + (counted ? 1 : 0)) {
+        case 0: return launch<0, false, Q>(c, a);
+        case 1: return launch<0, true, Q>(c, a);
+        case 2: return launch<1, false, Q>(c, a);
+        case 3: return launch<1, true, Q>(c, a);
+        case 4: return launch<2, false, Q>(c, a);
+        case 5: return launch<2, true, Q>(c, a);
+        case 6: return launch<3, false, Q>(c, a);
+        case 8: return launch<4, false, Q>(c, a);
+        default: return bihrt_fail(c, BIHRT_ERR_INVALID, "bad trace mode %d", mode);
+    }
 }
 
 int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a_in, int mode, bool counted) {
@@ -885,35 +860,8 @@ int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a_in, int mode, bool count
             a.tile_order = slot->valid ? slot->order : nullptr;
         }
     }
-    const bool shipped = a.vote_wait != 0 && a.vote_walk == TRACE_WALK;    // the unrolled instantiation
-    int rc = BIHRT_ERR_INVALID;
     a.status_map = c->d_status_map;
-    if (c->built_quality) {
-        // quality-mode tree: the shipped schedule only (TRACE_WALK node steps per vote); the instrumented build walks one step per vote
-        TraceArgs q = a; q.vote_wait = 1; q.vote_walk = 1;
-        switch (mode * 2 + (counted ? 1 : 0)) {
-            case 0: rc = launch<0, false, TRACE_WALK, true>(c, a); break;
-            case 1: rc = launch<0, true, 0, true>(c, q); break;
-            case 2: rc = launch<1, false, TRACE_WALK, true>(c, a); break;
-            case 3: rc = launch<1, true, 0, true>(c, q); break;
-            case 4: rc = launch<2, false, TRACE_WALK, true>(c, a); break;
-            case 5: rc = launch<2, true, 0, true>(c, q); break;
-            case 6: rc = launch<3, false, TRACE_WALK, true>(c, a); break;
-            case 8: rc = launch<4, false, TRACE_WALK, true>(c, a); break;
-            default: return bihrt_fail(c, BIHRT_ERR_INVALID, "bad trace mode %d", mode);
-        }
-    } else
-    switch (mode * 2 + (counted ? 1 : 0)) {
-        case 0: rc = shipped ? launch<0, false, TRACE_WALK>(c, a) : launch<0, false, 0>(c, a); break;
-        case 1: rc = launch<0, true, 0>(c, a); break;
-        case 2: rc = shipped ? launch<1, false, TRACE_WALK>(c, a) : launch<1, false, 0>(c, a); break;
-        case 3: rc = launch<1, true, 0>(c, a); break;
-        case 4: rc = shipped ? launch<2, false, TRACE_WALK>(c, a) : launch<2, false, 0>(c, a); break;
-        case 5: rc = launch<2, true, 0>(c, a); break;
-        case 6: rc = shipped ? launch<3, false, TRACE_WALK>(c, a) : launch<3, false, 0>(c, a); break;
-        case 8: rc = shipped ? launch<4, false, TRACE_WALK>(c, a) : launch<4, false, 0>(c, a); break;
-        default: return bihrt_fail(c, BIHRT_ERR_INVALID, "bad trace mode %d", mode);
-    }
+    int rc = c->built_quality ? launch_mode<true>(c, a, mode, counted) : launch_mode<false>(c, a, mode, counted);
     if (rc == BIHRT_OK && slot) {
         if ((rc = bihrt_tile_order_launch(c, slot->cost, slot->order, ntiles, rays < c->opt_tile_sort_below)) == BIHRT_OK) slot->valid = true;
     }

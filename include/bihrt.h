@@ -116,7 +116,7 @@ BIHRT_API const char* bihrt_last_error(const bihrt_ctx* ctx);                   
 BIHRT_API int         bihrt_set_stream(bihrt_ctx* ctx, void* cuda_stream);
 BIHRT_API int         bihrt_get_stream(bihrt_ctx* ctx, void** cuda_stream);     /* the cudaStream_t the context launches on */
 BIHRT_API int         bihrt_sync(bihrt_ctx* ctx);                               /* replaces the cudaDeviceSynchronize after each step, R/src/Renderer.cpp:428-503 */
-/* Options (DESIGN.md has the full list of tuning knobs).  The two that change WHAT is built:
+/* Options (INTEGRATION.md, "Options", lists them all; an unknown name is BIHRT_ERR_INVALID).  The two that change WHAT is built:
  *   "morton_bits" 30 (default): the reference's 10-bit grid per axis, R/src/Renderer.cpp:116-136 -- the parity path, bit-exact tree.
  *                 63: QUALITY MODE, not a parity path (SURVEY.md 8(f) f4): 21 bits per axis, ties broken by sorted position,
  *                 every subtree of at most "leaf_cap" (default 4, 1..64) triangles collapsed into one leaf.  Hits equal brute force

@@ -116,6 +116,11 @@ def test_error_codes(renderer):
     with pytest.raises(bihrt.BihrtError) as e:
         renderer.load_models("/nonexistent/file.obj")
     assert e.value.code == -5
+    # retired trace-scheduling options are unknown names now (BIHRT_ERR_INVALID)
+    for name in ("trace_refill_threshold", "trace_refill_incoherent", "trace_chunk_items", "trace_vote_wait", "trace_vote_walk"):
+        with pytest.raises(bihrt.BihrtError) as e:
+            renderer.set_option(name, 32)
+        assert e.value.code == -1 and "unknown option" in str(e.value)
 
 
 def test_refit_keeps_hits_correct(renderer, scenes, oracle):

@@ -1,7 +1,7 @@
 """Framebuffer renders are coverage queries: a sample ends at the first triangle it accepts.
 
 A pixel's colour (and the hit counts of the sharded renders) depends only on WHETHER each sample hits, so the framebuffer
-kernel (csrc/trace.cu, MODE 1, TRACE_COVERAGE_EXIT) stops a sample's walk at its first accepted triangle instead of
+kernel (csrc/trace.cu, MODE 1, COVER) stops a sample's walk at its first accepted triangle instead of
 searching on for the closest one.  tests/coverage_oracle.c restates that walk on the CPU (mode "first": the oracle's
 "box" traversal with that one exit).  The CPU tests check that "first" hits exactly where "ref" and "box" hit and never
 does more work than "box"; the GPU tests pin render_counted's counters to "first" exactly, and every framebuffer path to

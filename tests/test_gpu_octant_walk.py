@@ -1,4 +1,4 @@
-"""Framebuffer renders walk in the copy of the node phase that matches the warp's ray octant (csrc/trace.cu, TRACE_OCTANT_WALK).
+"""Framebuffer renders walk in the copy of the node phase that matches the warp's ray octant (csrc/trace.cu, OCTS).
 
 A warp whose live lanes agree on the sign of 1/d on every axis takes each box's near and far planes by compile-time sign;
 a warp that mixes signs takes the generic copy.  Every case below must give the image of the closest-hit oracle bit for

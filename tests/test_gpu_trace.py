@@ -189,13 +189,11 @@ def test_bih_blob_roundtrip(scenes, oracle):
     a.close(); b.close()
 
 
-@pytest.mark.parametrize("opts", [
-    {"trace_vote_wait": 0}, {"trace_vote_wait": 1, "trace_vote_walk": 1}, {"trace_vote_walk": 8}, {"trace_sm_queues": 1}, {"trace_sm_queues": 0},
-    {"trace_refill_threshold": 4, "trace_chunk_items": 96},
-    {"trace_refill_threshold": 1, "trace_vote_wait": 2, "trace_vote_walk": 1, "trace_blocks_per_sm": 3}])
+@pytest.mark.parametrize("opts", [{"trace_sm_queues": 1}, {"trace_sm_queues": 0}, {"trace_blocks_per_sm": 3}],
+                         ids=["sm_queues_1", "sm_queues_0", "blocks_per_sm_3"])
 def test_scheduling_variants_do_not_change_results(renderer, scenes, oracle, opts):
-    """Warp-scheduling knobs (early exit of the node phase, lane refill, occupancy) reorder work
-    inside a warp but never a ray's own sequence of leaf tests: hits must stay bit-identical."""
+    """Scheduling options (per-SM work queues, occupancy) reorder work across warps but never a ray's own
+    sequence of leaf tests: hits must stay bit-identical."""
     for tri, cam, w, h in ((scenes.atrium(0.2), scenes.atrium_camera(), 320, 180),
                            (scenes.displaced_sphere(187), scenes.pinhole_camera(), 480, 270)):
         ob = oracle.Bih(tri)

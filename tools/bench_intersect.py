@@ -63,6 +63,22 @@ def time_ms(fn, reps, warmup):
     return e0.elapsed_time(e1) / reps
 
 
+def sphere_primary_list(w, h):
+    """Pixel-centre primary rays of the 1 M-triangle sphere's camera, as a device list."""
+    import torch
+    from bihrt import scenes
+    return torch.from_numpy(scenes.camera_rays(scenes.pinhole_camera(aspect=w / h), w, h)).cuda()
+
+
+def atrium_lists(r, w, h):
+    """Shadow and diffuse bounce lists (bihrt_secondary_rays) of the atrium camera; the atrium must be built in r."""
+    from bihrt import scenes
+    cam = scenes.atrium_camera(w / h)
+    shadow, _ = r.secondary_rays(cam, w, h, spp=1, kind="shadow", light=(0.1, 0.8, -0.2))
+    diffuse, _ = r.secondary_rays(cam, w, h, spp=1, kind="diffuse")
+    return shadow.contiguous(), diffuse.contiguous()
+
+
 def workloads(r):
     """Yields (name, device rays, {arm: call}) one workload at a time (each loads its scene into r)."""
     import torch
@@ -72,7 +88,7 @@ def workloads(r):
 
     sphere = scenes.displaced_sphere(scenes.SPHERE_NSEG["1m"])
     r.load_models(sphere).build()
-    prim6 = torch.from_numpy(scenes.camera_rays(scenes.pinhole_camera(aspect=w / h), w, h)).cuda()
+    prim6 = sphere_primary_list(w, h)
     yield "sphere_1m_primary", prim6, {
         "trace": lambda x=prim6: r.trace(x),
         "intersect_t_slot_prim": lambda x=bihrt.interval_rays(prim6): r.intersect(x, outputs=("t", "slot", "prim")),
@@ -80,15 +96,11 @@ def workloads(r):
     }
 
     r.load_models(scenes.atrium()).build()
-    cam = scenes.atrium_camera(w / h)
-    shadow, _ = r.secondary_rays(cam, w, h, spp=1, kind="shadow", light=(0.1, 0.8, -0.2))
-    shadow = shadow.contiguous()
+    shadow, diffuse = atrium_lists(r, w, h)
     yield "atrium_shadow", shadow, {
         "trace_any_tmax1": lambda x=shadow: r.trace_any(x, tmax=1.0),
         "intersect_any_0_1_slot": lambda x=bihrt.interval_rays(shadow, 0.0, 1.0): r.intersect(x, any_hit=True, outputs=("slot",)),
     }
-    diffuse, _ = r.secondary_rays(cam, w, h, spp=1, kind="diffuse")
-    diffuse = diffuse.contiguous()
     yield "atrium_diffuse", diffuse, {
         "trace": lambda x=diffuse: r.trace(x),
         "intersect_all": lambda x=bihrt.interval_rays(diffuse): r.intersect(x, outputs=ALL),

@@ -34,9 +34,4 @@ run("a centre ray x32", np.repeat(rays[(h // 2) * w + w // 2:(h // 2) * w + w //
 run("a miss ray x32", np.repeat(rays[0:1], 32, axis=0))
 run("row 208 (480 rays)", rays[208 * w:209 * w])
 run("whole 480x270 frame as a list", rays)
-r.set_option("trace_refill_threshold", 8)
-run("whole frame, refill threshold 8", rays)
-r.set_option("trace_refill_threshold", 1)
-run("whole frame, refill threshold 1", rays)
-r.set_option("trace_refill_threshold", 32)
 print("render 480x270: %.3f ms" % timed(lambda: r.render(cam, w, h, spp=1)))

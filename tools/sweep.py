@@ -16,7 +16,7 @@ tri = scenes.atrium() if a.scene == "atrium" else scenes.displaced_sphere(scenes
 cam = scenes.atrium_camera(a.w / a.h) if a.scene == "atrium" else scenes.pinhole_camera(aspect=a.w / a.h)
 r.load_models(torch.from_numpy(tri).cuda()).build(); r.sync()
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-DEFAULTS = {"trace_vote_wait": 1, "trace_vote_walk": 3, "trace_refill_threshold": 32, "trace_chunk_items": 32, "trace_blocks_per_sm": 0, "trace_sm_queues": -1, "trace_lane_groups": -1}
+DEFAULTS = {"trace_blocks_per_sm": 0, "trace_sm_queues": -1, "trace_lane_groups": -1}
 for oset in a.sets.split(";"):
     opts = dict(DEFAULTS)
     for kv in filter(None, oset.split(",")):

@@ -1,4 +1,4 @@
-"""Primary rays traced as a device ray LIST (MODE 0) vs generated in the kernel (MODE 1): does lane refill pay?"""
+"""Primary rays traced as a device ray LIST (MODE 0) vs generated in the kernel (MODE 1), in row-major and in tile order."""
 import os, sys
 import numpy as np, torch
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -31,6 +31,4 @@ print("render (MODE 1)          %.0f Mr/s" % bench(lambda: r.render(cam, W, H, s
 for name, rr in (("row-major list", rays), ("8x4-tiled list", rays[order])):
     d = torch.from_numpy(np.ascontiguousarray(rr)).cuda(); n = len(rr)
     ot = torch.empty(n, device="cuda"); oi = torch.empty(n, dtype=torch.int32, device="cuda")
-    for th in (32, 16, 8, 4):
-        r.set_option("trace_refill_threshold", th)
-        print("%-16s refill %2d   %.0f Mr/s" % (name, th, bench(lambda: r.trace(d, t=ot, slot=oi, prim=oi), n)))
+    print("%-24s %.0f Mr/s" % (name, bench(lambda: r.trace(d, t=ot, slot=oi, prim=oi), n)))

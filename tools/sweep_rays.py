@@ -22,7 +22,7 @@ rng = np.random.default_rng(1984); dd = rng.normal(size=P.shape); dd /= np.linal
 light = np.array([0.0, 0.8, 0.0], np.float32)
 batches = {"shadow": np.concatenate([P, light - P], 1), "bounce": np.concatenate([P, dd], 1)}
 flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")
-DEF = {"trace_vote_wait": 1, "trace_vote_walk": 3, "trace_refill_threshold": 32, "trace_chunk_items": 32, "trace_sm_queues": -1}
+DEF = {"trace_sm_queues": -1}
 for oset in a.sets.split(";"):
     o = dict(DEF)
     for kv in filter(None, oset.split(",")):

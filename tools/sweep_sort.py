@@ -32,9 +32,7 @@ for scene in ("atrium", "1m"):
             print("  %-8s nodes/ray %.1f tris/ray %.1f hit %.2f" % (kind, cnt["nodes"] / n, cnt["tris"] / n, float((_s >= 0).float().mean())), flush=True)
             for srt in (0, 1):
                 r.set_option("trace_sort_rays", srt)
-                for thr in ((32, 8), (32, 32)) if kind == "diffuse" else ((32, 8),):
-                    r.set_option("trace_refill_threshold", thr[0]); r.set_option("trace_refill_incoherent", thr[1])
-                    r.trace(db, t=ot, slot=os_, prim=os_); r.sync()
-                    ms = timed(lambda: r.trace(db, t=ot, slot=os_, prim=os_))
-                    print("  %-8s sort=%d refill=%s: %.3f ms %.0f Mrays/s (%d rays)" % (kind, srt, thr, ms, n / ms / 1e3, n), flush=True)
-            r.set_option("trace_sort_rays", 0); r.set_option("trace_refill_threshold", 32); r.set_option("trace_refill_incoherent", 8)
+                r.trace(db, t=ot, slot=os_, prim=os_); r.sync()
+                ms = timed(lambda: r.trace(db, t=ot, slot=os_, prim=os_))
+                print("  %-8s sort=%d: %.3f ms %.0f Mrays/s (%d rays)" % (kind, srt, ms, n / ms / 1e3, n), flush=True)
+            r.set_option("trace_sort_rays", 0)
