@@ -20,9 +20,11 @@ from test_gpu_coverage import trace_first  # noqa: F401  (fixture: the coverage 
 pytestmark = pytest.mark.gpu
 
 
-def check_frame(renderer, oracle, trace_first, ob, cam, w, h, spp, jitter, groups=(-1,)):  # noqa: F811
+def check_frame(renderer, oracle, trace_first, ob, cam, w, h, spp, jitter, groups=(-1,), qtree=None):  # noqa: F811
+    """The renderer's tree is the parity tree of oracle.Bih `ob`, or with `qtree` (test_gpu_quality_walk.QTree) that quality
+    tree: the image is then held to its closest walk and render_counted to its 'first' walk."""
     rays = oracle.camera_rays(cam, w, h, spp=spp, jitter=jitter, seed=1984)
-    _, s0, _ = ob.trace(rays, "ref")
+    s0 = ob.trace(rays, "ref")[1] if qtree is None else qtree.walk(rays)[1]
     exp = oracle.pack_framebuffer(s0, w, h, spp).reshape(h, w)
     what = "%dx%d spp %d jitter %s" % (w, h, spp, jitter)
     try:
@@ -32,7 +34,7 @@ def check_frame(renderer, oracle, trace_first, ob, cam, w, h, spp, jitter, group
             np.testing.assert_array_equal(fb, exp, err_msg="%s groups %d" % (what, g))
     finally:
         renderer.set_option("trace_lane_groups", -1)
-    _, _, _, cf = trace_first(ob, rays)
+    cf = trace_first(ob, rays)[3] if qtree is None else qtree.walk(rays, "first")[3]
     cnt = renderer.render_counted(cam, w, h, spp=spp, seed=1984, jitter=jitter)
     assert cnt["rays"] == len(rays)
     assert (cnt["nodes"], cnt["tris"], cnt["max_stack"]) == (cf["nodes"], cf["tris"], cf["max_stack"]), what
