@@ -30,7 +30,7 @@
 // Logical per-ray algorithm = oracle/bih_oracle.c:traverse_box (pruned traversal + children boxes that returns what
 // the reference's TraverseTree returns, including on axis-aligned flat geometry where the reference's
 // strict comparisons decide); framebuffer renders (MODE 1) end a sample at its first accepted triangle, which
-// tests/coverage_oracle.c restates as mode "first" (COVER below).  Everything that decides a hit is IEEE binary32 without FMA contraction (explicit __f*_rn)
+// tests/walk_oracle.c restates as exit "first" (COVER below).  Everything that decides a hit is IEEE binary32 without FMA contraction (explicit __f*_rn)
 // so t is bit-identical to the oracle's; the box distances are explicit FMAs, mirrored with fmaf in the oracle.
 #include "bihrt_internal.cuh"
 #include <float.h>

@@ -2,54 +2,24 @@
 
 A pixel's colour (and the hit counts of the sharded renders) depends only on WHETHER each sample hits, so the framebuffer
 kernel (csrc/trace.cu, MODE 1, COVER) stops a sample's walk at its first accepted triangle instead of
-searching on for the closest one.  tests/coverage_oracle.c restates that walk on the CPU (mode "first": the oracle's
-"box" traversal with that one exit).  The CPU tests check that "first" hits exactly where "ref" and "box" hit and never
-does more work than "box"; the GPU tests pin render_counted's counters to "first" exactly, and every framebuffer path to
-the image of the closest-hit oracle.
+searching on for the closest one.  tests/walk_oracle.c restates that walk on the CPU (exit "first" of its walk on the
+parity tree: the oracle's "box" traversal with that one exit).  The CPU tests check that "first" hits exactly where "ref"
+and "box" hit and never does more work than "box"; the GPU tests pin render_counted's counters to "first" exactly, and
+every framebuffer path to the image of the closest-hit oracle.
 """
-import ctypes as C
-import os
-import subprocess
-
 import numpy as np
 import pytest
 
 from test_gpu_golden_scenes import SCENES as GOLDEN
-
-HERE = os.path.dirname(os.path.abspath(__file__))
-ORACLE_DIR = os.path.join(os.path.dirname(HERE), "oracle")
+from walk_oracle import degenerate_rays, tree  # noqa: F401  (tree: fixture)
 
 
-@pytest.fixture(scope="session")
-def trace_first(tmp_path_factory):
-    """Builds tests/coverage_oracle.c (the oracle's source plus mode "first") into a temporary directory; returns
-    trace_first(bih, rays) -> t, slot, prim, counters, with the arguments and results of oracle.Bih.trace."""
-    out = str(tmp_path_factory.mktemp("coverage_oracle") / "libcoverage_oracle.so")
-    cc = "/usr/bin/gcc" if os.access("/usr/bin/gcc", os.X_OK) else "gcc"
-    subprocess.check_call([cc, "-O2", "-ffp-contract=off", "-fopenmp", "-fPIC", "-fvisibility=hidden", "-std=c11",
-                           "-shared", "-I" + ORACLE_DIR, "-o", out, os.path.join(HERE, "coverage_oracle.c"), "-lm"])
-    lib = C.CDLL(out)
-
-    def _p(a):
-        return a.ctypes.data_as(C.c_void_p)
-
-    def run(ob, rays6):
-        rays6 = np.ascontiguousarray(rays6, dtype=np.float32).reshape(-1, 6)
-        nr = rays6.shape[0]
-        t, slot, prim = np.empty(nr, np.float32), np.empty(nr, np.int32), np.empty(nr, np.int32)
-        cnt = np.zeros(3, np.uint64)
-        keep = [np.ascontiguousarray(x) for x in (ob.tris_idx, ob.cnt, ob.first, ob.clip, ob.axis, ob.is_leaf, ob.children)]
-        lib.orc_trace_first(_p(ob.tri9), C.c_int64(ob.n), C.c_int64(ob.nu), *[_p(k) for k in keep], _p(ob.scene_lo),
-                            _p(ob.scene_hi), _p(rays6), C.c_int64(nr), _p(t), _p(slot), _p(prim), _p(cnt), C.c_int(0))
-        return t, slot, prim, {"nodes": int(cnt[0]), "tris": int(cnt[1]), "max_stack": int(cnt[2])}
-    return run
-
-
-def assert_first_covers_like_ref(trace_first, ob, rays):
+def assert_first_covers_like_ref(tree, ob, rays):
     """'first' hits exactly where 'ref' and 'box' hit, with no more nodes or triangle tests than 'box'; returns the counters."""
     t0, s0, _ = ob.trace(rays, "ref")
     t3, s3, _, c3 = ob.trace(rays, "box", want_counters=True)
-    tf, sf, pf, cf = trace_first(ob, rays)
+    f = tree(ob).walk(rays, "first")
+    tf, sf, pf, cf = f["t"], f["slot"], f["prim"], f["counters"]
     np.testing.assert_array_equal(sf >= 0, s0 >= 0)
     np.testing.assert_array_equal(sf >= 0, s3 >= 0)
     hit = sf >= 0
@@ -62,36 +32,23 @@ def assert_first_covers_like_ref(trace_first, ob, rays):
 # ------------------------------------------------------------------------------------------------ CPU: the restatement
 
 @pytest.mark.parametrize("name", list(GOLDEN))
-def test_first_hit_equals_reference_on_golden_scenes(oracle, scenes, trace_first, name):
+def test_first_hit_equals_reference_on_golden_scenes(oracle, scenes, tree, name):
     tri, cam, w, h = GOLDEN[name](scenes)
     ob = oracle.Bih(tri)
     for spp, jitter in ((1, False), (2, True)):
         rays = oracle.camera_rays(cam, w, h, spp=spp, jitter=jitter, seed=1984)
-        s0, cf, c3 = assert_first_covers_like_ref(trace_first, ob, rays)
+        s0, cf, c3 = assert_first_covers_like_ref(tree, ob, rays)
         if 0.02 < (s0 >= 0).mean():
             assert cf["tris"] < c3["tris"]                 # the exit does remove work wherever rays hit
 
 
-def test_first_hit_equals_reference_on_degenerate_rays(oracle, scenes, trace_first):
+def test_first_hit_equals_reference_on_degenerate_rays(oracle, scenes, tree):
     """Zero direction components, origins on grid planes and on the scene box, diagonal directions (the rays of
     test_oracle_semantics' box-mode regression test), and origins far from the scene."""
-    tri = np.concatenate([scenes.cornell_box(), scenes.displaced_sphere(24) * 0.3])
-    ob = oracle.Bih(tri)
     rng = np.random.default_rng(7)
-    n = 20000
-    o = rng.uniform(-1.2, 1.2, (n, 3)).astype(np.float32)
-    d = rng.normal(size=(n, 3)).astype(np.float32)
-    which = rng.integers(0, 7, n)
-    d[which == 0, 0] = 0.0
-    d[which == 1, 1] = 0.0
-    d[which == 2, 2] = 0.0
-    d[which == 3, :2] = 0.0
-    o[which == 4] = np.round(o[which == 4] * 4) / 4
-    d[which == 5] = np.sign(d[which == 5])
-    o[which == 6, 0] = -1.0
-    d[(which == 3) & (d[:, 2] == 0), 2] = 1.0
-    rays = np.concatenate([o, d], 1).astype(np.float32)
-    s0, _, _ = assert_first_covers_like_ref(trace_first, ob, rays)
+    tri, rays = degenerate_rays(scenes, rng)
+    ob = oracle.Bih(tri)
+    s0, _, _ = assert_first_covers_like_ref(tree, ob, rays)
     assert (s0 >= 0).sum() > 1000
     tri = scenes.displaced_sphere(48)
     ob = oracle.Bih(tri)
@@ -99,10 +56,10 @@ def test_first_hit_equals_reference_on_degenerate_rays(oracle, scenes, trace_fir
         target = rng.uniform(-0.6, 0.6, (4000, 3))
         dirs = rng.normal(size=(4000, 3)); dirs /= np.linalg.norm(dirs, axis=1, keepdims=True)
         rays = np.concatenate([(target - dirs * dist).astype(np.float32), dirs.astype(np.float32)], 1).astype(np.float32)
-        assert_first_covers_like_ref(trace_first, ob, rays)
+        assert_first_covers_like_ref(tree, ob, rays)
 
 
-def test_first_hit_keeps_the_reference_misses_on_flat_geometry(oracle, scenes, trace_first):
+def test_first_hit_keeps_the_reference_misses_on_flat_geometry(oracle, scenes, tree):
     """On axis-aligned walls the reference's strict test skips leaves brute force would test (it hits a farther wall);
     the coverage walk takes the same decisions up to its first hit, so it hits exactly where the reference does."""
     for tri, cam, w, h in ((scenes.cornell_box(), scenes.cornell_camera(), 256, 256),
@@ -110,7 +67,7 @@ def test_first_hit_keeps_the_reference_misses_on_flat_geometry(oracle, scenes, t
         ob = oracle.Bih(tri)
         for spp, jitter in ((1, False), (2, True)):
             rays = oracle.camera_rays(cam, w, h, spp=spp, jitter=jitter)
-            s0, _, _ = assert_first_covers_like_ref(trace_first, ob, rays)
+            s0, _, _ = assert_first_covers_like_ref(tree, ob, rays)
             if len(tri) < 100:
                 _, s2, _ = ob.trace(rays, "brute")
                 assert (s0 != s2).sum() > 0                  # the strict test decides on these rays
@@ -127,15 +84,15 @@ COUNTED_CASES = {
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", list(COUNTED_CASES))
-def test_render_counters_equal_first_hit_oracle(renderer, scenes, oracle, trace_first, name):
+def test_render_counters_equal_first_hit_oracle(renderer, scenes, oracle, tree, name):
     """render_counted (the instrumented framebuffer kernel) visits exactly the nodes and triangles of mode 'first'."""
     tri, cam, w, h = COUNTED_CASES[name](scenes)
-    ob = oracle.Bih(tri)
+    pt = tree(oracle.Bih(tri))
     renderer.load_models(tri).build()
     for spp in (1, 3, 4, 16):
         for jitter in (False, True):
             rays = oracle.camera_rays(cam, w, h, spp=spp, jitter=jitter, seed=1984)
-            _, _, _, cf = trace_first(ob, rays)
+            cf = pt.walk(rays, "first")["counters"]
             cnt = renderer.render_counted(cam, w, h, spp=spp, seed=1984, jitter=jitter)
             assert cnt["rays"] == len(rays)
             assert (cnt["nodes"], cnt["tris"], cnt["max_stack"]) == (cf["nodes"], cf["tris"], cf["max_stack"]), (spp, jitter)

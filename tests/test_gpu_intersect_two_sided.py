@@ -1,10 +1,10 @@
 """Double-sided ray queries: bihrt_intersect with BIHRT_INTERSECT_TWO_SIDED (csrc/trace.cu MODE 4).
 
 The flag changes one thing: a triangle is a candidate when !(|det| < 1e-6) instead of !(det < 1e-6).
-tests/range_oracle_two_sided.c restates it on the CPU next to the one-sided restatement of tests/range_oracle.c, which it
-includes unchanged.  The CPU tests tie the two-sided restatement to two-sided brute force, to the one-sided query
-(superset of hits, t never larger, front-face records unchanged) and to an independent numpy Moller-Trumbore; the GPU tests
-hold the kernel to the restatement bit for bit in all six outputs.
+tests/walk_oracle.c restates it on the CPU: the one-sided query's walk and brute force with its two_sided flag set.  The CPU
+tests tie the two-sided restatement to two-sided brute force, to the one-sided query (superset of hits, t never larger,
+front-face records unchanged) and to an independent numpy Moller-Trumbore; the GPU tests hold the kernel to the restatement
+bit for bit in all six outputs.
 
 Tie tolerance: where two different walks are compared, primitive ids may differ on exact-t ties on at most ID_MISMATCH_MAX
 of the rays (as in test_gpu_intersect.py); such comparisons are marked "tie tolerance".  Coplanar tolerance (quality-mode
@@ -13,80 +13,17 @@ the walk may report the one an ulp further; checked as exactly that class, on at
 other comparison is exact.
 """
 import ctypes as C
-import os
-import subprocess
 
 import numpy as np
 import pytest
 
 from test_gpu_golden_scenes import SCENES as GOLDEN
-from test_gpu_intersect import (FLT_MAX, ID_MISMATCH_MAX, OUTS, assert_records_equal, assorted_intervals, bits,
-                                degenerate_rays, rays8_of)
+from test_gpu_intersect import ID_MISMATCH_MAX
+from walk_oracle import (FLT_MAX, OUTS, assert_records_equal, assorted_intervals, bits, degenerate_rays, mt, rays8,
+                         tree)  # noqa: F401  (tree: fixture)
 
-HERE = os.path.dirname(os.path.abspath(__file__))
-ORACLE_DIR = os.path.join(os.path.dirname(HERE), "oracle")
 DET_EPS = np.array([0x358637be], np.uint32).view(np.float32)[0]
 INSIDE_CAMERA = dict(origin=(0.03, -0.02, 0.05), half=0.9, aspect=1.0)      # inside the displaced sphere, looking +z
-
-
-@pytest.fixture(scope="session")
-def trace_range(tmp_path_factory):
-    """Builds tests/range_oracle_two_sided.c (with tests/range_oracle.c inside) into a temporary directory; returns
-    trace_range(bih, rays8, mode="box"|"brute", any_hit=False, two_sided=True) -> {t, u, v, slot, prim, ng, counters}:
-    orc_trace_range_two_sided, or range_oracle.c's one-sided orc_trace_range for two_sided=False."""
-    out = str(tmp_path_factory.mktemp("range_oracle_two_sided") / "librange_oracle_two_sided.so")
-    cc = "/usr/bin/gcc" if os.access("/usr/bin/gcc", os.X_OK) else "gcc"
-    subprocess.check_call([cc, "-O2", "-ffp-contract=off", "-fopenmp", "-fPIC", "-fvisibility=hidden", "-std=c11",
-                           "-shared", "-I" + ORACLE_DIR, "-o", out, os.path.join(HERE, "range_oracle_two_sided.c"), "-lm"])
-    lib = C.CDLL(out)
-
-    def _p(a):
-        return a.ctypes.data_as(C.c_void_p)
-
-    def run(ob, rays8, mode="box", any_hit=False, two_sided=True):
-        rays8 = np.ascontiguousarray(rays8, dtype=np.float32).reshape(-1, 8)
-        nr = rays8.shape[0]
-        r = {"t": np.empty(nr, np.float32), "u": np.empty(nr, np.float32), "v": np.empty(nr, np.float32),
-             "slot": np.empty(nr, np.int32), "prim": np.empty(nr, np.int32), "ng": np.empty((nr, 3), np.float32)}
-        cnt = np.zeros(3, np.uint64)
-        keep = [np.ascontiguousarray(x) for x in (ob.tris_idx, ob.cnt, ob.first, ob.clip, ob.axis, ob.is_leaf, ob.children)]
-        fn = lib.orc_trace_range_two_sided if two_sided else lib.orc_trace_range
-        fn(C.c_int({"box": 0, "brute": 1}[mode]), C.c_uint32(1 if any_hit else 0), _p(ob.tri9),
-           C.c_int64(ob.n), C.c_int64(ob.nu), *[_p(k) for k in keep], _p(ob.scene_lo), _p(ob.scene_hi),
-           _p(rays8), C.c_int64(nr), _p(r["t"]), _p(r["u"]), _p(r["v"]), _p(r["slot"]), _p(r["prim"]),
-           _p(r["ng"]), _p(cnt), C.c_int(0))
-        r["counters"] = {"nodes": int(cnt[0]), "tris": int(cnt[1]), "max_stack": int(cnt[2])}
-        return r
-    return run
-
-
-def mt_two_sided(tri9, prim, rays6):
-    """Moller-Trumbore of ray i against triangle prim[i] in numpy binary32 with the non-culling det test |det| >= 1e-6, the
-    reference's operation order otherwise (R/src/CUDAKernels.cu:17-50): returns ok, det, t, u, v."""
-    f = np.float32
-    tri = tri9.reshape(-1, 9)[prim].astype(f)
-    v0, v1, v2 = tri[:, 0:3], tri[:, 3:6], tri[:, 6:9]
-    o, d = rays6[:, 0:3].astype(f), rays6[:, 3:6].astype(f)
-    e1, e2 = v1 - v0, v2 - v0
-
-    def cross(a, b):
-        return np.stack([a[:, 1] * b[:, 2] - b[:, 1] * a[:, 2], a[:, 2] * b[:, 0] - b[:, 2] * a[:, 0],
-                         a[:, 0] * b[:, 1] - b[:, 0] * a[:, 1]], 1)
-
-    def dot(a, b):
-        return (a[:, 0] * b[:, 0] + a[:, 1] * b[:, 1]) + a[:, 2] * b[:, 2]
-    p = cross(d, e2)
-    det = dot(e1, p)
-    ok = np.abs(det.astype(np.float64)) >= 1e-6
-    with np.errstate(all="ignore"):
-        inv = (1.0 / det.astype(np.float64)).astype(f)
-        tv = o - v0
-        u = dot(tv, p) * inv
-        q = cross(tv, e1)
-        v = dot(d, q) * inv
-        t = dot(e2, q) * inv
-    ok &= ~((u < 0) | (u > 1) | (v < 0) | ((u + v) > 1))
-    return ok, det, t, u, v
 
 
 def check_against_one_sided(one, two, tri, rays6):
@@ -97,7 +34,7 @@ def check_against_one_sided(one, two, tri, rays6):
     h1, h2 = one["slot"] >= 0, two["slot"] >= 0
     assert np.all(h2[h1]), "a one-sided hit is missing from the two-sided query"
     assert np.all(two["t"][h1] <= one["t"][h1])
-    ok, det, t, u, v = mt_two_sided(tri, two["prim"][h2], rays6[h2])
+    ok, det, t, u, v = mt(tri, two["prim"][h2], rays6[h2], two_sided=True)
     assert ok.all()
     np.testing.assert_array_equal(bits(two["t"][h2]), bits(t))
     np.testing.assert_array_equal(bits(two["u"][h2]), bits(u))
@@ -121,7 +58,7 @@ def assert_coplanar_near_ties(tri9, rays6, got, want, sel):
     both triangles are true hits that lie in one plane (coincident surfaces, such as the bottom of a box resting on a floor)."""
     tg, tw = got["t"][sel], want["t"][sel]
     assert np.all(bits(tg).astype(np.int64) - bits(tw).astype(np.int64) == 1)
-    ok, _, t, _, _ = mt_two_sided(tri9, got["prim"][sel], rays6[sel])
+    ok, _, t, _, _ = mt(tri9, got["prim"][sel], rays6[sel], two_sided=True)
     assert ok.all()
     np.testing.assert_array_equal(bits(t), bits(tg))
     T = tri9.reshape(-1, 9).astype(np.float64)
@@ -157,16 +94,16 @@ def test_det_threshold_is_symmetric():
 
 
 @pytest.mark.parametrize("which", ["sphere187", "sphere361", "soup", "inside_sphere"])
-def test_two_sided_box_equals_brute_force(oracle, scenes, trace_range, which):
+def test_two_sided_box_equals_brute_force(oracle, scenes, tree, which):
     if which == "inside_sphere":
         tri, rays = inside_sphere(scenes, oracle, 160, 160)
     else:
         tri, cam, w, h = GOLDEN[which](scenes)
         rays = oracle.camera_rays(cam, w, h)
-    ob = oracle.Bih(tri)
-    tmin, tmax = assorted_intervals(trace_range(ob, rays8_of(rays))["t"], seed=31)
-    for r8 in (rays8_of(rays), rays8_of(rays, tmin, tmax)):
-        a, b = trace_range(ob, r8, "box"), trace_range(ob, r8, "brute")
+    pt = tree(oracle.Bih(tri))
+    tmin, tmax = assorted_intervals(pt.walk(rays8(rays), two_sided=True)["t"], seed=31)
+    for r8 in (rays8(rays), rays8(rays, tmin, tmax)):
+        a, b = pt.walk(r8, two_sided=True), pt.brute(r8, two_sided=True)
         np.testing.assert_array_equal(bits(a["t"]), bits(b["t"]))
         bad = a["prim"] != b["prim"]
         assert bad.sum() <= max(1, ID_MISMATCH_MAX * len(rays))        # tie tolerance (exact-t ties only)
@@ -182,40 +119,41 @@ def scene_and_rays(name, oracle, scenes):
 
 
 @pytest.mark.parametrize("name", list(GOLDEN) + ["degenerate"])
-def test_two_sided_against_one_sided(oracle, scenes, trace_range, name):
+def test_two_sided_against_one_sided(oracle, scenes, tree, name):
     tri, rays = scene_and_rays(name, oracle, scenes)
     ob = oracle.Bih(tri)
+    pt = tree(ob)
     t3, _, _ = ob.trace(rays, "box")
     tmin, tmax = assorted_intervals(t3, seed=13)
-    for r8 in (rays8_of(rays), rays8_of(rays, tmin, tmax)):
-        one, two = trace_range(ob, r8, two_sided=False), trace_range(ob, r8)
+    for r8 in (rays8(rays), rays8(rays, tmin, tmax)):
+        one, two = pt.walk(r8), pt.walk(r8, two_sided=True)
         check_against_one_sided(one, two, tri, rays)
-        a = trace_range(ob, r8, any_hit=True)
+        a = pt.walk(r8, "any", two_sided=True)
         hit = a["slot"] >= 0
         np.testing.assert_array_equal(hit, two["slot"] >= 0)
         assert np.all(a["t"][hit] >= two["t"][hit])
-        ok, _, t, _, _ = mt_two_sided(tri, a["prim"][hit], rays[hit])
+        ok, _, t, _, _ = mt(tri, a["prim"][hit], rays[hit], two_sided=True)
         assert ok.all()
         np.testing.assert_array_equal(bits(a["t"][hit]), bits(t))
 
 
-def test_camera_inside_closed_mesh_sees_back_faces(oracle, scenes, trace_range):
+def test_camera_inside_closed_mesh_sees_back_faces(oracle, scenes, tree):
     tri, rays = inside_sphere(scenes, oracle, 160, 160)
-    ob = oracle.Bih(tri)
-    r8 = rays8_of(rays)
-    one, two = trace_range(ob, r8, two_sided=False), trace_range(ob, r8)
+    pt = tree(oracle.Bih(tri))
+    r8 = rays8(rays)
+    one, two = pt.walk(r8), pt.walk(r8, two_sided=True)
     assert (one["slot"] >= 0).sum() == 0
     hit = two["slot"] >= 0
     assert hit.mean() > 0.995                    # Moller-Trumbore is not watertight: a ray through an edge may miss both
     assert np.all((rays[hit, 3:].astype(np.float64) * two["ng"][hit]).sum(1) > 0)
 
 
-def test_peeling_visits_entry_and_exit_layers(oracle, scenes, trace_range):
+def test_peeling_visits_entry_and_exit_layers(oracle, scenes, tree):
     """A closed mesh seen from outside: two-sided peeling (tmin = the last t) yields front, back, front, back, ... at
     increasing t, the same sequence as brute force; one-sided peeling sees only the entries."""
     behind = (scenes.displaced_sphere(40).reshape(-1, 3) * 0.6 + np.float32([0.2, 0.1, 2.4])).reshape(-1, 9)
     tri = np.ascontiguousarray(np.concatenate([scenes.displaced_sphere(48), behind]), np.float32)
-    ob = oracle.Bih(tri)
+    pt = tree(oracle.Bih(tri))
     rays = oracle.camera_rays(scenes.pinhole_camera(origin=(0.1, 0.2, -2.5), aspect=1.0), 72, 72)
     seqs = {}
     for mode in ("box", "brute"):
@@ -224,7 +162,7 @@ def test_peeling_visits_entry_and_exit_layers(oracle, scenes, trace_range):
         seq = [[] for _ in range(len(rays))]
         while alive.any():
             idx = np.nonzero(alive)[0]
-            r = trace_range(ob, rays8_of(rays[idx], tmin[idx], np.inf), mode)
+            r = (pt.walk if mode == "box" else pt.brute)(rays8(rays[idx], tmin[idx], np.inf), two_sided=True)
             hit = r["slot"] >= 0
             side = (rays[idx[hit], 3:].astype(np.float64) * r["ng"][hit]).sum(1)
             for i, t, sd in zip(idx[hit], r["t"][hit], side):
@@ -239,7 +177,7 @@ def test_peeling_visits_entry_and_exit_layers(oracle, scenes, trace_range):
                             for s in seqs["box"]])
     assert (depth >= 2).mean() > 0.2 and depth.max() >= 4
     assert alternating[depth > 0].mean() > 0.99                # a ray through a shared edge may skip one layer
-    one = trace_range(ob, rays8_of(rays), two_sided=False)
+    one = pt.walk(rays8(rays))
     entries = np.array([s[0][0] if s else FLT_MAX for s in seqs["box"]], np.float32)
     np.testing.assert_array_equal(bits(one["t"][alternating]), bits(entries[alternating]))
 
@@ -256,20 +194,21 @@ def gpu_intersect_host_and_device(renderer, r8, any_hit, outputs=OUTS):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("name", list(GOLDEN))
-def test_two_sided_intersect_equals_restatement_bit_for_bit(renderer, oracle, scenes, trace_range, name):
+def test_two_sided_intersect_equals_restatement_bit_for_bit(renderer, oracle, scenes, tree, name):
     tri, cam, w, h = GOLDEN[name](scenes)
     ob = oracle.Bih(tri)
+    pt = tree(ob)
     rays = oracle.camera_rays(cam, w, h)
     renderer.load_models(tri).build()
     t3, _, _ = ob.trace(rays, "box")
     tmin, tmax = assorted_intervals(t3, seed=19)
-    r8 = rays8_of(rays, tmin, tmax)
+    r8 = rays8(rays, tmin, tmax)
     for any_hit in (False, True):
-        want = trace_range(ob, r8, any_hit=any_hit)
+        want = pt.walk(r8, "any" if any_hit else "closest", two_sided=True)
         host, dev = gpu_intersect_host_and_device(renderer, r8, any_hit)
         assert_records_equal(host, want, msg="host any=%s" % any_hit)
         assert_records_equal(dev, want, msg="device any=%s" % any_hit)
-    want = trace_range(ob, r8)
+    want = pt.walk(r8, two_sided=True)
     for subset in (("t",), ("slot", "prim"), ("u", "v"), ("ng",), ("t", "ng", "prim")):
         host, dev = gpu_intersect_host_and_device(renderer, r8, False, subset)
         assert set(host) == set(subset) == set(dev)
@@ -279,15 +218,15 @@ def test_two_sided_intersect_equals_restatement_bit_for_bit(renderer, oracle, sc
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("which", ["inside_sphere", "inside_box"])
-def test_camera_inside_equals_restatement(renderer, oracle, scenes, trace_range, which):
+def test_camera_inside_equals_restatement(renderer, oracle, scenes, tree, which):
     """Inside the displaced sphere, and inside an axis-aligned box(n=8) with outward faces: the parity tree equals the
     restatement bit for bit (on the box that includes the reference's flat-geometry misses)."""
     tri, rays = (inside_sphere if which == "inside_sphere" else inside_box)(scenes, oracle, 320, 180)
-    ob = oracle.Bih(tri)
+    pt = tree(oracle.Bih(tri))
     renderer.load_models(tri).build()
-    r8 = rays8_of(rays)
+    r8 = rays8(rays)
     for any_hit in (False, True):
-        want = trace_range(ob, r8, any_hit=any_hit)
+        want = pt.walk(r8, "any" if any_hit else "closest", two_sided=True)
         host, dev = gpu_intersect_host_and_device(renderer, r8, any_hit)
         assert_records_equal(host, want, msg="host any=%s" % any_hit)
         assert_records_equal(dev, want, msg="device any=%s" % any_hit)
@@ -303,19 +242,19 @@ def test_camera_inside_equals_restatement(renderer, oracle, scenes, trace_range,
 @pytest.mark.gpu
 @pytest.mark.parametrize("cap", [1, 4, 16])
 @pytest.mark.parametrize("name", ["cornell", "sphere187", "atrium", "soup", "inside_box"])
-def test_quality_mode_equals_two_sided_brute_force(renderer, oracle, scenes, trace_range, name, cap):
+def test_quality_mode_equals_two_sided_brute_force(renderer, oracle, scenes, tree, name, cap):
     if name == "inside_box":
         tri, rays = inside_box(scenes, oracle, 160, 160)
     else:
         tri, cam, w, h = GOLDEN[name](scenes)
         rays = oracle.camera_rays(cam, w, h)
-    ob = oracle.Bih(tri)
+    pt = tree(oracle.Bih(tri))
     renderer.set_option("morton_bits", 63)
     renderer.set_option("leaf_cap", cap)
     renderer.load_models(tri).build()
-    tmin, tmax = assorted_intervals(trace_range(ob, rays8_of(rays), "brute")["t"], seed=29)
-    for r8 in (rays8_of(rays), rays8_of(rays, tmin, tmax)):
-        want = trace_range(ob, r8, "brute")
+    tmin, tmax = assorted_intervals(pt.brute(rays8(rays), two_sided=True)["t"], seed=29)
+    for r8 in (rays8(rays), rays8(rays, tmin, tmax)):
+        want = pt.brute(r8, two_sided=True)
         got = renderer.intersect(r8, two_sided=True)
         near = bits(got["t"]) != bits(want["t"])
         assert near.sum() <= max(1, ID_MISMATCH_MAX * len(rays))       # coplanar tolerance
@@ -350,13 +289,13 @@ def test_atrium_bounce_list_against_one_sided(renderer, scenes):
 
 
 @pytest.mark.gpu
-def test_per_sm_queue_launch(renderer, oracle, scenes, trace_range):
+def test_per_sm_queue_launch(renderer, oracle, scenes, tree):
     """2^24 + 1 two-sided rays, many starting inside the sphere: the launch takes the per-SM work queues.  A sample of the
     rays equals the restatement bit for bit; all of them keep the properties against the one-sided query."""
     import torch
     from bihrt import interval_rays
     tri = scenes.displaced_sphere(187)
-    ob = oracle.Bih(tri)
+    pt = tree(oracle.Bih(tri))
     renderer.load_models(tri).build()
     g = torch.Generator(device="cuda").manual_seed(7)
     n = (1 << 24) + 1
@@ -370,7 +309,7 @@ def test_per_sm_queue_launch(renderer, oracle, scenes, trace_range):
     front = check_against_one_sided(one, two, tri, rays_np)
     assert (~front).sum() > n // 10
     pick = np.random.default_rng(3).choice(n, 200000, replace=False)
-    want = trace_range(ob, rays8_of(rays_np[pick]))
+    want = pt.walk(rays8(rays_np[pick]), two_sided=True)
     assert_records_equal({k: two[k][pick] for k in OUTS}, want)
 
 
