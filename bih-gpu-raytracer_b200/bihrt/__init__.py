@@ -66,9 +66,16 @@ class Hits(C.Structure):
                 ("ng", C.c_void_p)]
 
 
+class Closest(C.Structure):
+    """bihrt_closest: where bihrt_closest_point writes each part of the record (NULL = not wanted)."""
+    _fields_ = [("d2", C.c_void_p), ("u", C.c_void_p), ("v", C.c_void_p), ("slot", C.c_void_p), ("prim", C.c_void_p),
+                ("q", C.c_void_p), ("ng", C.c_void_p)]
+
+
 INTERSECT_ANY = 1
 INTERSECT_TWO_SIDED = 4
 HIT_OUTPUTS = ("t", "u", "v", "slot", "prim", "ng")
+CLOSEST_OUTPUTS = ("d2", "u", "v", "slot", "prim", "q", "ng")
 
 
 def interval_rays(rays6, tmin=0.0, tmax=np.inf):
@@ -88,11 +95,26 @@ def interval_rays(rays6, tmin=0.0, tmax=np.inf):
     return out
 
 
+def point_queries(points3, rmax=np.inf):
+    """(N,4) float32 queries p.xyz rmax for Renderer.closest_point, from (N,3) points and a scalar or per-point (N,) search
+    radius.  numpy in -> numpy out; torch in -> torch out on the same device."""
+    if isinstance(points3, np.ndarray):
+        p = np.asarray(points3, np.float32).reshape(-1, 3)
+        out = np.empty((p.shape[0], 4), np.float32)
+    else:
+        import torch
+        p = points3.reshape(-1, 3).to(torch.float32)
+        out = torch.empty((p.shape[0], 4), dtype=torch.float32, device=p.device)
+    out[:, 0:3] = p
+    out[:, 3] = rmax
+    return out
+
+
 # every symbol include/bihrt.h declares (tests check that the library exports all of them)
 ABI_SYMBOLS = [
     "bihrt_version", "bihrt_create", "bihrt_destroy", "bihrt_last_error", "bihrt_set_stream", "bihrt_get_stream", "bihrt_sync",
     "bihrt_set_option", "bihrt_get_stat", "bihrt_scene_load_triangles", "bihrt_scene_update_vertices", "bihrt_scene_load_obj",
-    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_trace_counted",
+    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_closest_point", "bihrt_trace_counted",
     "bihrt_render", "bihrt_render_counted", "bihrt_render_shard", "bihrt_render_samples", "bihrt_render_interleaved", "bihrt_render_interleaved_to", "bihrt_framebuffer_ipc_export", "bihrt_framebuffer_ipc_open", "bihrt_framebuffer_ipc_close", "bihrt_framebuffer_ipc_unexport", "bihrt_bih_region", "bihrt_bih_adopt", "bihrt_bih_copy", "bihrt_framebuffer_resolve", "bihrt_render_hits", "bihrt_secondary_rays", "bihrt_framebuffer", "bihrt_framebuffer_read",
     "bihrt_bih_blob_bytes", "bihrt_bih_export", "bihrt_bih_import",
     "bihrt_create_multi", "bihrt_destroy_multi", "bihrt_multi_size", "bihrt_multi_nccl_version", "bihrt_multi_broadcast",
@@ -360,6 +382,35 @@ class Renderer:
         if on_dev:
             self.wait_torch()            # rays (and recycled output blocks) were last touched on torch's current stream
         self._check(self._lib.bihrt_intersect(self._ctx, _ptr(rays8), C.c_int64(n), C.c_uint32(flags), C.byref(hits)))
+        if on_dev:
+            self.torch_wait()            # device outputs are written asynchronously on the context's stream
+        return res
+
+    def closest_point(self, queries4, outputs=CLOSEST_OUTPUTS):
+        """Closest-point queries (bihrt_closest_point).  queries4: (N,4) float32 p.xyz rmax (numpy or torch, host or device;
+        point_queries builds it).  A triangle counts when its squared distance d2 <= min(rmax^2, FLT_MAX); the result is the
+        one with the smallest (d2, slot).  Returns {name: array} for the requested outputs of d2 (N,), u (N,), v (N,),
+        slot (N,), prim (N,), q (N,3), ng (N,3): numpy for numpy input, torch tensors on the points' device for torch input.
+        A miss reads d2 = FLT_MAX, slot = prim = -1, u = v = q = ng = 0."""
+        unknown = set(outputs) - set(CLOSEST_OUTPUTS)
+        if unknown:
+            raise ValueError("unknown outputs %s (known: %s)" % (sorted(unknown), ", ".join(CLOSEST_OUTPUTS)))
+        shapes = {"d2": (), "u": (), "v": (), "slot": (), "prim": (), "q": (3,), "ng": (3,)}
+        if isinstance(queries4, np.ndarray):
+            queries4 = np.ascontiguousarray(queries4, dtype=np.float32)
+            n = queries4.size // 4
+            res = {k: np.empty((n,) + shapes[k], np.int32 if k in ("slot", "prim") else np.float32) for k in outputs}
+        else:
+            import torch
+            queries4 = queries4.contiguous()
+            n = queries4.numel() // 4
+            res = {k: torch.empty((n,) + shapes[k], dtype=torch.int32 if k in ("slot", "prim") else torch.float32,
+                                  device=queries4.device) for k in outputs}
+        rec = Closest(**{k: _ptr(res[k]) for k in res})
+        on_dev = getattr(queries4, "is_cuda", False)
+        if on_dev:
+            self.wait_torch()            # points (and recycled output blocks) were last touched on torch's current stream
+        self._check(self._lib.bihrt_closest_point(self._ctx, _ptr(queries4), C.c_int64(n), C.byref(rec)))
         if on_dev:
             self.torch_wait()            # device outputs are written asynchronously on the context's stream
         return res

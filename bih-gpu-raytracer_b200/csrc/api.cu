@@ -480,10 +480,11 @@ static void base_args(bihrt_ctx* c, TraceArgs& a) {
 }
 
 // outputs may individually be host or device; host ones are staged through d_io.  t, slot, prim (4 bytes per ray) for every
-// trace; u, v (4 bytes) and ng (12 bytes) for bihrt_intersect's hit records.  dev[k] is what the kernel writes (the caller's
-// device array, a staging block, or NULL), host[k] the caller's host array it is copied back to (NULL: none).
-enum { OUT_T, OUT_SLOT, OUT_PRIM, OUT_U, OUT_V, OUT_NG, OUT_COUNT };
-static const size_t out_bytes_per_ray[OUT_COUNT] = { 4, 4, 4, 4, 4, 12 };
+// trace; u, v (4 bytes) and ng (12 bytes) for bihrt_intersect's hit records; bihrt_closest_point routes d2 through t and adds
+// q (12 bytes).  dev[k] is what the kernel writes (the caller's device array, a staging block, or NULL), host[k] the caller's
+// host array it is copied back to (NULL: none).
+enum { OUT_T, OUT_SLOT, OUT_PRIM, OUT_U, OUT_V, OUT_NG, OUT_Q, OUT_COUNT };
+static const size_t out_bytes_per_ray[OUT_COUNT] = { 4, 4, 4, 4, 4, 12, 12 };
 struct OutStage {
     void* dev[OUT_COUNT]; void* host[OUT_COUNT];
     float* t() const { return (float*)dev[OUT_T]; }
@@ -492,8 +493,8 @@ struct OutStage {
 };
 
 static int stage_outputs(bihrt_ctx* c, int64_t n, size_t front_bytes, float* t, int32_t* slot, int32_t* prim, OutStage& o, uint8_t** front,
-                         float* u = nullptr, float* v = nullptr, float* ng = nullptr) {
-    void* const want[OUT_COUNT] = { t, slot, prim, u, v, ng };
+                         float* u = nullptr, float* v = nullptr, float* ng = nullptr, float* q = nullptr) {
+    void* const want[OUT_COUNT] = { t, slot, prim, u, v, ng, q };
     bool staged[OUT_COUNT];
     size_t need = front_bytes + 256;
     for (int k = 0; k < OUT_COUNT; k++) {
@@ -604,6 +605,37 @@ int bihrt_intersect(bihrt_ctx* c, const bihrt_ray_interval* rays, int64_t n, uin
     a.out_t = o.t(); a.out_slot = o.slot(); a.out_prim = o.prim();
     a.out_u = (float*)o.dev[OUT_U]; a.out_v = (float*)o.dev[OUT_V]; a.out_ng = (float*)o.dev[OUT_NG];
     if ((rc = bihrt_trace_launch(c, a, (flags & BIHRT_INTERSECT_TWO_SIDED) ? 4 : 3, false))) return rc;
+    return unstage_outputs(c, n, o);
+}
+
+// Closest-point queries with per-point radii and full records (include/bihrt.h): k_closest, csrc/closest.cu.
+int bihrt_closest_point(bihrt_ctx* c, const bihrt_point_query* pts, int64_t n, const bihrt_closest* out) {
+    ENTER(c);
+    if (!out) return bihrt_fail(c, BIHRT_ERR_INVALID, "no output record");
+    if (n < 0 || (n > 0 && !pts)) return bihrt_fail(c, BIHRT_ERR_INVALID, "bad point array");
+    if (n >= (1ll << 32) - (1ll << 24)) return bihrt_fail(c, BIHRT_ERR_INVALID, "too many points in one call (32-bit work counter)");
+    if (!c->built) return bihrt_fail(c, BIHRT_ERR_STATE, "BIH not built");
+    { int st = check_status(c); if (st) return st; }
+    if (n == 0) return BIHRT_OK;
+    const bool pts_dev = is_device_ptr(pts);
+    if (pts_dev && ((uintptr_t)pts & 15u)) return bihrt_fail(c, BIHRT_ERR_INVALID, "device points must be 16-byte aligned (one 128-bit load per point)");
+    OutStage o; uint8_t* front;
+    int rc = stage_outputs(c, n, pts_dev ? 0 : (size_t)n * sizeof(bihrt_point_query), out->d2, out->slot, out->prim, o, &front,
+                           out->u, out->v, out->ng, out->q);
+    if (rc) return rc;
+    ClosestArgs a;
+    memset(&a, 0, sizeof a);
+    a.hdr = c->d_hdr; a.nodes = c->d_nodes; a.tris = c->d_tris;
+    if (pts_dev) a.pts = pts;
+    else {
+        BIHRT_CUDA(c, cudaMemcpyAsync(front, pts, (size_t)n * sizeof(bihrt_point_query), cudaMemcpyHostToDevice, c->stream));
+        a.pts = (const bihrt_point_query*)front;
+    }
+    a.n = n;
+    a.out_d2 = o.t(); a.out_slot = o.slot(); a.out_prim = o.prim();
+    a.out_u = (float*)o.dev[OUT_U]; a.out_v = (float*)o.dev[OUT_V]; a.out_ng = (float*)o.dev[OUT_NG]; a.out_q = (float*)o.dev[OUT_Q];
+    a.work = c->d_work; a.status_map = c->d_status_map;
+    if ((rc = bihrt_closest_launch(c, a))) return rc;
     return unstage_outputs(c, n, o);
 }
 

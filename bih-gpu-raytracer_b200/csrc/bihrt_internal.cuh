@@ -172,6 +172,9 @@ int bihrt_build_launch(bihrt_ctx* c);
 int bihrt_build_setup(bihrt_ctx* c);      // once per context: scene-box accumulators and grid-barrier words in their rest state
 int bihrt_build_launch_q(bihrt_ctx* c);
 int bihrt_refit_launch(bihrt_ctx* c);
+// stack items per lane of a walk (trace.cu, closest.cu)
+#define STACK_DEPTH_PARITY  32  // <= 31 items: one per Morton bit on a root-to-leaf path, plus one
+#define STACK_DEPTH_QUALITY 96  // quality mode: 63 key bits + up to 29 position bits of tie-breaking
 // trace.cu
 struct TraceArgs {
     const BihHeader* hdr; const BihNode* nodes; const BihTri* tris;
@@ -199,6 +202,15 @@ struct TraceArgs {
 int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a, int mode /*0 rays,1 render fb,2 render hits,3 ray queries,4 two-sided ray queries*/, bool counted);
 int bihrt_resolve_launch(bihrt_ctx* c, uint32_t* fb, int npix, int spp);
 int bihrt_tile_order_launch(bihrt_ctx* c, uint32_t* cost, uint32_t* order, uint32_t ntiles, bool full_sort);
+// closest.cu: bihrt_closest_point (outputs NULL = not wanted)
+struct ClosestArgs {
+    const BihHeader* hdr; const BihNode* nodes; const BihTri* tris;
+    const bihrt_point_query* pts; int64_t n;
+    float* out_d2; float* out_u; float* out_v; int32_t* out_slot; int32_t* out_prim; float* out_q; float* out_ng;
+    uint32_t* work;         // persistent-kernel work counter
+    uint32_t* status_map;   // mapped host word: tree of the wrong kind for this kernel
+};
+int bihrt_closest_launch(bihrt_ctx* c, const ClosestArgs& a);
 // raysort.cu: permutation that groups a ray list by origin cell and direction octant (perm[i] = index of the i-th ray to trace)
 int bihrt_ray_sort_launch(bihrt_ctx* c, const bihrt_ray* rays, int64_t n, const uint32_t** perm);
 // shade.cu

@@ -36,8 +36,6 @@
 #include <float.h>
 
 #define FULL 0xffffffffu
-#define STACK_DEPTH_PARITY  32  // <= 31 items: one per Morton bit on a root-to-leaf path, plus one
-#define STACK_DEPTH_QUALITY 96  // quality mode: 63 key bits + up to 29 position bits of tie-breaking
 #define NONE 0xFFFFFFFFu        // "no item": leaf bit set, never a valid slot
 #define TRACE_THREADS 128
 #define TRACE_MIN_BLOCKS 8        // <= 64 registers per thread

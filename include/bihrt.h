@@ -209,6 +209,59 @@ typedef struct bihrt_hits {
 #define BIHRT_INTERSECT_ANY 1u   /* occlusion: end at the first accepted triangle of the interval */
 #define BIHRT_INTERSECT_TWO_SIDED 4u   /* back faces count too (|det| >= 1e-6); flag values 0, 1, 4 and 5 are valid */
 BIHRT_API int bihrt_intersect(bihrt_ctx* ctx, const bihrt_ray_interval* rays, int64_t n, uint32_t flags, const bihrt_hits* out);
+/* ---- closest-point queries: the triangle nearest to a point within the point's own search radius, full records.
+ *      Distance of point p to a triangle: one IEEE binary32 function, every product, sum and quotient rounded, no FMA,
+ *      computed from the triangle record's v0, e1 = v1 - v0, e2 = v2 - v0 (fl(v1 - v0), fl(v2 - v0), as bihrt_intersect
+ *      uses them).  It is Ericson's ClosestPtPointTriangle (Real-Time Collision Detection, 5.1.5) with a = v0, b = v1, c = v2:
+ *        ap = p - v0;  d1 = e1.ap, d2 = e2.ap                   (a.b = (ax*bx + ay*by) + az*bz throughout)
+ *        d1 <= 0 && d2 <= 0                          -> (u, v) = (0, 0)
+ *        bp = ap - e1; d3 = e1.bp, d4 = e2.bp
+ *        d3 >= 0 && d4 <= d3                          -> (1, 0)
+ *        vc = d1*d4 - d3*d2;  vc <= 0 && d1 >= 0 && d3 <= 0  -> (d1 / (d1 - d3), 0)                  [if d1 - d3 > 0]
+ *        cp = ap - e2; d5 = e1.cp, d6 = e2.cp
+ *        d6 >= 0 && d5 <= d6                          -> (0, 1)
+ *        vb = d5*d2 - d1*d6;  vb <= 0 && d2 >= 0 && d6 <= 0  -> (0, d2 / (d2 - d6))                  [if d2 - d6 > 0]
+ *        va = d3*d6 - d5*d4;  va <= 0 && d4 - d3 >= 0 && d5 - d6 >= 0
+ *                                                     -> w = (d4 - d3) / ((d4 - d3) + (d5 - d6)), (1 - w, w)
+ *                                                                                       [if (d4 - d3) + (d5 - d6) > 0]
+ *        s = (va + vb) + vc;  s > 0                   -> (vb / s, vc / s)   (quotients, not products with 1 / s: a zero
+ *                                                        weight stays 0 when 1 / s would overflow)
+ *        otherwise, and when an edge branch's bracketed condition fails (an edge of zero length, e.g. a repeated vertex):
+ *        zero or near-zero area, the nearest of the three edge segments, ties to AB, then AC, then BC.  Segment
+ *        from a with direction e (AB: ap, e1; AC: ap, e2; BC: bp, e2 - e1): t = (ap.e) / (e.e), t = 0 unless t > 0 (so also
+ *        for 0 / 0), t = 1 if t > 1; (u, v) = (t, 0), (0, t), (1 - t, t); each one's d2 as below.
+ *      then q = (v0 + u*e1) + v*e2 and d2 = ((p-q).x^2 + (p-q).y^2) + (p-q).z^2.  u, v are the barycentric weights of v1, v2.
+ *      For finite vertices and points whose differences and squares stay finite the result is never NaN.
+ *      A triangle is a CANDIDATE when d2 <= min(fl(rmax*rmax), FLT_MAX): rmax = +inf, or any rmax whose square overflows, is
+ *      unbounded; a triangle whose d2 overflows to +inf is never a candidate.  A query with a NaN or negative rmax, or a NaN or
+ *      infinite coordinate of p, misses without being walked.
+ *      Result: the candidate with the smallest (d2, slot), compared lexicographically -- ties go to the smaller slot -- so the
+ *      result does not depend on the walk's order and EQUALS BRUTE FORCE OVER ALL SLOTS BIT FOR BIT, in every output, on parity
+ *      and quality-mode trees alike.  The walk prunes with the children's exact boxes widened by a margin that covers the
+ *      rounding of the distance function (DESIGN.md section 8), so no candidate is ever pruned.
+ *      Record per query (every output pointer of bihrt_closest may be NULL; each one host or device):
+ *        d2, u, v   as above; slot, prim as bihrt_trace; q = (v0 + u*e1) + v*e2, 3 floats; ng = e1 x e2, as bihrt_hits.ng.
+ *        miss: d2 = FLT_MAX, slot = prim = -1, u = v = 0, q = ng = (0, 0, 0).
+ *      The trace options (trace_tile_order, trace_sm_queues, trace_sort_rays, trace_lane_groups, ...) do not apply: points are
+ *      taken in list order.  pts: host or device; device points must be 16-byte aligned (one 128-bit load per point).  Host
+ *      outputs: the call synchronises and leaves them untouched if the build's watchdog tripped; device outputs are written
+ *      asynchronously on the context's stream.
+ *      Errors: BIHRT_ERR_INVALID for out == NULL, n < 0, pts == NULL with n > 0, n >= 2^32 - 2^24 or misaligned device points;
+ *      BIHRT_ERR_STATE without a built BIH or for a replica of the other tree kind; BIHRT_ERR_INTERNAL after a tripped build
+ *      watchdog. ---------------------------------------------------------------------------------------------------------- */
+/* point with its own search radius: 16 B, one 128-bit load */
+typedef struct bihrt_point_query { float p[3]; float rmax; } bihrt_point_query;
+/* outputs of bihrt_closest_point: any pointer may be NULL; each one host or device */
+typedef struct bihrt_closest {
+    float*   d2;    /* [n]  squared distance to the closest point */
+    float*   u;     /* [n]  barycentric weight of v1 */
+    float*   v;     /* [n]  barycentric weight of v2 */
+    int32_t* slot;  /* [n]  as bihrt_trace */
+    int32_t* prim;  /* [n]  input triangle */
+    float*   q;     /* [3n] the closest point, xyz */
+    float*   ng;    /* [3n] geometric normal e1 x e2 of that triangle, as bihrt_hits.ng */
+} bihrt_closest;
+BIHRT_API int bihrt_closest_point(bihrt_ctx* ctx, const bihrt_point_query* pts, int64_t n, const bihrt_closest* out);
 /* instrumented trace: counters[0]=internal nodes visited, [1]=triangle tests, [2]=max stack depth,
  * [3]=rays; same results as bihrt_trace (outputs may be NULL). */
 BIHRT_API int bihrt_trace_counted(bihrt_ctx* ctx, const bihrt_ray* rays, int64_t n, float* t, int32_t* slot,
