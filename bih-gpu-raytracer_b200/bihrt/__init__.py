@@ -114,7 +114,7 @@ def point_queries(points3, rmax=np.inf):
 ABI_SYMBOLS = [
     "bihrt_version", "bihrt_create", "bihrt_destroy", "bihrt_last_error", "bihrt_set_stream", "bihrt_get_stream", "bihrt_sync",
     "bihrt_set_option", "bihrt_get_stat", "bihrt_scene_load_triangles", "bihrt_scene_update_vertices", "bihrt_scene_load_obj",
-    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_closest_point", "bihrt_trace_counted",
+    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_closest_point", "bihrt_winding_number", "bihrt_trace_counted",
     "bihrt_render", "bihrt_render_counted", "bihrt_render_shard", "bihrt_render_samples", "bihrt_render_interleaved", "bihrt_render_interleaved_to", "bihrt_framebuffer_ipc_export", "bihrt_framebuffer_ipc_open", "bihrt_framebuffer_ipc_close", "bihrt_framebuffer_ipc_unexport", "bihrt_bih_region", "bihrt_bih_adopt", "bihrt_bih_copy", "bihrt_framebuffer_resolve", "bihrt_render_hits", "bihrt_secondary_rays", "bihrt_framebuffer", "bihrt_framebuffer_read",
     "bihrt_bih_blob_bytes", "bihrt_bih_export", "bihrt_bih_import",
     "bihrt_create_multi", "bihrt_destroy_multi", "bihrt_multi_size", "bihrt_multi_nccl_version", "bihrt_multi_broadcast",
@@ -413,6 +413,54 @@ class Renderer:
         self._check(self._lib.bihrt_closest_point(self._ctx, _ptr(queries4), C.c_int64(n), C.byref(rec)))
         if on_dev:
             self.torch_wait()            # device outputs are written asynchronously on the context's stream
+        return res
+
+    def winding_number(self, queries4, beta=2.0):
+        """Generalized winding numbers (bihrt_winding_number): (1/4pi) x the signed solid angle of the mesh at each point, 1 inside
+        and 0 outside a closed outward-wound mesh.  queries4: (N,4) float32 p.xyz rmax as for closest_point (rmax is not read;
+        numpy or torch, host or device).  beta > 1 sets the accuracy of the far-field expansion (2 recommended; np.inf: the
+        exact sum, O(n) per point).  Returns (N,) float32: numpy for numpy input, a torch tensor on the points' device for
+        torch input."""
+        beta = float(beta)
+        if not beta > 1.0:
+            raise ValueError("beta must be > 1 or inf (got %r)" % beta)
+        if isinstance(queries4, np.ndarray):
+            queries4 = np.ascontiguousarray(queries4, dtype=np.float32)
+            n = queries4.size // 4
+            w = np.empty(n, np.float32)
+        else:
+            import torch
+            queries4 = queries4.contiguous()
+            n = queries4.numel() // 4
+            w = torch.empty(n, dtype=torch.float32, device=queries4.device)
+        on_dev = getattr(queries4, "is_cuda", False)
+        if on_dev:
+            self.wait_torch()            # points (and recycled output blocks) were last touched on torch's current stream
+        self._check(self._lib.bihrt_winding_number(self._ctx, _ptr(queries4), C.c_int64(n), C.c_float(beta), _ptr(w)))
+        if on_dev:
+            self.torch_wait()            # device outputs are written asynchronously on the context's stream
+        return w
+
+    def signed_distance(self, queries4, beta=2.0, outputs=("sd",)):
+        """Signed distance from the two queries on the same points: sd = -sqrt(d2) where the winding number w > 0.5 (inside),
+        +sqrt(d2) otherwise; a point whose search radius rmax reaches no triangle gets -inf / +inf.  outputs: "sd", "w" and any
+        of CLOSEST_OUTPUTS.  Returns {name: array} as closest_point does."""
+        unknown = set(outputs) - set(("sd", "w") + CLOSEST_OUTPUTS)
+        if unknown:
+            raise ValueError("unknown outputs %s (known: sd, w, %s)" % (sorted(unknown), ", ".join(CLOSEST_OUTPUTS)))
+        closest = self.closest_point(queries4, outputs=tuple(dict.fromkeys(("d2", "slot") + tuple(k for k in outputs if k in CLOSEST_OUTPUTS))))
+        w = self.winding_number(queries4, beta)
+        res = {k: v for k, v in closest.items() if k in outputs}
+        if "w" in outputs:
+            res["w"] = w
+        if "sd" in outputs:
+            if isinstance(w, np.ndarray):
+                dist = np.where(closest["slot"] >= 0, np.sqrt(closest["d2"]), np.float32(np.inf)).astype(np.float32)
+                res["sd"] = np.where(w > 0.5, -dist, dist).astype(np.float32)
+            else:
+                import torch
+                dist = torch.where(closest["slot"] >= 0, torch.sqrt(closest["d2"]), torch.full_like(closest["d2"], float("inf")))
+                res["sd"] = torch.where(w > 0.5, -dist, dist)
         return res
 
     def render(self, camera, w, h, spp=1, seed=1984, jitter=False, shard=(0, 1)):

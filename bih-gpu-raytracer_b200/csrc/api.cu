@@ -139,6 +139,7 @@ void bihrt_destroy(bihrt_ctx* c) {
     dev_free(&c->d_heaps); dev_free(&c->d_scenebox_enc);
     dev_free(&c->d_keys64[0]); dev_free(&c->d_keys64[1]); dev_free(&c->d_lookback_q);
     dev_free(&c->d_fb); dev_free(&c->d_counters); dev_free(&c->d_work);
+    dev_free(&c->d_wtab); dev_free(&c->d_wscratch);
     for (auto& ts : c->tile_slots) { dev_free(&ts.cost); dev_free(&ts.order); }
     if (c->d_io) { cudaFree(c->d_io); c->d_io = nullptr; }
     for (int i = 0; i < 2; i++) { dev_free(&c->d_rs_keys[i]); dev_free(&c->d_rs_vals[i]); }
@@ -374,6 +375,7 @@ int bihrt_build(bihrt_ctx* c) {
     }
     BIHRT_CUDA(c, cudaEventRecord(c->ev1, c->stream));
     c->built = true; c->build_timed = true; c->topology_valid = c->n > 0 && !quality; c->built_quality = quality && c->n > 0;
+    c->wtab_valid = false;
     return BIHRT_OK;
 }
 
@@ -386,7 +388,7 @@ int bihrt_refit(bihrt_ctx* c) {
     int rc = bihrt_refit_launch(c);
     if (rc) return rc;
     BIHRT_CUDA(c, cudaEventRecord(c->ev1, c->stream));
-    c->built = true; c->build_timed = true;
+    c->built = true; c->build_timed = true; c->wtab_valid = false;
     return BIHRT_OK;
 }
 
@@ -481,8 +483,8 @@ static void base_args(bihrt_ctx* c, TraceArgs& a) {
 
 // outputs may individually be host or device; host ones are staged through d_io.  t, slot, prim (4 bytes per ray) for every
 // trace; u, v (4 bytes) and ng (12 bytes) for bihrt_intersect's hit records; bihrt_closest_point routes d2 through t and adds
-// q (12 bytes).  dev[k] is what the kernel writes (the caller's device array, a staging block, or NULL), host[k] the caller's
-// host array it is copied back to (NULL: none).
+// q (12 bytes); bihrt_winding_number routes w through t.  dev[k] is what the kernel writes (the caller's device array, a
+// staging block, or NULL), host[k] the caller's host array it is copied back to (NULL: none).
 enum { OUT_T, OUT_SLOT, OUT_PRIM, OUT_U, OUT_V, OUT_NG, OUT_Q, OUT_COUNT };
 static const size_t out_bytes_per_ray[OUT_COUNT] = { 4, 4, 4, 4, 4, 12, 12 };
 struct OutStage {
@@ -636,6 +638,48 @@ int bihrt_closest_point(bihrt_ctx* c, const bihrt_point_query* pts, int64_t n, c
     a.out_u = (float*)o.dev[OUT_U]; a.out_v = (float*)o.dev[OUT_V]; a.out_ng = (float*)o.dev[OUT_NG]; a.out_q = (float*)o.dev[OUT_Q];
     a.work = c->d_work; a.status_map = c->d_status_map;
     if ((rc = bihrt_closest_launch(c, a))) return rc;
+    return unstage_outputs(c, n, o);
+}
+
+// Winding numbers (include/bihrt.h): k_winding, csrc/winding.cu.  The far-field table is built here, by the first call with
+// points after the BIH changed.
+int bihrt_winding_number(bihrt_ctx* c, const bihrt_point_query* pts, int64_t n, float beta, float* w) {
+    ENTER(c);
+    if (!w) return bihrt_fail(c, BIHRT_ERR_INVALID, "no output array");
+    if (n < 0 || (n > 0 && !pts)) return bihrt_fail(c, BIHRT_ERR_INVALID, "bad point array");
+    if (n >= (1ll << 32) - (1ll << 24)) return bihrt_fail(c, BIHRT_ERR_INVALID, "too many points in one call (32-bit work counter)");
+    if (!(beta > 1.f)) return bihrt_fail(c, BIHRT_ERR_INVALID, "beta must be > 1 (or +inf for the exact sum)");
+    if (!c->built) return bihrt_fail(c, BIHRT_ERR_STATE, "BIH not built");
+    { int st = check_status(c); if (st) return st; }
+    if (n == 0) return BIHRT_OK;
+    const bool pts_dev = is_device_ptr(pts);
+    if (pts_dev && ((uintptr_t)pts & 15u)) return bihrt_fail(c, BIHRT_ERR_INVALID, "device points must be 16-byte aligned (one 128-bit load per point)");
+    int rc;
+    if (!c->wtab_valid) {
+        const int64_t slots = std::max<int64_t>(c->n, 1);      // the blob's node region
+        if (slots > c->wtab_slots) {
+            dev_free(&c->d_wscratch); c->wtab_slots = 0;
+            if ((rc = dev_alloc(c, &c->d_wtab, (size_t)slots * 2 * WTAB_FLOATS))) return rc;
+            if ((rc = dev_alloc(c, &c->d_wscratch, WTAB_SCRATCH_WORDS(slots)))) { dev_free(&c->d_wtab); return rc; }
+            c->wtab_slots = slots;
+        }
+        if ((rc = bihrt_winding_table_launch(c))) return rc;
+        c->wtab_valid = true;
+    }
+    OutStage o; uint8_t* front;
+    rc = stage_outputs(c, n, pts_dev ? 0 : (size_t)n * sizeof(bihrt_point_query), w, nullptr, nullptr, o, &front);
+    if (rc) return rc;
+    WindingArgs a;
+    memset(&a, 0, sizeof a);
+    a.hdr = c->d_hdr; a.nodes = c->d_nodes; a.tris = c->d_tris; a.wtab = c->d_wtab;
+    if (pts_dev) a.pts = pts;
+    else {
+        BIHRT_CUDA(c, cudaMemcpyAsync(front, pts, (size_t)n * sizeof(bihrt_point_query), cudaMemcpyHostToDevice, c->stream));
+        a.pts = (const bihrt_point_query*)front;
+    }
+    a.n = n; a.b2 = beta * beta; a.out_w = o.t();
+    a.work = c->d_work; a.status_map = c->d_status_map;
+    if ((rc = bihrt_winding_launch(c, a))) return rc;
     return unstage_outputs(c, n, o);
 }
 
@@ -939,6 +983,7 @@ int bihrt_bih_import(bihrt_ctx* c, const void* dev_src, uint64_t bytes) {
     if (nb) BIHRT_CUDA(c, cudaMemcpyAsync(c->d_nodes, s + 64, nb, cudaMemcpyDeviceToDevice, c->stream));
     if (tb) BIHRT_CUDA(c, cudaMemcpyAsync(c->d_tris, s + 64 + nb, tb, cudaMemcpyDeviceToDevice, c->stream));
     c->n = h.n; c->built = true; c->build_timed = false; c->topology_valid = false; c->built_quality = h.quality != 0;
+    c->wtab_valid = false;
     return BIHRT_OK;
 }
 
@@ -1002,7 +1047,7 @@ int bihrt_bih_copy(bihrt_ctx* dst, bihrt_ctx* src) {
 int bihrt_bih_adopt(bihrt_ctx* c, int64_t n) {
     ENTER(c);
     if (n != c->n || !c->d_blob) return bihrt_fail(c, BIHRT_ERR_STATE, "bihrt_bih_adopt(%lld) without a matching bihrt_bih_region", (long long)n);
-    c->built = true; c->build_timed = false; c->topology_valid = false;
+    c->built = true; c->build_timed = false; c->topology_valid = false; c->wtab_valid = false;
     c->built_quality = c->opt_morton_bits == 63;                 // (the kernel refuses a tree of the other kind: see check_status)
     if (c->h_status) *c->h_status = 0;
     return BIHRT_OK;

@@ -150,6 +150,11 @@ struct bihrt_ctx {
     int opt_morton_bits = 30;   // 30: the reference's grid (parity path); 63: quality mode (SURVEY.md 8(f) f4, non-parity)
     int opt_leaf_cap = 4;       // quality mode: a subtree of at most this many triangles becomes one leaf
     bool built_quality = false; // the BIH in the blob is a quality-mode tree (deeper: the traversal needs the long stack, and no reference quirks)
+    // winding numbers (winding.cu): far-field table, 256 B per node slot, built lazily; every place that sets `built` clears
+    // wtab_valid
+    float*    d_wtab = nullptr; int64_t wtab_slots = 0;
+    uint32_t* d_wscratch = nullptr;                    // its build's queue, parents, leaf list and arrival counters
+    bool      wtab_valid = false;
     int opt_debug_trip_watchdog = 0;   // tests: the next build reports this watchdog status (as if a sort pass had timed out)
     int opt_profile = 0;    // record an event after every build stage (bihrt_get_stat "build_stage_us_<i>")
     cudaEvent_t prof_ev[BIHRT_PROF_EVENTS] = {};
@@ -211,6 +216,21 @@ struct ClosestArgs {
     uint32_t* status_map;   // mapped host word: tree of the wrong kind for this kernel
 };
 int bihrt_closest_launch(bihrt_ctx* c, const ClosestArgs& a);
+// winding.cu: bihrt_winding_number.  Far-field table: per node slot, the order-2 expansion of each child about its box centre,
+// WTAB_FLOATS floats per child (N[3], M[3][3] row-major, Q[i][jk] for jk = 00 01 02 11 12 22, 2 unused).
+#define WTAB_FLOATS 32
+#define WTAB_SCRATCH_WORDS(n) (4 * (size_t)(n) + 16)   // queue, parent, leaf list, arrivals + counters
+struct WindingArgs {
+    const BihHeader* hdr; const BihNode* nodes; const BihTri* tris;
+    const float* wtab;
+    const bihrt_point_query* pts; int64_t n;
+    float b2;               // fl(beta * beta); +inf: exact
+    float* out_w;
+    uint32_t* work;         // persistent-kernel work counter
+    uint32_t* status_map;   // mapped host word: tree of the wrong kind for this kernel
+};
+int bihrt_winding_table_launch(bihrt_ctx* c);      // fills c->d_wtab from the blob (c->d_wtab / d_wscratch sized for c->n)
+int bihrt_winding_launch(bihrt_ctx* c, const WindingArgs& a);
 // raysort.cu: permutation that groups a ray list by origin cell and direction octant (perm[i] = index of the i-th ray to trace)
 int bihrt_ray_sort_launch(bihrt_ctx* c, const bihrt_ray* rays, int64_t n, const uint32_t** perm);
 // shade.cu
