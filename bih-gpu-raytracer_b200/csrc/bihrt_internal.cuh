@@ -203,6 +203,9 @@ struct TraceArgs {
     // any_hit = BIHRT_INTERSECT_ANY (tmax comes with every ray)
     const bihrt_ray_interval* rays_iv;
     float* out_u; float* out_v; float* out_ng;
+    // camera modes, set by bihrt_trace_launch: tiles per row and 0xFFFFFFFF / tile_cols, so that a warp finds its unit's
+    // tile row with a multiply-high (and one correction) instead of a divide
+    uint32_t tile_cols, tile_cols_rcp;
 };
 int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a, int mode /*0 rays,1 render fb,2 render hits,3 ray queries,4 two-sided ray queries*/, bool counted);
 int bihrt_resolve_launch(bihrt_ctx* c, uint32_t* fb, int npix, int spp);

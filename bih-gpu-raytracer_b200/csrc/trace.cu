@@ -34,6 +34,7 @@
 // so t is bit-identical to the oracle's; the box distances are explicit FMAs, mirrored with fmaf in the oracle.
 #include "bihrt_internal.cuh"
 #include <float.h>
+#include <type_traits>
 
 #define FULL 0xffffffffu
 #define NONE 0xFFFFFFFFu        // "no item": leaf bit set, never a valid slot
@@ -186,16 +187,18 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
     uint32_t nnodes = 0, ntris = 0, maxsp = 0;
     uint32_t wnode = 0, wleaf = 0;              // COUNTED: warp-level executions of the node step / the triangle test (SIMD efficiency = lane steps / 32 / these)
 
-    // work items
-    uint64_t total;
-    int tx = 1;
+    // work items: 32-bit in the camera modes, whose launches bihrt_trace_launch refuses from 2^32 - 2^24 padded items on
+    // (the margin covers every warp's last fetch past the end)
+    using item_t = std::conditional_t<LIST, uint64_t, uint32_t>;
+    constexpr item_t NO_ITEM = ~item_t(0);
+    item_t total;
     // ray lists with cost-ordered chunks: the list is dealt in chunks of 1024 rays (the last one padded)
     if (LIST) total = a.tile_cost ? (((uint64_t)a.nrays + 1023u) >> 10) << 10 : (uint64_t)a.nrays;
     else {
-        tx = (a.w + 31) / 32;
+        const int tx = (a.w + 31) / 32;
         const int ty = (a.h + 31) / 32, T = tx * ty;
         const int my_tiles = T > a.shard_index ? (T - a.shard_index + a.shard_count - 1) / a.shard_count : 0;
-        total = ((uint64_t)my_tiles * 1024u) << a.gshift;
+        total = ((item_t)my_tiles * 1024u) << a.gshift;
     }
     // Camera modes: the samples [s_begin, s_end) of a pixel are split into 2^gshift groups that sit in
     // CONSECUTIVE LANES (item = pixel * groups + group); a lane traces its group's samples one after the
@@ -204,12 +207,13 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
     const int nsamp = LIST ? 1 : ((a.s_end - a.s_begin) >> gshift);    // samples per item
     uint32_t my_queue = 0;
     if (a.queues > 1) { asm("mov.u32 %0, %%smid;" : "=r"(my_queue)); my_queue %= (uint32_t)a.queues; }
-    uint64_t pool_next = 0, pool_end = 0;      // warp-uniform
+    item_t pool_next = 0, pool_end = 0;        // warp-uniform
+    uint32_t pool_xy = 0;                      // warp-uniform, camera modes: first pixel of the pool's tile, x | y << 16
     long long unit_t0 = 0; uint32_t unit_tile = 0xFFFFFFFFu;   // warp-uniform: start time / tile of the packet being traced
     bool exhausted = false;                    // warp-uniform: the global counter ran past `total`
 
     // lane state
-    uint64_t item = ~0ull;                     // current work item, ~0 = none
+    item_t item = NO_ITEM;                     // current work item
     int s = 0, s0 = 0;                         // sample of the item being traced, first sample of the item
     uint32_t hits = 0, pixel = 0, pxy = 0;
     // the box tests need all three axes: 1/direction, -origin/direction (plane distance = one FMA) and the absolute rounding
@@ -285,10 +289,10 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                         if (MODE == 1 && gshift > 0) finishing = true;      // written below, by the pixel's lanes together
                         else if (MODE == 1 && (a.flags & BIHRT_RENDER_COUNTS)) a.fb[pixel] = hits;     // resolved after the reduce
                         else if (MODE == 1) a.fb[pixel] = pack_colour(hits, nsamp);
-                        item = ~0ull;
+                        item = NO_ITEM;
                     }
                 }
-                want_item = (item == ~0ull);
+                want_item = (item == NO_ITEM);
             }
             if (MODE == 1 && gshift > 0) {
                 // the lanes of one pixel finish together (always, when the warp moves in lock step).  The participants are
@@ -321,84 +325,102 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                     // warp of an SM drains its own SM's queue first, so the warps resident on one SM walk the
                     // same one or two tiles and share nodes and triangles in L1; an SM that runs dry steals
                     // from the others.  a.queues == 1 is one global counter (one unit per fetch).
-                    uint64_t base = ~0ull;
-                    uint32_t got = 0;
+                    item_t base = NO_ITEM;
+                    uint32_t got = 0, unit_m = 0, unit_xy = 0;
                     if (lane == 0) {
                         // unit interleave across GPUs (il_count ranks): this rank owns every il_count-th 32-item unit
                         // of every tile, so all ranks walk all tiles (same locality, perfect balance) and every
                         // pixel keeps all its samples -- and their lane grouping -- on one GPU
                         const uint32_t ilc = (uint32_t)a.il_count, ili = (uint32_t)a.il_index, ics = (uint32_t)a.il_cshift;
                         if (a.queues <= 1) {
-                            const uint64_t fetched = atomicAdd(a.work, 32u); got = 32;
-                            const uint64_t lu = fetched >> 5;          // this rank's unit -> the frame's unit (runs of 2^il_cshift units)
-                            base = ilc > 1 ? ((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u))) << 5 : fetched;
-                            if (base >= total) base = ~0ull;
+                            const item_t fetched = atomicAdd(a.work, 32u); got = 32;
+                            const item_t lu = fetched >> 5;            // this rank's unit -> the frame's unit (runs of 2^il_cshift units)
+                            if constexpr (LIST) {
+                                base = ilc > 1 ? ((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u))) << 5 : fetched;
+                                if (base >= total) base = NO_ITEM;
+                            } else {
+                                // compared as units: past the end of an interleaved launch the frame's unit may reach 2^27,
+                                // where its first item would wrap
+                                const uint32_t fu = ilc > 1 ? (((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u)) : lu;
+                                if (fu < (total >> 5)) base = fu << 5;
+                            }
                         } else {
                             const uint32_t tshift = 10 + gshift, ushift = 5 + gshift;       // items / units per tile
-                            const uint64_t ntile = (total + ((1ull << tshift) - 1)) >> tshift;
+                            const item_t ntile = (total + ((item_t(1) << tshift) - 1)) >> tshift;
                             for (uint32_t k = 0; k < (uint32_t)a.queues; k++) {
                                 uint32_t q = my_queue + k; if (q >= (uint32_t)a.queues) q -= (uint32_t)a.queues;
                                 if (q >= ntile) continue;
                                 const uint32_t upt = (1u << ushift) / ilc;                                  // this rank's units per tile
-                                const uint64_t units = ((ntile - q + a.queues - 1) / a.queues) * upt;       // of queue q
+                                const item_t units = ((ntile - q + a.queues - 1) / a.queues) * upt;         // of queue q
                                 if (ld_relaxed(a.work + q) >= units) continue;
                                 const uint32_t u = atomicAdd(a.work + q, 1u);
                                 if (u >= units) continue;
                                 const uint32_t lu = u % upt;
-                                const uint64_t b = (((uint64_t)(u / upt) * a.queues + q) << tshift) + ((uint64_t)((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u))) << 5);
+                                const item_t b = (((item_t)(u / upt) * a.queues + q) << tshift) + ((item_t)((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u))) << 5);
                                 if (b < total) { base = b; got = 32; break; }
                             }
                         }
+                        if (!LIST && base != NO_ITEM) {
+                            // the unit's tile, once for its 32 items: m-th in cost order, its row and column (tile < 2^22: the
+                            // multiply-high is the row or one below it), its first pixel packed as x | y << 16 (w, h <= 65535)
+                            const uint32_t mi = (uint32_t)base >> (10 + gshift);
+                            unit_m = a.tile_order ? __ldg(a.tile_order + mi) : mi;
+                            const uint32_t tile = (uint32_t)a.shard_index + unit_m * (uint32_t)a.shard_count;
+                            uint32_t row = __umulhi(tile, a.tile_cols_rcp), col = tile - row * a.tile_cols;
+                            if (col >= a.tile_cols) { row++; col -= a.tile_cols; }
+                            unit_xy = (col << 5) | (row << 21);
+                        }
                     }
                     base = __shfl_sync(FULL, base, 0);
-                    got = __shfl_sync(FULL, got, 0);
+                    if (LIST) got = __shfl_sync(FULL, got, 0);
                     if (LIST && a.tile_cost && unit_tile != 0xFFFFFFFFu) {
                         // ray lists: the time between two fetches of the warp is charged to the chunk of the earlier one
                         if (lane == 0) atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
                         unit_tile = 0xFFFFFFFFu;
                     }
-                    if (base == ~0ull) { exhausted = true; break; }
+                    if (base == NO_ITEM) { exhausted = true; break; }
                     pool_next = base;
-                    pool_end = min(base + got, total);
+                    pool_end = LIST ? min(base + got, total) : base + 32u;     // (camera units never straddle the end: whole tiles)
+                    if (!LIST) pool_xy = __shfl_sync(FULL, unit_xy, 0);
                     if (a.tile_cost && unit_tile == 0xFFFFFFFFu) {
-                        const uint32_t m = (uint32_t)(base >> (10 + gshift));
-                        unit_tile = a.tile_order ? __ldg(a.tile_order + m) : m;
+                        if (LIST) {
+                            const uint32_t m = (uint32_t)(base >> (10 + gshift));
+                            unit_tile = a.tile_order ? __ldg(a.tile_order + m) : m;
+                        } else unit_tile = __shfl_sync(FULL, unit_m, 0);
                         unit_t0 = clock64();
                     }
                 }
-                const uint64_t avail = pool_end - pool_next;
+                const item_t avail = pool_end - pool_next;
                 const uint32_t rank = __popc(want & lt);
-                const bool served = want_item && (uint64_t)rank < avail;
+                const bool served = want_item && (item_t)rank < avail;
                 if (served) {
                     item = pool_next + rank; s = 0; hits = 0; want_item = false;
                     if (LIST && a.tile_cost) {
                         // logical item -> ray: chunk (item >> 10) is the chunk traced m-th in cost order
                         const uint32_t mi = (uint32_t)(item >> 10);
                         const uint64_t ray = ((uint64_t)(a.tile_order ? __ldg(a.tile_order + mi) : mi) << 10) | (item & 1023u);
-                        item = ray < (uint64_t)a.nrays ? ray : ~0ull;        // padding of the last chunk
-                        if (item == ~0ull) want_item = true;
+                        item = ray < (uint64_t)a.nrays ? ray : NO_ITEM;      // padding of the last chunk
+                        if (item == NO_ITEM) want_item = true;
                     }
                     // sorted ray lists: the i-th item is ray perm[i]; from here on `item` is the ray's own index (load and store)
-                    if (MODE == 0 && a.perm && item != ~0ull) item = __ldg(a.perm + item);
+                    if (MODE == 0 && a.perm && item != NO_ITEM) item = __ldg(a.perm + item);
                     if (!LIST) {
-                        const uint64_t pix = item >> gshift;
+                        // the item's pixel: the unit's first pixel plus the pixel's place in the tile (8x4 blocks of 8x4 pixels)
+                        const uint32_t q = (uint32_t)(item >> gshift) & 1023u;
                         s0 = a.s_begin + (int)((uint32_t)item & ((1u << gshift) - 1u)) * nsamp;
-                        const uint32_t mi = (uint32_t)(pix >> 10), q = (uint32_t)pix & 1023u;
-                        const uint32_t m = a.tile_order ? __ldg(a.tile_order + mi) : mi;      // m-th tile in cost order
-                        const int tile = a.shard_index + (int)m * a.shard_count;
-                        const int px = (tile % tx) * 32 + (int)((q >> 5) & 3u) * 8 + (int)(q & 7u);
-                        const int py = (tile / tx) * 32 + (int)(q >> 7) * 4 + (int)((q >> 3) & 3u);
-                        if (px < a.w && py < a.h) { pixel = (uint32_t)(py * a.w + px); pxy = (uint32_t)px | ((uint32_t)py << 16); }
-                        else item = ~0ull;                                   // padding pixel of an edge tile
-                        if (item == ~0ull) want_item = true;
+                        const uint32_t xy = pool_xy + (((q >> 2) & 0x18u) | (q & 7u)) + ((((q >> 5) & 0x1cu) | ((q >> 3) & 3u)) << 16);
+                        const uint32_t px = xy & 0xFFFFu, py = xy >> 16;
+                        if (px < (uint32_t)a.w && py < (uint32_t)a.h) { pixel = py * (uint32_t)a.w + px; pxy = xy; }
+                        else item = NO_ITEM;                                 // padding pixel of an edge tile
+                        if (item == NO_ITEM) want_item = true;
                     }
                 }
-                pool_next += min((uint64_t)__popc(want), avail);
+                pool_next += min((item_t)__popc(want), avail);
                 // lanes that drew a padding pixel, or were not served, ask again
                 want = __ballot_sync(FULL, want_item);
             }
             // start the next ray of every idle lane that owns an item
-            if (cur == NONE && item != ~0ull) {
+            if (cur == NONE && item != NO_ITEM) {
                 float ox, oy, oz, dx, dy, dz;
                 float tlo = 0.f, thi = FLT_MAX;           // MODE 3: max(tmin, 0), min(tmax, FLT_MAX)
                 bool live = true;                         // MODE 3: max(tmin, 0) < tmax (false for a NaN bound): else a miss, not traced
@@ -492,7 +514,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 my_ray[9] = __int_as_float(oct);
             }
             if (__ballot_sync(FULL, cur != NONE || tracing) == 0 && exhausted &&
-                __ballot_sync(FULL, item != ~0ull) == 0) break;
+                __ballot_sync(FULL, item != NO_ITEM) == 0) break;
         }
 
         // ================= phase 1: internal nodes =====================================================
@@ -816,6 +838,7 @@ int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a_in, int mode, bool count
         const int mine = T > a.shard_index ? (T - a.shard_index + a.shard_count - 1) / a.shard_count : 0;
         if ((((uint64_t)mine * 1024u) << a.gshift) >= (1ull << 32) - (1ull << 24))
             return bihrt_fail(c, BIHRT_ERR_INVALID, "launch of %d tiles x 1024 pixels x %d lane groups exceeds the 32-bit work counter", mine, 1 << a.gshift);
+        a.tile_cols = (uint32_t)tx; a.tile_cols_rcp = 0xFFFFFFFFu / (uint32_t)tx;
     }
     // (launches of tens of milliseconds have no tail to speak of and lose ~0.5 % to the changed tile neighbourhood; tiny
     // scenes have no long units -- the Cornell box frame is 25 us -- and only pay for the extra k_tile_order launch)
