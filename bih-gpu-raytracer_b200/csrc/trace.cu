@@ -33,6 +33,7 @@
 // tests/walk_oracle.c restates as exit "first" (COVER below).  Everything that decides a hit is IEEE binary32 without FMA contraction (explicit __f*_rn)
 // so t is bit-identical to the oracle's; the box distances are explicit FMAs, mirrored with fmaf in the oracle.
 #include "bihrt_internal.cuh"
+#include "fb_math.cuh"
 #include <float.h>
 #include <type_traits>
 
@@ -67,17 +68,6 @@ struct Hit { float t; int slot; };
 
 __device__ __forceinline__ float fmin3(float a, float b, float c) { float r; asm("min.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c)); return r; }
 __device__ __forceinline__ float fmax3(float a, float b, float c) { float r; asm("max.f32 %0, %1, %2, %3;" : "=f"(r) : "f"(a), "f"(b), "f"(c)); return r; }
-
-// Color + rgbToInt, R/src/CUDAKernels.cu:82-88,385-387,420-422: mean over the samples of hit (255,255,0) /
-// miss (20,20,40), packed r | g<<8 | b<<16 (sums of 255/20/40 are exact in binary32)
-__device__ __forceinline__ uint32_t pack_colour(uint32_t hits, int samples) {
-    const float fh = (float)hits, fm = (float)(samples - (int)hits), fs = (float)samples;
-    float cr = __fdiv_rn(__fadd_rn(__fmul_rn(fh, 255.f), __fmul_rn(fm, 20.f)), fs);
-    float cb = __fdiv_rn(__fmul_rn(fm, 40.f), fs);
-    cr = fmaxf(0.f, fminf(255.f, cr));
-    cb = fmaxf(0.f, fminf(255.f, cb));
-    return ((uint32_t)(int)cb << 16) | ((uint32_t)(int)cr << 8) | (uint32_t)(int)cr;
-}
 
 // Moller-Trumbore in three steps (R/src/CUDAKernels.cu:24-42).  The triangle test of the walk and the hit-record epilogue
 // of MODE 3 both call these, so the u, v a ray query reports are the ones its walk computed, bit for bit.
@@ -184,6 +174,21 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
         return;
     }
     const float blo[3] = { a.hdr->lo[0], a.hdr->lo[1], a.hdr->lo[2] }, bhi[3] = { a.hdr->hi[0], a.hdr->hi[1], a.hdr->hi[2] };
+    // Framebuffer renders (MODE 1): what every refill needs of the launch sits in shared memory, not in registers (the kernel
+    // is at its register cap, and the scene box had been spilled to local memory): the camera divides' constants (1/w, -w,
+    // 1/h, -h; fb_math.cuh), the scene box (lo xyz, hi xyz) and the packed colour of every hit count of a pixel.
+    __shared__ __align__(16) float s_fb[12];
+    __shared__ uint32_t s_colour[COLOUR_TABLE_MAX + 1];
+    if constexpr (MODE == 1) {
+        if (threadIdx.x == 0) {
+            const float fw = (float)a.w, fh = (float)a.h;
+            s_fb[0] = camera_rcp(fw); s_fb[1] = -fw; s_fb[2] = camera_rcp(fh); s_fb[3] = -fh;
+            s_fb[4] = blo[0]; s_fb[5] = blo[1]; s_fb[6] = blo[2]; s_fb[7] = bhi[0]; s_fb[8] = bhi[1]; s_fb[9] = bhi[2];
+        }
+        const int n = ((a.s_end - a.s_begin) >> a.gshift) << a.gshift;      // samples per written pixel: nsamp << gshift below
+        if (n <= COLOUR_TABLE_MAX) fill_colour_table(s_colour, n, threadIdx.x, TRACE_THREADS);
+        __syncthreads();
+    }
     uint32_t nnodes = 0, ntris = 0, maxsp = 0;
     uint32_t wnode = 0, wleaf = 0;              // COUNTED: warp-level executions of the node step / the triangle test (SIMD efficiency = lane steps / 32 / these)
 
@@ -288,7 +293,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                     if (s == nsamp) {
                         if (MODE == 1 && gshift > 0) finishing = true;      // written below, by the pixel's lanes together
                         else if (MODE == 1 && (a.flags & BIHRT_RENDER_COUNTS)) a.fb[pixel] = hits;     // resolved after the reduce
-                        else if (MODE == 1) a.fb[pixel] = pack_colour(hits, nsamp);
+                        else if (MODE == 1) a.fb[pixel] = nsamp <= COLOUR_TABLE_MAX ? s_colour[hits] : pack_colour(hits, nsamp);
                         item = NO_ITEM;
                     }
                 }
@@ -306,7 +311,10 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                         // colours: the pixel's lanes hold all its samples -> one plain store of the final value
                         // (a.fb may be another GPU's framebuffer: the store then travels over NVLink);
                         // counts (a pixel's samples are spread over ranks): one atomic per pixel and warp
-                        if (direct) a.fb[pixel] = pack_colour(sum, nsamp << gshift);
+                        if (direct) {
+                            const int n = nsamp << gshift;
+                            a.fb[pixel] = n <= COLOUR_TABLE_MAX ? s_colour[sum] : pack_colour(sum, n);
+                        }
                         else if (sum) atomicAdd(&a.fb[pixel], sum);
                     }
                 }
@@ -440,8 +448,15 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                     const int px = (int)(pxy & 0xFFFFu), py = (int)(pxy >> 16);
                     const float ru = (a.flags & BIHRT_RENDER_JITTER) ? bihrt_jitter(a.seed, pixel, (uint32_t)(s0 + s), 0) : 0.5f;
                     const float rv = (a.flags & BIHRT_RENDER_JITTER) ? bihrt_jitter(a.seed, pixel, (uint32_t)(s0 + s), 1) : 0.5f;
-                    const float uu = __fdiv_rn(__fadd_rn((float)px, ru), (float)a.w);
-                    const float vv = __fdiv_rn(__fadd_rn((float)py, rv), (float)a.h);
+                    float uu, vv;
+                    if constexpr (MODE == 1) {            // == __fdiv_rn: the launch-constant half of the divide is in s_fb
+                        const float4 k = *reinterpret_cast<const float4*>(s_fb);
+                        uu = camera_div(__fadd_rn((float)px, ru), k.y, k.x);
+                        vv = camera_div(__fadd_rn((float)py, rv), k.w, k.z);
+                    } else {
+                        uu = __fdiv_rn(__fadd_rn((float)px, ru), (float)a.w);
+                        vv = __fdiv_rn(__fadd_rn((float)py, rv), (float)a.h);
+                    }
                     ox = a.cam.origin[0]; oy = a.cam.origin[1]; oz = a.cam.origin[2];
                     dx = __fsub_rn(__fadd_rn(__fadd_rn(a.cam.lower_left[0], __fmul_rn(uu, a.cam.horizontal[0])), __fmul_rn(vv, a.cam.vertical[0])), ox);
                     dy = __fsub_rn(__fadd_rn(__fadd_rn(a.cam.lower_left[1], __fmul_rn(uu, a.cam.horizontal[1])), __fmul_rn(vv, a.cam.vertical[1])), oy);
@@ -463,15 +478,20 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 h.t = RANGE ? thi : (MODE == 0 && a.any_hit) ? a.tmax : FLT_MAX; h.slot = -1; STACK_RESET(); tracing = true;
                 // slab test against the scene box, R/src/CUDAKernels.cu:237-262 (same operation order)
                 bool in = nu > 0 && live;
-                float tMin = __fmul_rn(__fsub_rn(ix < 0.f ? bhi[0] : blo[0], ox), ix);
-                float tMax = __fmul_rn(__fsub_rn(ix < 0.f ? blo[0] : bhi[0], ox), ix);
-                const float tymin = __fmul_rn(__fsub_rn(iy < 0.f ? bhi[1] : blo[1], oy), iy);
-                const float tymax = __fmul_rn(__fsub_rn(iy < 0.f ? blo[1] : bhi[1], oy), iy);
+                float lo0 = blo[0], lo1 = blo[1], lo2 = blo[2], hi0 = bhi[0], hi1 = bhi[1], hi2 = bhi[2];
+                if constexpr (MODE == 1) {
+                    const float4 b0 = *reinterpret_cast<const float4*>(s_fb + 4), b1 = *reinterpret_cast<const float4*>(s_fb + 8);
+                    lo0 = b0.x; lo1 = b0.y; lo2 = b0.z; hi0 = b0.w; hi1 = b1.x; hi2 = b1.y;
+                }
+                float tMin = __fmul_rn(__fsub_rn(ix < 0.f ? hi0 : lo0, ox), ix);
+                float tMax = __fmul_rn(__fsub_rn(ix < 0.f ? lo0 : hi0, ox), ix);
+                const float tymin = __fmul_rn(__fsub_rn(iy < 0.f ? hi1 : lo1, oy), iy);
+                const float tymax = __fmul_rn(__fsub_rn(iy < 0.f ? lo1 : hi1, oy), iy);
                 if ((tMin > tymax) || (tymin > tMax)) in = false;
                 if (tymin > tMin) tMin = tymin;
                 if (tymax < tMax) tMax = tymax;
-                const float tzmin = __fmul_rn(__fsub_rn(iz < 0.f ? bhi[2] : blo[2], oz), iz);
-                const float tzmax = __fmul_rn(__fsub_rn(iz < 0.f ? blo[2] : bhi[2], oz), iz);
+                const float tzmin = __fmul_rn(__fsub_rn(iz < 0.f ? hi2 : lo2, oz), iz);
+                const float tzmax = __fmul_rn(__fsub_rn(iz < 0.f ? lo2 : hi2, oz), iz);
                 if ((tMin > tzmax) || (tzmin > tMax)) in = false;
                 if (tzmin > tMin) tMin = tzmin;
                 if (tzmax < tMax) tMax = tzmax;
@@ -505,16 +525,19 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 // triangles) and 21 % (atrium) against the generic walk alone
                 int oct = OCT_MIXED;
                 if (gshift > 0) {
-                    const bool w = cur != NONE;
-                    const uint32_t xn = __ballot_sync(FULL, w && ix < 0.f), xp = __ballot_sync(FULL, w && ix > 0.f);
-                    const uint32_t yn = __ballot_sync(FULL, w && iy < 0.f), yp = __ballot_sync(FULL, w && iy > 0.f);
-                    const uint32_t zn = __ballot_sync(FULL, w && iz < 0.f), zp = __ballot_sync(FULL, w && iz > 0.f);
-                    if (!((xn && xp) || (yn && yp) || (zn && zp))) oct = (xn != 0) | (yn != 0) << 1 | (zn != 0) << 2;
+                    // one OR over the warp of every walking lane's signs: bit 2k "1/d < 0", bit 2k + 1 "1/d > 0" on axis k;
+                    // the warp mixes signs when both bits of some axis are set
+                    const uint32_t sg = cur == NONE ? 0u : (uint32_t)(ix < 0.f) | (uint32_t)(ix > 0.f) << 1 | (uint32_t)(iy < 0.f) << 2 |
+                                                           (uint32_t)(iy > 0.f) << 3 | (uint32_t)(iz < 0.f) << 4 | (uint32_t)(iz > 0.f) << 5;
+                    const uint32_t any = __reduce_or_sync(FULL, sg);
+                    if ((any & (any >> 1) & 0x15u) == 0) oct = (any & 1u) | (any >> 1 & 2u) | (any >> 2 & 4u);
                 }
                 my_ray[9] = __int_as_float(oct);
             }
-            if (__ballot_sync(FULL, cur != NONE || tracing) == 0 && exhausted &&
-                __ballot_sync(FULL, item != NO_ITEM) == 0) break;
+            // framebuffer renders vote only once the counter has run out (exhausted is warp-uniform: the warp votes together
+            // or not at all); the other modes keep the code they were measured with
+            if (MODE == 1 ? exhausted && __ballot_sync(FULL, cur != NONE || tracing || item != NO_ITEM) == 0
+                          : __ballot_sync(FULL, cur != NONE || tracing) == 0 && exhausted && __ballot_sync(FULL, item != NO_ITEM) == 0) break;
         }
 
         // ================= phase 1: internal nodes =====================================================
