@@ -7,8 +7,10 @@
 //     global atomic counter (or from per-SM queues, 1 spp launches of >= 16 M rays).  Camera modes: an item is a
 //     pixel's sample group -- the samples of a pixel sit in CONSECUTIVE LANES, the warp moves from sample to sample
 //     in lock step and a pixel is written once, as its final colour, by the lane that completes it (possibly into
-//     another GPU's framebuffer: bihrt_render_interleaved_to).  A warp is refilled once every lane's ray has ended: each
-//     lane starts its item's next sample or takes a new item.  An option traces a ray list through a sort permutation
+//     another GPU's framebuffer: bihrt_render_interleaved_to).  A warp is refilled once every lane's ray has ended.
+//     Camera modes refill in lock step: one unit is one packet per sample, lane i traces item i of the unit (padding
+//     pixels sit it out), and lane 0 fetches the warp's next unit when it takes one (a unit ahead; when it is taken in
+//     launches that measure tile costs).  Ray lists keep a pool: a lane that is done takes the warp's next ray.  An option traces a ray list through a sort permutation
 //     (csrc/raysort.cu);
 //   * the tiles of a camera frame are traced in the order k_tile_order derived from the PREVIOUS launch of the same
 //     frame geometry (longest unit per tile, expensive tiles first): the launch is as long as its longest unit;
@@ -132,6 +134,15 @@ __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, fl
     }
 }
 
+// The camera modes' global counter counts units, and lane 0 alone draws them.  atomicAdd on that uniform address is
+// aggregated over the warp by ptxas (vote, leader, shuffle of the result), and the shuffle waits for the atomic's L2 round
+// trip on the spot, even when the result is only read a packet later.  atom.inc cannot be combined that way: with a
+// limit no launch reaches (at most 2^27 units + one fetch per warp) it is a plain increment, and its result is waited
+// for where it is used.
+__device__ __forceinline__ uint32_t unit_inc(uint32_t* p) {
+    uint32_t r; asm volatile("atom.global.inc.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "r"(0x7FFFFFFFu) : "memory"); return r;
+}
+
 // ------------------------------------------------------------------------------------------
 // MODE 0: ray list -> (t, slot, prim);  1: camera -> packed framebuffer;  2: camera -> per-sample hits;
 // 3: ray list with per-ray intervals [tmin, tmax] -> hit records (t, u, v, slot, prim, ng): bihrt_intersect;
@@ -212,15 +223,34 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
     const int nsamp = LIST ? 1 : ((a.s_end - a.s_begin) >> gshift);    // samples per item
     uint32_t my_queue = 0;
     if (a.queues > 1) { asm("mov.u32 %0, %%smid;" : "=r"(my_queue)); my_queue %= (uint32_t)a.queues; }
-    item_t pool_next = 0, pool_end = 0;        // warp-uniform
-    uint32_t pool_xy = 0;                      // warp-uniform, camera modes: first pixel of the pool's tile, x | y << 16
-    long long unit_t0 = 0; uint32_t unit_tile = 0xFFFFFFFFu;   // warp-uniform: start time / tile of the packet being traced
-    bool exhausted = false;                    // warp-uniform: the global counter ran past `total`
+    // ray lists: the warp's pool of items (warp-uniform)
+    item_t pool_next = 0, pool_end = 0;
+    bool exhausted = false;                    // the global counter ran past `total`
+    long long unit_t0 = 0; uint32_t unit_tile = 0xFFFFFFFFu;   // start time / tile of the unit being traced (camera modes: lane 0's)
 
     // lane state
-    item_t item = NO_ITEM;                     // current work item
+    item_t item = NO_ITEM;                     // ray lists: current work item
     int s = 0, s0 = 0;                         // sample of the item being traced, first sample of the item
     uint32_t hits = 0, pixel = 0, pxy = 0;
+    // Camera modes walk their units in lock step: lane i traces item base + i of the warp's unit, so its sample group and
+    // its pixel's place in the unit are launch constants.  A unit starts at a multiple of 32 >> gshift pixels in the tile's
+    // 8x4-block order, whose decode maps every bit of the pixel index to its own bit of x or y: the lane's pixel is the
+    // unit's first pixel plus xy(lane >> gshift), one add.  s counts the unit's samples in step over the warp; a fresh
+    // warp starts at the end of a (non-existent) unit.
+    bool own = false;                          // camera modes: the lane's pixel of the current unit is in the frame
+    uint32_t lane_xy = 0, next = 0;            // camera modes: the lane's pixel offset; lane 0: the prefetched counter value
+    // Lane 0 fetches the warp's next unit when it takes one, so the L2 round trip of the atomic is off the refill's path --
+    // except in launches that measure tile costs for a cost-ordered schedule: their expensive units come first, and a unit
+    // held by a warp that is still tracing a long one waits for it (B200 at 1000 W, 1080p x 1 spp on the 1 M-triangle sphere:
+    // 7066 -> 6197 Mrays/s with the prefetch in every launch; DESIGN §4).  There the unit is fetched when it is taken.
+#define AHEAD (a.tile_cost == nullptr)
+    if constexpr (!LIST) {
+        const uint32_t q = (uint32_t)lane >> gshift;
+        lane_xy = (((q >> 2) & 0x18u) | (q & 7u)) + ((((q >> 5) & 0x1cu) | ((q >> 3) & 3u)) << 16);
+        s0 = a.s_begin + (lane & ((1 << gshift) - 1)) * nsamp;
+        s = nsamp - 1;
+        if (lane == 0 && a.queues <= 1 && AHEAD) next = unit_inc(a.work);     // the warp's first unit
+    }
     // the box tests need all three axes: 1/direction, -origin/direction (plane distance = one FMA) and the absolute rounding
     // margin that goes with it; origin and direction themselves are only needed per axis (plane test) and by the triangle
     // test, and live in shared memory
@@ -235,200 +265,233 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
 #define STACK_PUSH(item) do { stack[sp] = (item); sp++; } while (0)
 #define STACK_POP(e) do { sp--; (e) = stack[sp]; } while (0)
     const uint32_t root_ref = BIH_REF_NODE(0, a.hdr->root_axis);
-    // colours with a pixel's samples in several lanes: the warp moves from sample to sample in lock step, so the lanes
-    // of a pixel hold its complete hit count when they finish and the pixel is written once, without atomics
-    const bool direct = MODE == 1 && gshift > 0 && !(a.flags & BIHRT_RENDER_COUNTS);
     const uint32_t ray_smem = (uint32_t)__cvta_generic_to_shared(my_ray);
+
+    // unit interleave across GPUs (il_count ranks): this rank owns every il_count-th 32-item unit of every tile (runs of
+    // 2^il_cshift units), so all ranks walk all tiles (same locality, perfect balance) and every pixel keeps all its samples
+    // -- and their lane grouping -- on one GPU.  IL_UNIT: the rank's unit lu -> the frame's unit.
+#define IL_UNIT(lu) ((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u)))
+    // Per-SM queues (a.queues > 1): tile t belongs to queue t % queues and every warp of an SM drains its own SM's queue
+    // first, so the warps resident on one SM walk the same one or two tiles and share nodes and triangles in L1; an SM that
+    // runs dry steals from the others.  QUEUE_UNIT sets base to the first item of the unit taken and got to 32, and leaves
+    // both as they are once every queue is empty.  (Macros, like the node phase below: ray lists compile to the code they had.)
+#define QUEUE_UNIT(base, got)                                                                                       \
+    do {                                                                                                            \
+        const uint32_t tshift = 10 + gshift, ushift = 5 + gshift;       /* items / units per tile */                \
+        const item_t ntile = (total + ((item_t(1) << tshift) - 1)) >> tshift;                                       \
+        for (uint32_t k = 0; k < (uint32_t)a.queues; k++) {                                                         \
+            uint32_t q = my_queue + k; if (q >= (uint32_t)a.queues) q -= (uint32_t)a.queues;                        \
+            if (q >= ntile) continue;                                                                               \
+            const uint32_t upt = (1u << ushift) / ilc;                                  /* this rank's units per tile */ \
+            const item_t units = ((ntile - q + a.queues - 1) / a.queues) * upt;         /* of queue q */            \
+            if (ld_relaxed(a.work + q) >= units) continue;                                                          \
+            const uint32_t u = atomicAdd(a.work + q, 1u);                                                           \
+            if (u >= units) continue;                                                                               \
+            const uint32_t lu = u % upt;                                                                            \
+            const item_t b = (((item_t)(u / upt) * a.queues + q) << tshift) + ((item_t)IL_UNIT(lu) << 5);           \
+            if (b < total) { (base) = b; (got) = 32; break; }                                                       \
+        }                                                                                                           \
+    } while (0)
 
     for (;;) {
         // ================= refill: once the whole warp has drained, every lane records its ray and gets the next one ========
-        // A lane moves on to the next SAMPLE of its own item, or takes a new ITEM when its item is done, so the warp starts
-        // each packet together.  (Refilling the idle lanes of a warp that is still walking was measured as a loss with the
-        // children boxes: DESIGN §4.)  Lanes that have nothing left park until the launch ends.
+        // The warp starts each packet together.  (Refilling the idle lanes of a warp that is still walking was measured as a
+        // loss with the children boxes: DESIGN §4.)
         const uint32_t busy = ~__ballot_sync(FULL, cur == NONE);
         if (busy == 0) {
-            bool want_item = false, finishing = false;
-            if (cur == NONE) {
+            if constexpr (LIST) {
+                // ---- ray lists: a lane that has recorded its ray takes the next item of the warp's pool; lanes that have
+                // nothing left park until the launch ends
+                bool want_item = false;
+                if (cur == NONE) {
+                    if (tracing) {                               // record the ray that just ended
+                        tracing = false;
+                        if (RANGE) {
+                            // hit record epilogue: the hit triangle again (48 bytes just read by the walk, likely in L1), u and v
+                            // by the walk's arithmetic on the ray still in shared memory, ng = e1 x e2 (products rounded, no FMA)
+                            const bool hit = h.slot >= 0;
+                            const bool rec = a.out_u || a.out_v || a.out_ng;
+                            float u = 0.f, v = 0.f, gx = 0.f, gy = 0.f, gz = 0.f;
+                            int32_t prim = -1;
+                            if (hit && (rec || a.out_prim)) {
+                                const float4* tq = reinterpret_cast<const float4*>(tris + h.slot);
+                                const float4 q0 = __ldg(tq), q1 = __ldg(tq + 1), q2 = __ldg(tq + 2);
+                                prim = (int32_t)__float_as_uint(q2.y);
+                                if (rec) {
+                                    const float e1x = q0.w, e1y = q1.x, e1z = q1.y, e2x = q1.z, e2y = q1.w, e2z = q2.x;
+                                    const float2 dxy = *reinterpret_cast<const float2*>(my_ray + 6);
+                                    const float dx = dxy.x, dy = dxy.y, dz = my_ray[8];
+                                    float px, py, pz, tx, ty, tz, qx, qy, qz;
+                                    const float inv = __frcp_rn(mt_det(dx, dy, dz, e1x, e1y, e1z, e2x, e2y, e2z, px, py, pz));
+                                    u = mt_u(my_ray[0], my_ray[2], my_ray[4], q0, px, py, pz, inv, tx, ty, tz);
+                                    v = mt_v(dx, dy, dz, e1x, e1y, e1z, tx, ty, tz, inv, qx, qy, qz);
+                                    gx = __fsub_rn(__fmul_rn(e1y, e2z), __fmul_rn(e1z, e2y));
+                                    gy = __fsub_rn(__fmul_rn(e1z, e2x), __fmul_rn(e1x, e2z));
+                                    gz = __fsub_rn(__fmul_rn(e1x, e2y), __fmul_rn(e1y, e2x));
+                                }
+                            }
+                            // (h.t of a miss may be the cut tmax: the record says FLT_MAX)
+                            if (a.out_t) a.out_t[item] = hit ? h.t : FLT_MAX;
+                            if (a.out_slot) a.out_slot[item] = h.slot;
+                            if (a.out_prim) a.out_prim[item] = prim;
+                            if (a.out_u) a.out_u[item] = u;
+                            if (a.out_v) a.out_v[item] = v;
+                            if (a.out_ng) { float* g = a.out_ng + 3 * item; g[0] = gx; g[1] = gy; g[2] = gz; }
+                        } else {
+                            if (a.out_t) a.out_t[item] = h.t;
+                            if (a.out_slot) a.out_slot[item] = h.slot;
+                            if (a.out_prim) a.out_prim[item] = h.slot >= 0 ? (int32_t)tris[h.slot].prim : -1;
+                        }
+                        s++;
+                        if (s == nsamp) item = NO_ITEM;
+                    }
+                    want_item = (item == NO_ITEM);
+                }
+                // hand out new items (warp-uniform control flow)
+                uint32_t want = __ballot_sync(FULL, want_item);
+                while (want && !exhausted) {
+                    if (pool_next >= pool_end) {
+                        // Work comes in units of 32 rays, grouped in chunks of 1024 (see the camera modes below for the
+                        // per-SM queues and the unit interleave across GPUs).
+                        item_t base = NO_ITEM;
+                        uint32_t got = 0;
+                        if (lane == 0) {
+                            const uint32_t ilc = (uint32_t)a.il_count, ili = (uint32_t)a.il_index, ics = (uint32_t)a.il_cshift;
+                            if (a.queues <= 1) {
+                                const item_t fetched = atomicAdd(a.work, 32u); got = 32;
+                                const item_t lu = fetched >> 5;            // this rank's unit -> the frame's unit
+                                base = ilc > 1 ? IL_UNIT(lu) << 5 : fetched;
+                                if (base >= total) base = NO_ITEM;
+                            } else QUEUE_UNIT(base, got);
+                        }
+                        base = __shfl_sync(FULL, base, 0);
+                        got = __shfl_sync(FULL, got, 0);
+                        if (a.tile_cost && unit_tile != 0xFFFFFFFFu) {
+                            // the time between two fetches of the warp is charged to the chunk of the earlier one
+                            if (lane == 0) atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
+                            unit_tile = 0xFFFFFFFFu;
+                        }
+                        if (base == NO_ITEM) { exhausted = true; break; }
+                        pool_next = base;
+                        pool_end = min(base + got, total);
+                        if (a.tile_cost && unit_tile == 0xFFFFFFFFu) {
+                            const uint32_t m = (uint32_t)(base >> 10);
+                            unit_tile = a.tile_order ? __ldg(a.tile_order + m) : m;
+                            unit_t0 = clock64();
+                        }
+                    }
+                    const item_t avail = pool_end - pool_next;
+                    const uint32_t rank = __popc(want & lt);
+                    const bool served = want_item && (item_t)rank < avail;
+                    if (served) {
+                        item = pool_next + rank; s = 0; hits = 0; want_item = false;
+                        if (a.tile_cost) {
+                            // logical item -> ray: chunk (item >> 10) is the chunk traced m-th in cost order
+                            const uint32_t mi = (uint32_t)(item >> 10);
+                            const uint64_t ray = ((uint64_t)(a.tile_order ? __ldg(a.tile_order + mi) : mi) << 10) | (item & 1023u);
+                            item = ray < (uint64_t)a.nrays ? ray : NO_ITEM;      // padding of the last chunk
+                            if (item == NO_ITEM) want_item = true;
+                        }
+                        // sorted ray lists: the i-th item is ray perm[i]; from here on `item` is the ray's own index (load and store)
+                        if (MODE == 0 && a.perm && item != NO_ITEM) item = __ldg(a.perm + item);
+                    }
+                    pool_next += min((item_t)__popc(want), avail);
+                    // lanes that drew a padding ray, or were not served, ask again
+                    want = __ballot_sync(FULL, want_item);
+                }
+            } else {
+                // ---- camera modes: the warp's unit in lock step.  Every lane records its sample; once the unit's last
+                // sample is in, the pixels are written and the warp takes its next unit, 32 items, one per lane.
                 if (tracing) {                                   // record the ray that just ended
                     tracing = false;
                     if (MODE == 1) hits += (h.slot >= 0);
-                    else if (RANGE) {
-                        // hit record epilogue: the hit triangle again (48 bytes just read by the walk, likely in L1), u and v
-                        // by the walk's arithmetic on the ray still in shared memory, ng = e1 x e2 (products rounded, no FMA)
-                        const bool hit = h.slot >= 0;
-                        const bool rec = a.out_u || a.out_v || a.out_ng;
-                        float u = 0.f, v = 0.f, gx = 0.f, gy = 0.f, gz = 0.f;
-                        int32_t prim = -1;
-                        if (hit && (rec || a.out_prim)) {
-                            const float4* tq = reinterpret_cast<const float4*>(tris + h.slot);
-                            const float4 q0 = __ldg(tq), q1 = __ldg(tq + 1), q2 = __ldg(tq + 2);
-                            prim = (int32_t)__float_as_uint(q2.y);
-                            if (rec) {
-                                const float e1x = q0.w, e1y = q1.x, e1z = q1.y, e2x = q1.z, e2y = q1.w, e2z = q2.x;
-                                const float2 dxy = *reinterpret_cast<const float2*>(my_ray + 6);
-                                const float dx = dxy.x, dy = dxy.y, dz = my_ray[8];
-                                float px, py, pz, tx, ty, tz, qx, qy, qz;
-                                const float inv = __frcp_rn(mt_det(dx, dy, dz, e1x, e1y, e1z, e2x, e2y, e2z, px, py, pz));
-                                u = mt_u(my_ray[0], my_ray[2], my_ray[4], q0, px, py, pz, inv, tx, ty, tz);
-                                v = mt_v(dx, dy, dz, e1x, e1y, e1z, tx, ty, tz, inv, qx, qy, qz);
-                                gx = __fsub_rn(__fmul_rn(e1y, e2z), __fmul_rn(e1z, e2y));
-                                gy = __fsub_rn(__fmul_rn(e1z, e2x), __fmul_rn(e1x, e2z));
-                                gz = __fsub_rn(__fmul_rn(e1x, e2y), __fmul_rn(e1y, e2x));
-                            }
-                        }
-                        // (h.t of a miss may be the cut tmax: the record says FLT_MAX)
-                        if (a.out_t) a.out_t[item] = hit ? h.t : FLT_MAX;
-                        if (a.out_slot) a.out_slot[item] = h.slot;
-                        if (a.out_prim) a.out_prim[item] = prim;
-                        if (a.out_u) a.out_u[item] = u;
-                        if (a.out_v) a.out_v[item] = v;
-                        if (a.out_ng) { float* g = a.out_ng + 3 * item; g[0] = gx; g[1] = gy; g[2] = gz; }
-                    } else {
-                        const uint64_t o = MODE == 0 ? item : (uint64_t)pixel * (uint32_t)a.spp + (uint32_t)(s0 + s);
+                    else {
+                        const uint64_t o = (uint64_t)pixel * (uint32_t)a.spp + (uint32_t)(s0 + s);
                         if (a.out_t) a.out_t[o] = h.t;
                         if (a.out_slot) a.out_slot[o] = h.slot;
                         if (a.out_prim) a.out_prim[o] = h.slot >= 0 ? (int32_t)tris[h.slot].prim : -1;
                     }
-                    s++;
-                    if (s == nsamp) {
-                        if (MODE == 1 && gshift > 0) finishing = true;      // written below, by the pixel's lanes together
-                        else if (MODE == 1 && (a.flags & BIHRT_RENDER_COUNTS)) a.fb[pixel] = hits;     // resolved after the reduce
-                        else if (MODE == 1) a.fb[pixel] = nsamp <= COLOUR_TABLE_MAX ? s_colour[hits] : pack_colour(hits, nsamp);
-                        item = NO_ITEM;
-                    }
                 }
-                want_item = (item == NO_ITEM);
-            }
-            if (MODE == 1 && gshift > 0) {
-                // the lanes of one pixel finish together (always, when the warp moves in lock step).  The participants are
-                // named by a ballot taken where the whole warp is converged (the refill block is entered warp-uniformly),
-                // not by __activemask() inside the divergent branch, which promises nothing about convergence.
-                const uint32_t fin = __ballot_sync(FULL, finishing);
-                if (finishing) {
-                    const uint32_t same = __match_any_sync(fin, pixel);
-                    const uint32_t sum = __reduce_add_sync(same, hits);
-                    if (lane == __ffs(same) - 1) {
-                        // colours: the pixel's lanes hold all its samples -> one plain store of the final value
-                        // (a.fb may be another GPU's framebuffer: the store then travels over NVLink);
-                        // counts (a pixel's samples are spread over ranks): one atomic per pixel and warp
-                        if (direct) {
+                if (++s == nsamp) {                              // warp-uniform: the unit is done
+                    if (MODE == 1) {
+                        // The lanes of a pixel finish its last sample together and hold all its hits: the pixel is written
+                        // once, by its first lane.  The warp is converged here (the refill is entered warp-uniformly), so
+                        // the ballot and the shuffles name every lane (ADVICE r1: not __activemask() in a divergent branch).
+                        uint32_t sum = hits;
+                        bool writer = own;
+                        if (gshift > 0) {
+                            const uint32_t gl = 1u << gshift;                     // lanes of a pixel
+                            if (nsamp == 1) sum = __popc(__ballot_sync(FULL, hits) & ((FULL >> (32u - gl)) << (lane & (32u - gl))));
+                            else for (uint32_t o = 1; o < gl; o <<= 1) sum += __shfl_xor_sync(FULL, sum, o);
+                            writer = own && (lane & (gl - 1u)) == 0;
+                        }
+                        if (writer) {
+                            // colours: one plain store of the final value (a.fb may be another GPU's framebuffer: the store
+                            // then travels over NVLink); counts of lane groups (a pixel's samples may be spread over ranks):
+                            // one atomic per pixel and unit; counts of 1-lane pixels are resolved after the reduce
                             const int n = nsamp << gshift;
-                            a.fb[pixel] = n <= COLOUR_TABLE_MAX ? s_colour[sum] : pack_colour(sum, n);
+                            if (!(a.flags & BIHRT_RENDER_COUNTS)) a.fb[pixel] = n <= COLOUR_TABLE_MAX ? s_colour[sum] : pack_colour(sum, n);
+                            else if (gshift == 0) a.fb[pixel] = sum;
+                            else if (sum) atomicAdd(&a.fb[pixel], sum);
                         }
-                        else if (sum) atomicAdd(&a.fb[pixel], sum);
                     }
-                }
-            }
-            // the packet that just drained: its duration is the cost of its tile for the next frame's order
-            if (!LIST && a.tile_cost && unit_tile != 0xFFFFFFFFu) {
-                if (lane == 0) atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
-                unit_tile = 0xFFFFFFFFu;
-            }
-            // hand out new items (warp-uniform control flow)
-            uint32_t want = __ballot_sync(FULL, want_item);
-            while (want && !exhausted) {
-                if (pool_next >= pool_end) {
-                    // Work comes in units of 32 items, grouped in tiles of 32 units (a 32x32-pixel tile / 1024
-                    // rays).  With per-SM queues (a.queues > 1) tile t belongs to queue t % queues and every
-                    // warp of an SM drains its own SM's queue first, so the warps resident on one SM walk the
-                    // same one or two tiles and share nodes and triangles in L1; an SM that runs dry steals
-                    // from the others.  a.queues == 1 is one global counter (one unit per fetch).
-                    item_t base = NO_ITEM;
-                    uint32_t got = 0, unit_m = 0, unit_xy = 0;
+                    // the unit's duration is the cost of its tile for the next frame's order
+                    if (lane == 0 && a.tile_cost && unit_tile != 0xFFFFFFFFu)
+                        atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
+                    // Lane 0 takes the next unit with a pixel in the frame and resolves its first pixel, x | y << 16 (w, h <=
+                    // 65535), or leaves NONE when the work has run out.  Work comes in units of 32 items, grouped in tiles of
+                    // 32 units (a 32x32-pixel tile).  One global counter of units (a.queues == 1, unit_inc): the unit is
+                    // the counter value fetched when the previous unit was taken, and taking it fetches the next one (or,
+                    // without AHEAD, the unit is fetched now).  A warp fetches no further once it has drawn a unit past the
+                    // end, so it draws at most one, and the first item of every unit it maps stays below 2^32 (the launch
+                    // limit's margin of 2^24 items).  Per-SM queues (a.queues > 1) are read when a unit is needed.
+                    uint32_t xy0 = 0xFFFFFFFFu;
                     if (lane == 0) {
-                        // unit interleave across GPUs (il_count ranks): this rank owns every il_count-th 32-item unit
-                        // of every tile, so all ranks walk all tiles (same locality, perfect balance) and every
-                        // pixel keeps all its samples -- and their lane grouping -- on one GPU
                         const uint32_t ilc = (uint32_t)a.il_count, ili = (uint32_t)a.il_index, ics = (uint32_t)a.il_cshift;
-                        if (a.queues <= 1) {
-                            const item_t fetched = atomicAdd(a.work, 32u); got = 32;
-                            const item_t lu = fetched >> 5;            // this rank's unit -> the frame's unit (runs of 2^il_cshift units)
-                            if constexpr (LIST) {
-                                base = ilc > 1 ? ((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u))) << 5 : fetched;
-                                if (base >= total) base = NO_ITEM;
+                        for (;;) {
+                            uint32_t base = NO_ITEM, got;
+                            if (a.queues <= 1) {
+                                // this rank's unit -> the frame's unit, compared as units: past the end of an interleaved
+                                // launch the frame's unit may reach 2^27, where its first item would wrap
+                                if (!AHEAD) next = unit_inc(a.work);
+                                const uint32_t lu = next;
+                                const uint32_t fu = ilc > 1 ? IL_UNIT(lu) : lu;
+                                if (fu >= (total >> 5)) break;
+                                if (AHEAD) next = unit_inc(a.work);
+                                base = fu << 5;
                             } else {
-                                // compared as units: past the end of an interleaved launch the frame's unit may reach 2^27,
-                                // where its first item would wrap
-                                const uint32_t fu = ilc > 1 ? (((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u)) : lu;
-                                if (fu < (total >> 5)) base = fu << 5;
+                                QUEUE_UNIT(base, got);
+                                if (base == NO_ITEM) break;
                             }
-                        } else {
-                            const uint32_t tshift = 10 + gshift, ushift = 5 + gshift;       // items / units per tile
-                            const item_t ntile = (total + ((item_t(1) << tshift) - 1)) >> tshift;
-                            for (uint32_t k = 0; k < (uint32_t)a.queues; k++) {
-                                uint32_t q = my_queue + k; if (q >= (uint32_t)a.queues) q -= (uint32_t)a.queues;
-                                if (q >= ntile) continue;
-                                const uint32_t upt = (1u << ushift) / ilc;                                  // this rank's units per tile
-                                const item_t units = ((ntile - q + a.queues - 1) / a.queues) * upt;         // of queue q
-                                if (ld_relaxed(a.work + q) >= units) continue;
-                                const uint32_t u = atomicAdd(a.work + q, 1u);
-                                if (u >= units) continue;
-                                const uint32_t lu = u % upt;
-                                const item_t b = (((item_t)(u / upt) * a.queues + q) << tshift) + ((item_t)((((lu >> ics) * ilc + ili) << ics) | (lu & ((1u << ics) - 1u))) << 5);
-                                if (b < total) { base = b; got = 32; break; }
-                            }
-                        }
-                        if (!LIST && base != NO_ITEM) {
-                            // the unit's tile, once for its 32 items: m-th in cost order, its row and column (tile < 2^22: the
-                            // multiply-high is the row or one below it), its first pixel packed as x | y << 16 (w, h <= 65535)
-                            const uint32_t mi = (uint32_t)base >> (10 + gshift);
-                            unit_m = a.tile_order ? __ldg(a.tile_order + mi) : mi;
-                            const uint32_t tile = (uint32_t)a.shard_index + unit_m * (uint32_t)a.shard_count;
+                            // the unit's tile: m-th in cost order, its row and column (tile < 2^22: the multiply-high is the
+                            // row or one below it); then the unit's first pixel in the tile (8x4 blocks of 8x4 pixels)
+                            const uint32_t mi = base >> (10 + gshift);
+                            const uint32_t m = a.tile_order ? __ldg(a.tile_order + mi) : mi;
+                            const uint32_t tile = (uint32_t)a.shard_index + m * (uint32_t)a.shard_count;
                             uint32_t row = __umulhi(tile, a.tile_cols_rcp), col = tile - row * a.tile_cols;
                             if (col >= a.tile_cols) { row++; col -= a.tile_cols; }
-                            unit_xy = (col << 5) | (row << 21);
+                            const uint32_t q = (base >> gshift) & 1023u;
+                            const uint32_t xy = ((col << 5) | (row << 21)) + ((((q >> 2) & 0x18u) | (q & 7u)) + ((((q >> 5) & 0x1cu) | ((q >> 3) & 3u)) << 16));
+                            // the first pixel has the unit's smallest x and y: outside the frame, every pixel of the unit
+                            // is padding of an edge tile, and the unit is skipped without setting up a ray
+                            if ((xy & 0xFFFFu) < (uint32_t)a.w && (xy >> 16) < (uint32_t)a.h) {
+                                xy0 = xy;
+                                if (a.tile_cost) { unit_tile = m; unit_t0 = clock64(); }
+                                break;
+                            }
                         }
                     }
-                    base = __shfl_sync(FULL, base, 0);
-                    if (LIST) got = __shfl_sync(FULL, got, 0);
-                    if (LIST && a.tile_cost && unit_tile != 0xFFFFFFFFu) {
-                        // ray lists: the time between two fetches of the warp is charged to the chunk of the earlier one
-                        if (lane == 0) atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
-                        unit_tile = 0xFFFFFFFFu;
-                    }
-                    if (base == NO_ITEM) { exhausted = true; break; }
-                    pool_next = base;
-                    pool_end = LIST ? min(base + got, total) : base + 32u;     // (camera units never straddle the end: whole tiles)
-                    if (!LIST) pool_xy = __shfl_sync(FULL, unit_xy, 0);
-                    if (a.tile_cost && unit_tile == 0xFFFFFFFFu) {
-                        if (LIST) {
-                            const uint32_t m = (uint32_t)(base >> (10 + gshift));
-                            unit_tile = a.tile_order ? __ldg(a.tile_order + m) : m;
-                        } else unit_tile = __shfl_sync(FULL, unit_m, 0);
-                        unit_t0 = clock64();
-                    }
+                    xy0 = __shfl_sync(FULL, xy0, 0);
+                    if (xy0 == 0xFFFFFFFFu) break;               // warp-uniform: no work left
+                    pxy = xy0 + lane_xy;
+                    const uint32_t px = pxy & 0xFFFFu, py = pxy >> 16;
+                    own = px < (uint32_t)a.w && py < (uint32_t)a.h;  // else a padding pixel of an edge tile: sits the unit out
+                    pixel = py * (uint32_t)a.w + px;
+                    s = 0; hits = 0;
                 }
-                const item_t avail = pool_end - pool_next;
-                const uint32_t rank = __popc(want & lt);
-                const bool served = want_item && (item_t)rank < avail;
-                if (served) {
-                    item = pool_next + rank; s = 0; hits = 0; want_item = false;
-                    if (LIST && a.tile_cost) {
-                        // logical item -> ray: chunk (item >> 10) is the chunk traced m-th in cost order
-                        const uint32_t mi = (uint32_t)(item >> 10);
-                        const uint64_t ray = ((uint64_t)(a.tile_order ? __ldg(a.tile_order + mi) : mi) << 10) | (item & 1023u);
-                        item = ray < (uint64_t)a.nrays ? ray : NO_ITEM;      // padding of the last chunk
-                        if (item == NO_ITEM) want_item = true;
-                    }
-                    // sorted ray lists: the i-th item is ray perm[i]; from here on `item` is the ray's own index (load and store)
-                    if (MODE == 0 && a.perm && item != NO_ITEM) item = __ldg(a.perm + item);
-                    if (!LIST) {
-                        // the item's pixel: the unit's first pixel plus the pixel's place in the tile (8x4 blocks of 8x4 pixels)
-                        const uint32_t q = (uint32_t)(item >> gshift) & 1023u;
-                        s0 = a.s_begin + (int)((uint32_t)item & ((1u << gshift) - 1u)) * nsamp;
-                        const uint32_t xy = pool_xy + (((q >> 2) & 0x18u) | (q & 7u)) + ((((q >> 5) & 0x1cu) | ((q >> 3) & 3u)) << 16);
-                        const uint32_t px = xy & 0xFFFFu, py = xy >> 16;
-                        if (px < (uint32_t)a.w && py < (uint32_t)a.h) { pixel = py * (uint32_t)a.w + px; pxy = xy; }
-                        else item = NO_ITEM;                                 // padding pixel of an edge tile
-                        if (item == NO_ITEM) want_item = true;
-                    }
-                }
-                pool_next += min((item_t)__popc(want), avail);
-                // lanes that drew a padding pixel, or were not served, ask again
-                want = __ballot_sync(FULL, want_item);
             }
-            // start the next ray of every idle lane that owns an item
-            if (cur == NONE && item != NO_ITEM) {
+            // start the next ray of every lane that owns an item
+            if (LIST ? cur == NONE && item != NO_ITEM : own) {
                 float ox, oy, oz, dx, dy, dz;
                 float tlo = 0.f, thi = FLT_MAX;           // MODE 3: max(tmin, 0), min(tmax, FLT_MAX)
                 bool live = true;                         // MODE 3: max(tmin, 0) < tmax (false for a NaN bound): else a miss, not traced
@@ -534,10 +597,8 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 }
                 my_ray[9] = __int_as_float(oct);
             }
-            // framebuffer renders vote only once the counter has run out (exhausted is warp-uniform: the warp votes together
-            // or not at all); the other modes keep the code they were measured with
-            if (MODE == 1 ? exhausted && __ballot_sync(FULL, cur != NONE || tracing || item != NO_ITEM) == 0
-                          : __ballot_sync(FULL, cur != NONE || tracing) == 0 && exhausted && __ballot_sync(FULL, item != NO_ITEM) == 0) break;
+            // ray lists end once every lane is idle and the counter has run out (camera warps leave at the fetch above)
+            if (LIST && __ballot_sync(FULL, cur != NONE || tracing) == 0 && exhausted && __ballot_sync(FULL, item != NO_ITEM) == 0) break;
         }
 
         // ================= phase 1: internal nodes =====================================================
@@ -685,6 +746,9 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
             else POP_VALID();
         }
 #undef NODE_PHASE
+#undef QUEUE_UNIT
+#undef AHEAD
+#undef IL_UNIT
 #undef DEBUG_STACK_TRAP
 #undef POP_VALID
 #undef BOX_SLAB

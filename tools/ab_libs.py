@@ -9,6 +9,8 @@ alternates too).  Every run of an arm measures:
   * renders at 1920x1080 (L2 not flushed): the 1 M-triangle sphere and the atrium at 1 spp (1 spp warps span 8x4 pixels),
     the bench's 60-frame orbit around the sphere at 1 spp, the atrium at 4 spp jittered (the smallest pixel groups that
     walk in their ray octant), and the atrium at 4 spp jittered on a quality-mode tree (morton_bits = 63);
+  * per-sample hit records at 1920x1080 (bihrt_render_hits, outputs copied to the host): the 1 M-triangle sphere at
+    1 spp and the atrium at 4 spp jittered;
   * ray lists, device-resident and timed with CUDA events (tools/bench_intersect.py builds them): the atrium's diffuse
     bounce list through bihrt_trace, its shadow list through bihrt_trace_any, and the sphere's 1920x1080 primary list
     through bihrt_intersect with all outputs, one- and two-sided.
@@ -64,6 +66,22 @@ def render_timing(r, cams, spp, reps):
     return {"ms": ms, "mrays_s": W * H * spp / (ms * 1e-3) / 1e6, "crc32": "%08x" % crc}
 
 
+def hits_timing(r, cam, spp, reps):
+    """ms per W x H render_hits call (per-sample t, slot, prim copied to the host; jittered at spp > 1) and a CRC of them."""
+    import numpy as np
+    for _ in range(20):                                      # warm-up, and the tile schedule's history
+        r.render_hits(cam, W, H, spp=spp, jitter=spp > 1)
+    n = max(1, reps // spp)
+    t0 = time.perf_counter()
+    for _ in range(n):
+        out = r.render_hits(cam, W, H, spp=spp, jitter=spp > 1)
+    ms = (time.perf_counter() - t0) * 1e3 / n
+    crc = 0
+    for x in out:
+        crc = zlib.crc32(np.ascontiguousarray(x).tobytes(), crc)
+    return {"ms": ms, "mrays_s": W * H * spp / (ms * 1e-3) / 1e6, "crc32": "%08x" % crc}
+
+
 def list_timing(fn, nrays, reps):
     """ms per call of a ray-list query (CUDA events) and a CRC of all its outputs."""
     import torch
@@ -93,6 +111,7 @@ def timing(reps):
     r.load_models(sphere).build()
     out["sphere_1m_1080p_1spp"] = render_timing(r, [scenes.pinhole_camera(aspect=W / H)], 1, reps)
     out["orbit_1m_1080p_1spp"] = render_timing(r, orbit_cameras(scenes, W, H), 1, reps)
+    out["sphere_1m_1080p_1spp_render_hits"] = hits_timing(r, scenes.pinhole_camera(aspect=W / H), 1, reps)
     prim = bihrt.interval_rays(sphere_primary_list(W, H))
     n = prim.shape[0]
     out["sphere_1m_primary_intersect_all"] = list_timing(lambda: r.intersect(prim, outputs=ALL), n, reps)
@@ -101,6 +120,7 @@ def timing(reps):
     r.load_models(atrium).build()
     out["atrium_1080p_1spp"] = render_timing(r, atrium_cam, 1, reps)
     out["atrium_1080p_4spp"] = render_timing(r, atrium_cam, 4, reps)
+    out["atrium_1080p_4spp_render_hits"] = hits_timing(r, atrium_cam[0], 4, reps)
     shadow, diffuse = atrium_lists(r, W, H)
     out["atrium_diffuse_trace"] = list_timing(lambda: r.trace(diffuse), diffuse.shape[0], reps)
     out["atrium_shadow_trace_any"] = list_timing(lambda: r.trace_any(shadow, tmax=1.0), shadow.shape[0], reps)
