@@ -76,6 +76,8 @@ INTERSECT_ANY = 1
 INTERSECT_TWO_SIDED = 4
 HIT_OUTPUTS = ("t", "u", "v", "slot", "prim", "ng")
 CLOSEST_OUTPUTS = ("d2", "u", "v", "slot", "prim", "q", "ng")
+CLOSEST_K_OUTPUTS = CLOSEST_OUTPUTS + ("count", "total")
+CLOSEST_K_MAX = 64
 
 
 def interval_rays(rays6, tmin=0.0, tmax=np.inf):
@@ -114,7 +116,7 @@ def point_queries(points3, rmax=np.inf):
 ABI_SYMBOLS = [
     "bihrt_version", "bihrt_create", "bihrt_destroy", "bihrt_last_error", "bihrt_set_stream", "bihrt_get_stream", "bihrt_sync",
     "bihrt_set_option", "bihrt_get_stat", "bihrt_scene_load_triangles", "bihrt_scene_update_vertices", "bihrt_scene_load_obj",
-    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_closest_point", "bihrt_winding_number", "bihrt_trace_counted",
+    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_closest_point", "bihrt_closest_k", "bihrt_winding_number", "bihrt_trace_counted",
     "bihrt_render", "bihrt_render_counted", "bihrt_render_shard", "bihrt_render_samples", "bihrt_render_interleaved", "bihrt_render_interleaved_to", "bihrt_framebuffer_ipc_export", "bihrt_framebuffer_ipc_open", "bihrt_framebuffer_ipc_close", "bihrt_framebuffer_ipc_unexport", "bihrt_bih_region", "bihrt_bih_adopt", "bihrt_bih_copy", "bihrt_framebuffer_resolve", "bihrt_render_hits", "bihrt_secondary_rays", "bihrt_framebuffer", "bihrt_framebuffer_read",
     "bihrt_bih_blob_bytes", "bihrt_bih_export", "bihrt_bih_import",
     "bihrt_create_multi", "bihrt_destroy_multi", "bihrt_multi_size", "bihrt_multi_nccl_version", "bihrt_multi_broadcast",
@@ -411,6 +413,41 @@ class Renderer:
         if on_dev:
             self.wait_torch()            # points (and recycled output blocks) were last touched on torch's current stream
         self._check(self._lib.bihrt_closest_point(self._ctx, _ptr(queries4), C.c_int64(n), C.byref(rec)))
+        if on_dev:
+            self.torch_wait()            # device outputs are written asynchronously on the context's stream
+        return res
+
+    def closest_k(self, queries4, k, outputs=CLOSEST_OUTPUTS + ("count",)):
+        """k-nearest-triangle queries (bihrt_closest_k).  queries4 as for closest_point.  Each point's candidates (d2 <=
+        min(rmax^2, FLT_MAX)) ordered by (d2, slot); the first min(k, candidates) fill its rows, the rest read as misses.
+        0 <= k <= CLOSEST_K_MAX.  Returns {name: array} for the requested outputs of d2, u, v, slot, prim (N,k), q, ng (N,k,3),
+        count (N,) rows written and total (N,) all candidates within the radius: numpy for numpy input, torch tensors on the
+        points' device for torch input.  "total" is left out by default: asking for it makes the walk prune at the radius
+        only, so its cost grows with the number of triangles in range."""
+        unknown = set(outputs) - set(CLOSEST_K_OUTPUTS)
+        if unknown:
+            raise ValueError("unknown outputs %s (known: %s)" % (sorted(unknown), ", ".join(CLOSEST_K_OUTPUTS)))
+        k = int(k)
+        if not 0 <= k <= CLOSEST_K_MAX:
+            raise ValueError("k must be in 0 .. %d (got %d)" % (CLOSEST_K_MAX, k))
+        shapes = {"d2": (k,), "u": (k,), "v": (k,), "slot": (k,), "prim": (k,), "q": (k, 3), "ng": (k, 3), "count": (), "total": ()}
+        ints = ("slot", "prim", "count", "total")
+        if isinstance(queries4, np.ndarray):
+            queries4 = np.ascontiguousarray(queries4, dtype=np.float32)
+            n = queries4.size // 4
+            res = {o: np.empty((n,) + shapes[o], np.int32 if o in ints else np.float32) for o in outputs}
+        else:
+            import torch
+            queries4 = queries4.contiguous()
+            n = queries4.numel() // 4
+            res = {o: torch.empty((n,) + shapes[o], dtype=torch.int32 if o in ints else torch.float32, device=queries4.device)
+                   for o in outputs}
+        rec = Closest(**{o: _ptr(res[o]) for o in res if o in CLOSEST_OUTPUTS})
+        on_dev = getattr(queries4, "is_cuda", False)
+        if on_dev:
+            self.wait_torch()            # points (and recycled output blocks) were last touched on torch's current stream
+        self._check(self._lib.bihrt_closest_k(self._ctx, _ptr(queries4), C.c_int64(n), C.c_int32(k), C.byref(rec),
+                                              _ptr(res.get("count")), _ptr(res.get("total"))))
         if on_dev:
             self.torch_wait()            # device outputs are written asynchronously on the context's stream
         return res

@@ -494,40 +494,53 @@ struct OutStage {
     int32_t* prim() const { return (int32_t*)dev[OUT_PRIM]; }
 };
 
-static int stage_outputs(bihrt_ctx* c, int64_t n, size_t front_bytes, float* t, int32_t* slot, int32_t* prim, OutStage& o, uint8_t** front,
-                         float* u = nullptr, float* v = nullptr, float* ng = nullptr, float* q = nullptr) {
-    void* const want[OUT_COUNT] = { t, slot, prim, u, v, ng, q };
-    bool staged[OUT_COUNT];
+// Host staging of outputs of any size: want[k] is the caller's array (NULL: not wanted) of bytes[k] bytes.  A host array gets
+// a block of d_io after the front block (the staged inputs), every block 16-byte aligned; dev[k] is what the kernel writes
+// (the caller's device array, a staging block, or NULL), host[k] the caller's host array it is copied back to (NULL: none).
+static int stage_arrays(bihrt_ctx* c, size_t front_bytes, int count, void* const* want, const size_t* bytes, void** dev, void** host,
+                        uint8_t** front) {
     size_t need = front_bytes + 256;
-    for (int k = 0; k < OUT_COUNT; k++) {
-        staged[k] = want[k] && !is_device_ptr(want[k]);
-        if (staged[k]) need += (size_t)n * out_bytes_per_ray[k] + 16;    // (+16: every staged array starts 16-byte aligned)
-    }
+    for (int k = 0; k < count; k++)
+        if (want[k] && !is_device_ptr(want[k])) need += bytes[k] + 16;    // (+16: every staged array starts 16-byte aligned)
     int rc = ensure_io(c, need);
     if (rc) return rc;
     uint8_t* p = (uint8_t*)c->d_io;
     *front = p;
     p += (front_bytes + 255) / 256 * 256;
-    for (int k = 0; k < OUT_COUNT; k++) {
-        o.dev[k] = want[k]; o.host[k] = nullptr;
-        if (staged[k]) { o.host[k] = want[k]; o.dev[k] = p; p += ((size_t)n * out_bytes_per_ray[k] + 15) / 16 * 16; }
+    for (int k = 0; k < count; k++) {
+        dev[k] = want[k]; host[k] = nullptr;
+        if (want[k] && !is_device_ptr(want[k])) { host[k] = want[k]; dev[k] = p; p += (bytes[k] + 15) / 16 * 16; }
     }
     return BIHRT_OK;
 }
 
-static int unstage_outputs(bihrt_ctx* c, int64_t n, const OutStage& o) {
+static int unstage_arrays(bihrt_ctx* c, int count, void* const* dev, void* const* host, const size_t* bytes) {
     bool any = false;
-    for (int k = 0; k < OUT_COUNT; k++) any |= o.host[k] != nullptr;
+    for (int k = 0; k < count; k++) any |= host[k] != nullptr;
     if (!any) return BIHRT_OK;
     // host outputs: the call is synchronous anyway -- learn first whether the BIH that was traced is valid (a tripped
     // build watchdog makes the kernel trace nothing), and leave the caller's arrays untouched if it is not
     BIHRT_CUDA(c, cudaStreamSynchronize(c->stream));
     int rc = check_status(c);
     if (rc) return rc;
-    for (int k = 0; k < OUT_COUNT; k++)
-        if (o.host[k]) BIHRT_CUDA(c, cudaMemcpyAsync(o.host[k], o.dev[k], (size_t)n * out_bytes_per_ray[k], cudaMemcpyDeviceToHost, c->stream));
+    for (int k = 0; k < count; k++)
+        if (host[k]) BIHRT_CUDA(c, cudaMemcpyAsync(host[k], dev[k], bytes[k], cudaMemcpyDeviceToHost, c->stream));
     BIHRT_CUDA(c, cudaStreamSynchronize(c->stream));
     return BIHRT_OK;
+}
+
+static int stage_outputs(bihrt_ctx* c, int64_t n, size_t front_bytes, float* t, int32_t* slot, int32_t* prim, OutStage& o, uint8_t** front,
+                         float* u = nullptr, float* v = nullptr, float* ng = nullptr, float* q = nullptr) {
+    void* const want[OUT_COUNT] = { t, slot, prim, u, v, ng, q };
+    size_t bytes[OUT_COUNT];
+    for (int k = 0; k < OUT_COUNT; k++) bytes[k] = (size_t)n * out_bytes_per_ray[k];
+    return stage_arrays(c, front_bytes, OUT_COUNT, want, bytes, o.dev, o.host, front);
+}
+
+static int unstage_outputs(bihrt_ctx* c, int64_t n, const OutStage& o) {
+    size_t bytes[OUT_COUNT];
+    for (int k = 0; k < OUT_COUNT; k++) bytes[k] = (size_t)n * out_bytes_per_ray[k];
+    return unstage_arrays(c, OUT_COUNT, o.dev, o.host, bytes);
 }
 
 static int trace_impl(bihrt_ctx* c, const bihrt_ray* rays, int64_t n, float* t, int32_t* slot, int32_t* prim, uint64_t* counters,
@@ -639,6 +652,44 @@ int bihrt_closest_point(bihrt_ctx* c, const bihrt_point_query* pts, int64_t n, c
     a.work = c->d_work; a.status_map = c->d_status_map;
     if ((rc = bihrt_closest_launch(c, a))) return rc;
     return unstage_outputs(c, n, o);
+}
+
+// k-nearest-triangle queries (include/bihrt.h): k_closest_k, csrc/closest.cu.  The record arrays have n*k rows, count and
+// total n entries; host ones are staged like every other output.
+int bihrt_closest_k(bihrt_ctx* c, const bihrt_point_query* pts, int64_t n, int32_t k, const bihrt_closest* rec, int32_t* count,
+                    int32_t* total) {
+    ENTER(c);
+    if (!rec) return bihrt_fail(c, BIHRT_ERR_INVALID, "no output record");
+    if (k < 0 || k > BIHRT_CLOSEST_K_MAX) return bihrt_fail(c, BIHRT_ERR_INVALID, "k = %d outside 0 .. %d", k, BIHRT_CLOSEST_K_MAX);
+    if (n < 0 || (n > 0 && !pts)) return bihrt_fail(c, BIHRT_ERR_INVALID, "bad point array");
+    if (n >= (1ll << 32) - (1ll << 24)) return bihrt_fail(c, BIHRT_ERR_INVALID, "too many points in one call (32-bit work counter)");
+    if (!c->built) return bihrt_fail(c, BIHRT_ERR_STATE, "BIH not built");
+    { int st = check_status(c); if (st) return st; }
+    if (n == 0) return BIHRT_OK;
+    const bool pts_dev = is_device_ptr(pts);
+    if (pts_dev && ((uintptr_t)pts & 15u)) return bihrt_fail(c, BIHRT_ERR_INVALID, "device points must be 16-byte aligned (one 128-bit load per point)");
+    enum { K_D2, K_U, K_V, K_SLOT, K_PRIM, K_Q, K_NG, K_COUNT, K_TOTAL, K_ARRAYS };
+    void* const want[K_ARRAYS] = { rec->d2, rec->u, rec->v, rec->slot, rec->prim, rec->q, rec->ng, count, total };
+    const size_t rows = (size_t)n * (size_t)k;
+    const size_t bytes[K_ARRAYS] = { 4 * rows, 4 * rows, 4 * rows, 4 * rows, 4 * rows, 12 * rows, 12 * rows, 4 * (size_t)n, 4 * (size_t)n };
+    void* dev[K_ARRAYS]; void* host[K_ARRAYS]; uint8_t* front;
+    int rc = stage_arrays(c, pts_dev ? 0 : (size_t)n * sizeof(bihrt_point_query), K_ARRAYS, want, bytes, dev, host, &front);
+    if (rc) return rc;
+    ClosestKArgs a;
+    memset(&a, 0, sizeof a);
+    a.hdr = c->d_hdr; a.nodes = c->d_nodes; a.tris = c->d_tris;
+    if (pts_dev) a.pts = pts;
+    else {
+        BIHRT_CUDA(c, cudaMemcpyAsync(front, pts, (size_t)n * sizeof(bihrt_point_query), cudaMemcpyHostToDevice, c->stream));
+        a.pts = (const bihrt_point_query*)front;
+    }
+    a.n = n; a.k = k;
+    a.out_d2 = (float*)dev[K_D2]; a.out_u = (float*)dev[K_U]; a.out_v = (float*)dev[K_V];
+    a.out_slot = (int32_t*)dev[K_SLOT]; a.out_prim = (int32_t*)dev[K_PRIM]; a.out_q = (float*)dev[K_Q]; a.out_ng = (float*)dev[K_NG];
+    a.out_count = (int32_t*)dev[K_COUNT]; a.out_total = (int32_t*)dev[K_TOTAL];
+    a.work = c->d_work; a.status_map = c->d_status_map;
+    if ((rc = bihrt_closest_k_launch(c, a))) return rc;
+    return unstage_arrays(c, K_ARRAYS, dev, host, bytes);
 }
 
 // Winding numbers (include/bihrt.h): k_winding, csrc/winding.cu.  The far-field table is built here, by the first call with

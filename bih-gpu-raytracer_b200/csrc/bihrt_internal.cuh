@@ -219,6 +219,17 @@ struct ClosestArgs {
     uint32_t* status_map;   // mapped host word: tree of the wrong kind for this kernel
 };
 int bihrt_closest_launch(bihrt_ctx* c, const ClosestArgs& a);
+// closest.cu: bihrt_closest_k (outputs NULL = not wanted; rows i*k + j, q and ng 3 floats per row)
+struct ClosestKArgs {
+    const BihHeader* hdr; const BihNode* nodes; const BihTri* tris;
+    const bihrt_point_query* pts; int64_t n; int32_t k;
+    float* out_d2; float* out_u; float* out_v; int32_t* out_slot; int32_t* out_prim; float* out_q; float* out_ng;
+    int32_t* out_count;
+    int32_t* out_total;     // non-NULL: count every candidate, so the walk prunes at the radius only
+    uint32_t* work;         // persistent-kernel work counter
+    uint32_t* status_map;   // mapped host word: tree of the wrong kind for this kernel
+};
+int bihrt_closest_k_launch(bihrt_ctx* c, const ClosestKArgs& a);
 // winding.cu: bihrt_winding_number.  Far-field table: per node slot, the order-2 expansion of each child about its box centre,
 // WTAB_FLOATS floats per child (N[3], M[3][3] row-major, Q[i][jk] for jk = 00 01 02 11 12 22, 2 unused).
 #define WTAB_FLOATS 32

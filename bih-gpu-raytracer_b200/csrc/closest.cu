@@ -1,5 +1,6 @@
 // Closest-point queries on sm_100a (bihrt_closest_point, include/bihrt.h): for every point, the triangle nearest to it within
-// the point's own search radius, and where on it.
+// the point's own search radius, and where on it; and k-nearest-triangle queries (bihrt_closest_k, k_closest_k below), the
+// same walk with a list of the k best in place of the best.
 //
 // Kernel shape
 //   * persistent warps (grid = SMs x the resident blocks of 4 warps); a warp takes units of 32 points from one global atomic
@@ -205,6 +206,137 @@ __global__ void __launch_bounds__(CLOSEST_THREADS, CLOSEST_MIN_BLOCKS) k_closest
     }
 }
 
+// k-nearest-triangle queries (bihrt_closest_k): k_closest's walk with a list in place of the best.  Each lane keeps its
+// point's best candidates as a sorted list of up to k keys (d2 bits << 32 | slot) in local memory; d2 is never negative or
+// NaN, so the keys order exactly as (d2, slot) does.  A candidate (d2 <= the radius cut) enters while the list is short or when
+// its key is below the k-th one.  Without out_total the cut is min(radius cut, k-th d2) once the list is full, so boxes are
+// pruned as k_closest prunes them at k = 1; with out_total it stays the radius cut and every candidate is counted.  Pruning is
+// strict (bound > cut), so a triangle that ties the k-th d2 with a smaller slot is still reached: by the margin argument of
+// DESIGN.md section 8 the result is brute force's.  The rows are recomputed at the end from the kept slots.
+template <bool Q>
+__global__ void __launch_bounds__(CLOSEST_THREADS, CLOSEST_MIN_BLOCKS) k_closest_k(ClosestKArgs a) {
+    constexpr int STACK_DEPTH = Q ? STACK_DEPTH_QUALITY : STACK_DEPTH_PARITY;
+    if (a.hdr->status != 0) return;             // the build's device watchdog tripped (the host reports it)
+    if ((a.hdr->quality != 0) != Q) {           // a tree of the other kind
+        if (blockIdx.x == 0 && threadIdx.x == 0 && a.status_map) *a.status_map = 0x100u;
+        return;
+    }
+    const uint32_t nu = a.hdr->nu;
+    const float lx = a.hdr->lo[0], ly = a.hdr->lo[1], lz = a.hdr->lo[2], hx = a.hdr->hi[0], hy = a.hdr->hi[1], hz = a.hdr->hi[2];
+    const float smag = fmaxf(fmaxf(fmaxf(fabsf(lx), fabsf(ly)), fmaxf(fabsf(lz), fabsf(hx))), fmaxf(fabsf(hy), fabsf(hz)));
+    const uint32_t root_ref = BIH_REF_NODE(0, a.hdr->root_axis);
+    const float4* __restrict__ nodes = reinterpret_cast<const float4*>(a.nodes);
+    const float4* __restrict__ tris = reinterpret_cast<const float4*>(a.tris);
+    const int lane = threadIdx.x & 31;
+    const int k = a.k;
+    const bool prune_k = a.out_total == nullptr;
+    uint2 stack[STACK_DEPTH];                   // (child reference, its lower bound)
+    unsigned long long list[BIHRT_CLOSEST_K_MAX];   // the best keys so far, ascending
+
+    for (;;) {
+        uint32_t base = 0;
+        if (lane == 0) base = atomicAdd(a.work, 32u);
+        base = __shfl_sync(FULL, base, 0);
+        if ((uint64_t)base >= (uint64_t)a.n) break;
+        const uint64_t i = (uint64_t)base + (uint32_t)lane;
+        if (i < (uint64_t)a.n) {
+            const float4 P = __ldg(reinterpret_cast<const float4*>(a.pts) + i);
+            const float px = P.x, py = P.y, pz = P.z;
+            const bool live = P.w >= 0.f && fabsf(px) <= FLT_MAX && fabsf(py) <= FLT_MAX && fabsf(pz) <= FLT_MAX;
+            const float rcut = fminf(__fmul_rn(P.w, P.w), FLT_MAX);   // min(fl(rmax^2), FLT_MAX)
+            float cut = rcut;                                         // the pruning bound
+            int cnt = 0;                                              // keys in the list
+            uint32_t tot = 0;                                         // candidates met
+            unsigned long long kkey = k > 0 ? ~0ull : 0ull;           // the k-th key once the list is full: below it enters
+            const float m = __fmul_rn(CLOSEST_EPS, fmaxf(smag, fmaxf(fmaxf(fabsf(px), fabsf(py)), fabsf(pz))));
+            uint32_t cur = NONE;
+            if (live && (k > 0 || !prune_k) && nu > 0 && !(box_d2(lx, ly, lz, hx, hy, hz, px, py, pz, m) > cut))
+                cur = nu == 1 ? BIH_REF_LEAFREF(0) : root_ref;
+            int sp = 0;
+            while (cur != NONE) {
+                if (cur & BIH_REF_LEAF) {
+                    const float4* tp = tris + 3 * (size_t)BIH_REF_INDEX(cur);
+                    for (;;) {
+                        const float4 q0 = __ldg(tp), q1 = __ldg(tp + 1), q2 = __ldg(tp + 2);
+                        float u, v;
+                        const float d2 = pt_tri(px, py, pz, q0.x, q0.y, q0.z, q0.w, q1.x, q1.y, q1.z, q1.w, q2.x, u, v);
+                        if (d2 <= rcut) {
+                            tot++;
+                            const unsigned long long key = (unsigned long long)__float_as_uint(d2) << 32 | __float_as_uint(q2.w);
+                            if (key < kkey) {
+                                // insertion from the free place (the last one when full: the k-th key drops out)
+                                int j = cnt < k ? cnt++ : k - 1;
+                                for (; j > 0; j--) {
+                                    const unsigned long long e = list[j - 1];
+                                    if (e < key) break;
+                                    list[j] = e;
+                                }
+                                list[j] = key;
+                                if (cnt == k) {
+                                    kkey = list[k - 1];
+                                    if (prune_k) cut = __uint_as_float((uint32_t)(kkey >> 32));
+                                }
+                            }
+                        }
+                        if (__float_as_uint(q2.z) & 1u) break;     // last triangle of the leaf
+                        tp += 3;
+                    }
+                    cur = NONE;
+                } else {
+                    const float4* np = nodes + 4 * (size_t)BIH_REF_INDEX(cur);
+                    const float4 nd = __ldg(np), b0 = __ldg(np + 1), b1 = __ldg(np + 2), b2 = __ldg(np + 3);
+                    const float bl = box_d2(b0.x, b0.y, b0.z, b0.w, b1.x, b1.y, px, py, pz, m);
+                    const float br = box_d2(b1.z, b1.w, b2.x, b2.y, b2.z, b2.w, px, py, pz, m);
+                    const bool rfirst = br < bl;                   // the nearer child first; the left one on equal bounds
+                    const float bn = rfirst ? br : bl, bf = rfirst ? bl : br;
+                    const uint32_t rn = __float_as_uint(rfirst ? nd.w : nd.z), rf = __float_as_uint(rfirst ? nd.z : nd.w);
+                    if (bn > cut) cur = NONE;
+                    else {
+                        if (!(bf > cut)) { stack[sp] = make_uint2(rf, __float_as_uint(bf)); sp++; }
+                        cur = rn;
+                    }
+                }
+                if (cur == NONE) {
+                    while (sp > 0) {
+                        sp--;
+                        const uint2 e = stack[sp];
+                        if (!(__uint_as_float(e.y) > cut)) { cur = e.x; break; }
+                    }
+                }
+            }
+            // the rows: each kept triangle again, by the walk's own function; misses after them
+            for (int j = 0; j < k; j++) {
+                float d2 = FLT_MAX, u = 0.f, v = 0.f, qx = 0.f, qy = 0.f, qz = 0.f, gx = 0.f, gy = 0.f, gz = 0.f;
+                int32_t slot = -1, prim = -1;
+                if (j < cnt) {
+                    const unsigned long long key = list[j];
+                    d2 = __uint_as_float((uint32_t)(key >> 32));
+                    slot = (int32_t)(uint32_t)key;
+                    const float4* tp = tris + 3 * (size_t)(uint32_t)key;
+                    const float4 q0 = __ldg(tp), q1 = __ldg(tp + 1), q2 = __ldg(tp + 2);
+                    const float e1x = q0.w, e1y = q1.x, e1z = q1.y, e2x = q1.z, e2y = q1.w, e2z = q2.x;
+                    pt_tri(px, py, pz, q0.x, q0.y, q0.z, e1x, e1y, e1z, e2x, e2y, e2z, u, v);
+                    pt_q(px, py, pz, q0.x, q0.y, q0.z, e1x, e1y, e1z, e2x, e2y, e2z, u, v, qx, qy, qz);
+                    gx = __fsub_rn(__fmul_rn(e1y, e2z), __fmul_rn(e1z, e2y));
+                    gy = __fsub_rn(__fmul_rn(e1z, e2x), __fmul_rn(e1x, e2z));
+                    gz = __fsub_rn(__fmul_rn(e1x, e2y), __fmul_rn(e1y, e2x));
+                    prim = (int32_t)__float_as_uint(q2.y);
+                }
+                const uint64_t row = i * (uint64_t)k + (uint64_t)j;
+                if (a.out_d2) a.out_d2[row] = d2;
+                if (a.out_u) a.out_u[row] = u;
+                if (a.out_v) a.out_v[row] = v;
+                if (a.out_slot) a.out_slot[row] = slot;
+                if (a.out_prim) a.out_prim[row] = prim;
+                if (a.out_q) { float* g = a.out_q + 3 * row; g[0] = qx; g[1] = qy; g[2] = qz; }
+                if (a.out_ng) { float* g = a.out_ng + 3 * row; g[0] = gx; g[1] = gy; g[2] = gz; }
+            }
+            if (a.out_count) a.out_count[i] = cnt;
+            if (a.out_total) a.out_total[i] = (int32_t)tot;
+        }
+    }
+}
+
 template <bool Q>
 static int launch(bihrt_ctx* c, const ClosestArgs& a) {
     int per_sm = 0;
@@ -219,4 +351,20 @@ static int launch(bihrt_ctx* c, const ClosestArgs& a) {
 
 int bihrt_closest_launch(bihrt_ctx* c, const ClosestArgs& a) {
     return c->built_quality ? launch<true>(c, a) : launch<false>(c, a);
+}
+
+template <bool Q>
+static int launch_k(bihrt_ctx* c, const ClosestKArgs& a) {
+    int per_sm = 0;
+    BIHRT_CUDA(c, cudaOccupancyMaxActiveBlocksPerMultiprocessor(&per_sm, k_closest_k<Q>, CLOSEST_THREADS, 0));
+    if (per_sm < 1) per_sm = 1;
+    BIHRT_CUDA(c, cudaMemsetAsync(a.work, 0, 4, c->stream));
+    k_closest_k<Q><<<c->sm_count * per_sm, CLOSEST_THREADS, 0, c->stream>>>(a);
+    c->kernel_launches += 1;
+    BIHRT_CUDA(c, cudaGetLastError());
+    return BIHRT_OK;
+}
+
+int bihrt_closest_k_launch(bihrt_ctx* c, const ClosestKArgs& a) {
+    return c->built_quality ? launch_k<true>(c, a) : launch_k<false>(c, a);
 }

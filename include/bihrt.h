@@ -273,6 +273,28 @@ typedef struct bihrt_closest {
     float*   ng;    /* [3n] geometric normal e1 x e2 of that triangle, as bihrt_hits.ng */
 } bihrt_closest;
 BIHRT_API int bihrt_closest_point(bihrt_ctx* ctx, const bihrt_point_query* pts, int64_t n, const bihrt_closest* out);
+/* ---- k-nearest-triangle queries: the k triangles nearest to a point within the point's own search radius, nearest first, and
+ *      the number of all triangles within that radius.
+ *      Points, the distance function and the candidates are those of bihrt_closest_point: a triangle is a candidate when its
+ *      d2 <= min(fl(rmax*rmax), FLT_MAX); a query with a NaN or negative rmax, or a NaN or infinite coordinate, has none and is
+ *      not walked.
+ *      Result for point i: its candidates ordered by (d2, slot) ascending, ties to the smaller slot; the first min(k, candidates)
+ *      of them go to rows i*k + 0, 1, ... of the arrays of rec (each row as bihrt_closest_point's record: d2, u, v, slot, prim,
+ *      q, ng).  The rows after them hold the miss record (d2 = FLT_MAX, slot = prim = -1, u = v = q = ng = 0).  count[i] is
+ *      the number of rows written; total[i] the number of ALL candidates of point i, also where that is more than k (a radius
+ *      query whose total[i] > k overflowed: ask again with a larger k).  Every output EQUALS BRUTE FORCE OVER ALL SLOTS BIT FOR
+ *      BIT, on parity, quality-mode and refit trees alike; with k == 1 every row is bihrt_closest_point's record.
+ *      Cost: without total the walk prunes at the current k-th best (d2, slot), like bihrt_closest_point at k = 1.  With total
+ *      it prunes at the radius only, so it visits every leaf that holds a triangle in range: the records are the same, but the
+ *      cost grows with the number of triangles within the radius (rmax = +inf visits every leaf).
+ *      k == 0 writes no rows: with total it counts the triangles within the radius, without it the call only fills count with 0.
+ *      rec: arrays of n*k entries (q and ng: 3*n*k floats), any of them NULL; count, total: n entries, either NULL.  Each one
+ *      host or device.  pts, staging, synchronisation, watchdog and replica behaviour as bihrt_closest_point.
+ *      Errors: those of bihrt_closest_point, and BIHRT_ERR_INVALID for k < 0, k > BIHRT_CLOSEST_K_MAX or rec == NULL;
+ *      BIHRT_ERR_NOMEM when the staging buffer of host outputs cannot be allocated. ------------------------------------------- */
+#define BIHRT_CLOSEST_K_MAX 64
+BIHRT_API int bihrt_closest_k(bihrt_ctx* ctx, const bihrt_point_query* pts, int64_t n, int32_t k, const bihrt_closest* rec,
+                              int32_t* count, int32_t* total);
 /* ---- winding-number queries: inside / outside of closed meshes, and with bihrt_closest_point a signed distance.
  *      w(p) = (1/4pi) x the sum over all triangles of the signed solid angle the triangle subtends at p (the generalized winding
  *      number, Jacobson et al. 2013): 1 inside and 0 outside a closed mesh wound counter-clockwise seen from outside (the
