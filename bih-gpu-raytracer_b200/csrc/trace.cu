@@ -9,9 +9,11 @@
 //     in lock step and a pixel is written once, as its final colour, by the lane that completes it (possibly into
 //     another GPU's framebuffer: bihrt_render_interleaved_to).  A warp is refilled once every lane's ray has ended.
 //     Camera modes refill in lock step: one unit is one packet per sample, lane i traces item i of the unit (padding
-//     pixels sit it out), and lane 0 fetches the warp's next unit when it takes one (a unit ahead; when it is taken in
-//     launches that measure tile costs).  Ray lists keep a pool: a lane that is done takes the warp's next ray.  An option traces a ray list through a sort permutation
-//     (csrc/raysort.cu);
+//     pixels sit it out).  From the global counter the warp takes UNIT_BATCH units at a time: lane j resolves unit j of
+//     the batch to its first pixel, and a packet takes the lowest unit left with one shared-memory load; lane 0 fetches
+//     the next batch when it takes one.  Launches that measure tile costs and per-SM queues take one unit at a time,
+//     resolved by lane 0 (fetched when it is taken).  Ray lists keep a pool: a lane that is done takes the warp's next
+//     ray.  An option traces a ray list through a sort permutation (csrc/raysort.cu);
 //   * the tiles of a camera frame are traced in the order k_tile_order derived from the PREVIOUS launch of the same
 //     frame geometry (longest unit per tile, expensive tiles first): the launch is as long as its longest unit;
 //   * every lane walks its own ray with a short stack of 16-byte items (child reference + the three
@@ -134,13 +136,31 @@ __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, fl
     }
 }
 
-// The camera modes' global counter counts units, and lane 0 alone draws them.  atomicAdd on that uniform address is
-// aggregated over the warp by ptxas (vote, leader, shuffle of the result), and the shuffle waits for the atomic's L2 round
-// trip on the spot, even when the result is only read a packet later.  atom.inc cannot be combined that way: with a
-// limit no launch reaches (at most 2^27 units + one fetch per warp) it is a plain increment, and its result is waited
-// for where it is used.
+// The camera modes' global counter counts batches of units (units, in launches that measure tile costs), and lane 0 alone
+// draws them.  atomicAdd on that uniform address is aggregated over the warp by ptxas (vote, leader, shuffle of the
+// result), and the shuffle waits for the atomic's L2 round trip on the spot, even when the result is only read a packet
+// later.  atom.inc cannot be combined that way: with a limit no launch reaches (at most 2^27 units + one fetch per warp)
+// it is a plain increment, and its result is waited for where it is used.
 __device__ __forceinline__ uint32_t unit_inc(uint32_t* p) {
     uint32_t r; asm volatile("atom.global.inc.u32 %0, [%1], %2;" : "=r"(r) : "l"(p), "r"(0x7FFFFFFFu) : "memory"); return r;
+}
+
+// Units a camera warp takes per fetch of the global counter (a power of two <= 32).  Lane j resolves unit j of the batch,
+// so a packet's hand-out is one shared-memory load.  Larger batches spread the units in flight over more of the frame
+// (warps x UNIT_BATCH units), and the walks lose locality faster than the refill saves instructions: B200 at 1000 W,
+// 3840x2160 x 16 spp on the 1 M-triangle sphere, 2 / 4 / 8 / 16 units: +3.7 / +2.6 / -1.4 / -7.7 % against one unit per
+// fetch (DESIGN §4).
+constexpr uint32_t UNIT_BATCH = 2;
+
+// First pixel, x | y << 16 (w, h <= 65535), of the camera unit whose first item is `base`, in the shard's m-th tile.  The
+// tile's row comes from a launch-time reciprocal of the tiles per row (tile < 2^22: the multiply-high is the row or one
+// below it); the unit's place in the tile from its item index (8x4 blocks of 8x4 pixels).
+__device__ __forceinline__ uint32_t unit_first_pixel(const TraceArgs& a, uint32_t m, uint32_t base, int gshift) {
+    const uint32_t tile = (uint32_t)a.shard_index + m * (uint32_t)a.shard_count;
+    uint32_t row = __umulhi(tile, a.tile_cols_rcp), col = tile - row * a.tile_cols;
+    if (col >= a.tile_cols) { row++; col -= a.tile_cols; }
+    const uint32_t q = (base >> gshift) & 1023u;
+    return ((col << 5) | (row << 21)) + ((((q >> 2) & 0x18u) | (q & 7u)) + ((((q >> 5) & 0x1cu) | ((q >> 3) & 3u)) << 16));
 }
 
 // ------------------------------------------------------------------------------------------
@@ -238,18 +258,20 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
     // unit's first pixel plus xy(lane >> gshift), one add.  s counts the unit's samples in step over the warp; a fresh
     // warp starts at the end of a (non-existent) unit.
     bool own = false;                          // camera modes: the lane's pixel of the current unit is in the frame
-    uint32_t lane_xy = 0, next = 0;            // camera modes: the lane's pixel offset; lane 0: the prefetched counter value
-    // Lane 0 fetches the warp's next unit when it takes one, so the L2 round trip of the atomic is off the refill's path --
-    // except in launches that measure tile costs for a cost-ordered schedule: their expensive units come first, and a unit
-    // held by a warp that is still tracing a long one waits for it (B200 at 1000 W, 1080p x 1 spp on the 1 M-triangle sphere:
-    // 7066 -> 6197 Mrays/s with the prefetch in every launch; DESIGN §4).  There the unit is fetched when it is taken.
-#define AHEAD (a.tile_cost == nullptr)
+    uint32_t lane_xy = 0, next = 0;            // camera modes: the lane's pixel offset; lane 0: the prefetched batch
+    uint32_t batch = 0;                        // BATCHED: the units of the warp's batch left to trace (bit j: unit j)
+    // One global counter (a.queues <= 1) counts batches of UNIT_BATCH units, and lane 0 fetches the warp's next batch when it
+    // takes one, so the L2 round trip of the atomic is off the refill's path -- except in launches that measure tile costs
+    // for a cost-ordered schedule: their expensive units come first, and a unit held by a warp that is still tracing a long
+    // one waits for it (B200 at 1000 W, 1080p x 1 spp on the 1 M-triangle sphere: 7066 -> 6197 Mrays/s with the prefetch in
+    // every launch; DESIGN §4).  There, and with per-SM queues, one unit is fetched when it is taken.
+#define BATCHED (a.queues <= 1 && a.tile_cost == nullptr)
     if constexpr (!LIST) {
         const uint32_t q = (uint32_t)lane >> gshift;
         lane_xy = (((q >> 2) & 0x18u) | (q & 7u)) + ((((q >> 5) & 0x1cu) | ((q >> 3) & 3u)) << 16);
         s0 = a.s_begin + (lane & ((1 << gshift) - 1)) * nsamp;
         s = nsamp - 1;
-        if (lane == 0 && a.queues <= 1 && AHEAD) next = unit_inc(a.work);     // the warp's first unit
+        if (lane == 0 && BATCHED) next = unit_inc(a.work);                     // the warp's first batch
     }
     // the box tests need all three axes: 1/direction, -origin/direction (plane distance = one FMA) and the absolute rounding
     // margin that goes with it; origin and direction themselves are only needed per axis (plane test) and by the triangle
@@ -435,53 +457,70 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                             else if (sum) atomicAdd(&a.fb[pixel], sum);
                         }
                     }
-                    // the unit's duration is the cost of its tile for the next frame's order
-                    if (lane == 0 && a.tile_cost && unit_tile != 0xFFFFFFFFu)
-                        atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
-                    // Lane 0 takes the next unit with a pixel in the frame and resolves its first pixel, x | y << 16 (w, h <=
-                    // 65535), or leaves NONE when the work has run out.  Work comes in units of 32 items, grouped in tiles of
-                    // 32 units (a 32x32-pixel tile).  One global counter of units (a.queues == 1, unit_inc): the unit is
-                    // the counter value fetched when the previous unit was taken, and taking it fetches the next one (or,
-                    // without AHEAD, the unit is fetched now).  A warp fetches no further once it has drawn a unit past the
-                    // end, so it draws at most one, and the first item of every unit it maps stays below 2^32 (the launch
-                    // limit's margin of 2^24 items).  Per-SM queues (a.queues > 1) are read when a unit is needed.
+                    // The warp takes its next unit with a pixel in the frame, as the unit's first pixel x | y << 16, or NONE
+                    // when the work has run out.  Work comes in units of 32 items, grouped in tiles of 32 << gshift units (a
+                    // 32x32-pixel tile).  The first pixel has the unit's smallest x and y: outside the frame, every pixel of
+                    // the unit is padding of an edge tile, and the unit is skipped without setting up a ray.  This rank's unit
+                    // lu maps to the frame's unit fu, compared with the unit count as units: past the end of an interleaved
+                    // launch fu may reach 2^27, where its first item would wrap.
+                    const uint32_t ilc = (uint32_t)a.il_count, ili = (uint32_t)a.il_index, ics = (uint32_t)a.il_cshift;
+                    __shared__ uint32_t s_unit_xy[TRACE_THREADS];           // lane j: the first pixel of the batch's unit j
                     uint32_t xy0 = 0xFFFFFFFFu;
-                    if (lane == 0) {
-                        const uint32_t ilc = (uint32_t)a.il_count, ili = (uint32_t)a.il_index, ics = (uint32_t)a.il_cshift;
+                    if (batch == 0 && BATCHED) {
+                        // Batch b, the counter value lane 0 fetched when the warp took its previous batch, holds this rank's
+                        // units b * UNIT_BATCH + j; lane j resolves unit j, and the units with a pixel in the frame are handed
+                        // out lowest first, one per packet.  Taking a batch fetches the next one.  fu grows with lu, so a
+                        // batch whose first unit is past the end is the warp's last fetch, and one of padding units only (the
+                        // bottom row of edge tiles) is skipped.  The counter ends at most one batch per warp past the last
+                        // (UNIT_BATCH x 32 items per warp, far inside the launch limit's margin of 2^24 items); the pixel a
+                        // lane resolves for a unit past the end (its first item may wrap) is never used.  The tile order is
+                        // the identity here: the launch sets it only together with tile costs.
                         for (;;) {
-                            uint32_t base = NO_ITEM, got;
-                            if (a.queues <= 1) {
-                                // this rank's unit -> the frame's unit, compared as units: past the end of an interleaved
-                                // launch the frame's unit may reach 2^27, where its first item would wrap
-                                if (!AHEAD) next = unit_inc(a.work);
-                                const uint32_t lu = next;
-                                const uint32_t fu = ilc > 1 ? IL_UNIT(lu) : lu;
-                                if (fu >= (total >> 5)) break;
-                                if (AHEAD) next = unit_inc(a.work);
-                                base = fu << 5;
-                            } else {
-                                QUEUE_UNIT(base, got);
-                                if (base == NO_ITEM) break;
-                            }
-                            // the unit's tile: m-th in cost order, its row and column (tile < 2^22: the multiply-high is the
-                            // row or one below it); then the unit's first pixel in the tile (8x4 blocks of 8x4 pixels)
-                            const uint32_t mi = base >> (10 + gshift);
-                            const uint32_t m = a.tile_order ? __ldg(a.tile_order + mi) : mi;
-                            const uint32_t tile = (uint32_t)a.shard_index + m * (uint32_t)a.shard_count;
-                            uint32_t row = __umulhi(tile, a.tile_cols_rcp), col = tile - row * a.tile_cols;
-                            if (col >= a.tile_cols) { row++; col -= a.tile_cols; }
-                            const uint32_t q = (base >> gshift) & 1023u;
-                            const uint32_t xy = ((col << 5) | (row << 21)) + ((((q >> 2) & 0x18u) | (q & 7u)) + ((((q >> 5) & 0x1cu) | ((q >> 3) & 3u)) << 16));
-                            // the first pixel has the unit's smallest x and y: outside the frame, every pixel of the unit
-                            // is padding of an edge tile, and the unit is skipped without setting up a ray
-                            if ((xy & 0xFFFFu) < (uint32_t)a.w && (xy >> 16) < (uint32_t)a.h) {
-                                xy0 = xy;
-                                if (a.tile_cost) { unit_tile = m; unit_t0 = clock64(); }
-                                break;
-                            }
+                            const uint32_t lu = __shfl_sync(FULL, next, 0) * UNIT_BATCH + (uint32_t)lane;
+                            const uint32_t fu = ilc > 1 ? IL_UNIT(lu) : lu;
+                            const bool in = (uint32_t)lane < UNIT_BATCH && fu < (total >> 5);
+                            if (!(__ballot_sync(FULL, in) & 1u)) break;
+                            if (lane == 0) next = unit_inc(a.work);
+                            const uint32_t xy = unit_first_pixel(a, fu >> (5 + gshift), fu << 5, gshift);
+                            s_unit_xy[threadIdx.x] = xy;
+                            __syncwarp();
+                            batch = __ballot_sync(FULL, in && (xy & 0xFFFFu) < (uint32_t)a.w && (xy >> 16) < (uint32_t)a.h);
+                            if (batch) break;
                         }
                     }
-                    xy0 = __shfl_sync(FULL, xy0, 0);
+                    if (batch) {                                 // (batched launches only) the batch's next unit
+                        xy0 = s_unit_xy[(threadIdx.x & ~31u) + __ffs(batch) - 1];
+                        batch &= batch - 1;
+                    } else if (!BATCHED) {
+                        // Lane 0 takes one unit at a time: from the global counter when it is needed (launches that
+                        // measure tile costs), or from the per-SM queues (a.queues > 1); the unit's tile is m-th in cost order.
+                        // The unit's duration is the cost of its tile for the next frame's order.
+                        if (lane == 0 && a.tile_cost && unit_tile != 0xFFFFFFFFu)
+                            atomicMax(a.tile_cost + unit_tile, (uint32_t)min((unsigned long long)(clock64() - unit_t0) >> 8, 0xFFFFFFFFull));
+                        if (lane == 0) {
+                            for (;;) {
+                                uint32_t base = NO_ITEM, got;
+                                if (a.queues <= 1) {
+                                    const uint32_t lu = unit_inc(a.work);
+                                    const uint32_t fu = ilc > 1 ? IL_UNIT(lu) : lu;
+                                    if (fu >= (total >> 5)) break;
+                                    base = fu << 5;
+                                } else {
+                                    QUEUE_UNIT(base, got);
+                                    if (base == NO_ITEM) break;
+                                }
+                                const uint32_t mi = base >> (10 + gshift);
+                                const uint32_t m = a.tile_order ? __ldg(a.tile_order + mi) : mi;
+                                const uint32_t xy = unit_first_pixel(a, m, base, gshift);
+                                if ((xy & 0xFFFFu) < (uint32_t)a.w && (xy >> 16) < (uint32_t)a.h) {
+                                    xy0 = xy;
+                                    if (a.tile_cost) { unit_tile = m; unit_t0 = clock64(); }
+                                    break;
+                                }
+                            }
+                        }
+                        xy0 = __shfl_sync(FULL, xy0, 0);
+                    }
                     if (xy0 == 0xFFFFFFFFu) break;               // warp-uniform: no work left
                     pxy = xy0 + lane_xy;
                     const uint32_t px = pxy & 0xFFFFu, py = pxy >> 16;
@@ -747,7 +786,7 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
         }
 #undef NODE_PHASE
 #undef QUEUE_UNIT
-#undef AHEAD
+#undef BATCHED
 #undef IL_UNIT
 #undef DEBUG_STACK_TRAP
 #undef POP_VALID
