@@ -78,6 +78,7 @@ HIT_OUTPUTS = ("t", "u", "v", "slot", "prim", "ng")
 CLOSEST_OUTPUTS = ("d2", "u", "v", "slot", "prim", "q", "ng")
 CLOSEST_K_OUTPUTS = CLOSEST_OUTPUTS + ("count", "total")
 CLOSEST_K_MAX = 64
+INTERSECT_K_MAX = 64
 
 
 def interval_rays(rays6, tmin=0.0, tmax=np.inf):
@@ -116,7 +117,7 @@ def point_queries(points3, rmax=np.inf):
 ABI_SYMBOLS = [
     "bihrt_version", "bihrt_create", "bihrt_destroy", "bihrt_last_error", "bihrt_set_stream", "bihrt_get_stream", "bihrt_sync",
     "bihrt_set_option", "bihrt_get_stat", "bihrt_scene_load_triangles", "bihrt_scene_update_vertices", "bihrt_scene_load_obj",
-    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_closest_point", "bihrt_closest_k", "bihrt_winding_number", "bihrt_trace_counted",
+    "bihrt_build", "bihrt_refit", "bihrt_get_build_info", "bihrt_export_reference_view", "bihrt_trace", "bihrt_trace_any", "bihrt_intersect", "bihrt_intersect_k", "bihrt_closest_point", "bihrt_closest_k", "bihrt_winding_number", "bihrt_trace_counted",
     "bihrt_render", "bihrt_render_counted", "bihrt_render_shard", "bihrt_render_samples", "bihrt_render_interleaved", "bihrt_render_interleaved_to", "bihrt_framebuffer_ipc_export", "bihrt_framebuffer_ipc_open", "bihrt_framebuffer_ipc_close", "bihrt_framebuffer_ipc_unexport", "bihrt_bih_region", "bihrt_bih_adopt", "bihrt_bih_copy", "bihrt_framebuffer_resolve", "bihrt_render_hits", "bihrt_secondary_rays", "bihrt_framebuffer", "bihrt_framebuffer_read",
     "bihrt_bih_blob_bytes", "bihrt_bih_export", "bihrt_bih_import",
     "bihrt_create_multi", "bihrt_destroy_multi", "bihrt_multi_size", "bihrt_multi_nccl_version", "bihrt_multi_broadcast",
@@ -384,6 +385,43 @@ class Renderer:
         if on_dev:
             self.wait_torch()            # rays (and recycled output blocks) were last touched on torch's current stream
         self._check(self._lib.bihrt_intersect(self._ctx, _ptr(rays8), C.c_int64(n), C.c_uint32(flags), C.byref(hits)))
+        if on_dev:
+            self.torch_wait()            # device outputs are written asynchronously on the context's stream
+        return res
+
+    def intersect_k(self, rays8, k, two_sided=False, outputs=HIT_OUTPUTS + ("count",)):
+        """Multi-hit ray queries (bihrt_intersect_k).  rays8 and acceptance as for intersect (no any_hit).  Each ray's accepted
+        triangles ordered by (t, slot), front to back; the first min(k, accepted) fill its rows, the rest read as misses.
+        0 <= k <= INTERSECT_K_MAX.  Returns {name: array} for the requested outputs of t, u, v, slot, prim (N,k), ng (N,k,3),
+        count (N,) rows written and total (N,) all accepted triangles over the interval: numpy for numpy input, torch tensors
+        on the rays' device for torch input.  "total" is left out by default: asking for it makes the walk visit every leaf
+        the interval crosses, so its cost grows with the ray's depth complexity."""
+        known = HIT_OUTPUTS + ("count", "total")
+        unknown = set(outputs) - set(known)
+        if unknown:
+            raise ValueError("unknown outputs %s (known: %s)" % (sorted(unknown), ", ".join(known)))
+        k = int(k)
+        if not 0 <= k <= INTERSECT_K_MAX:
+            raise ValueError("k must be in 0 .. %d (got %d)" % (INTERSECT_K_MAX, k))
+        shapes = {"t": (k,), "u": (k,), "v": (k,), "slot": (k,), "prim": (k,), "ng": (k, 3), "count": (), "total": ()}
+        ints = ("slot", "prim", "count", "total")
+        if isinstance(rays8, np.ndarray):
+            rays8 = np.ascontiguousarray(rays8, dtype=np.float32)
+            n = rays8.size // 8
+            res = {o: np.empty((n,) + shapes[o], np.int32 if o in ints else np.float32) for o in outputs}
+        else:
+            import torch
+            rays8 = rays8.contiguous()
+            n = rays8.numel() // 8
+            res = {o: torch.empty((n,) + shapes[o], dtype=torch.int32 if o in ints else torch.float32, device=rays8.device)
+                   for o in outputs}
+        rec = Hits(**{o: _ptr(res[o]) for o in res if o in HIT_OUTPUTS})
+        flags = INTERSECT_TWO_SIDED if two_sided else 0
+        on_dev = getattr(rays8, "is_cuda", False)
+        if on_dev:
+            self.wait_torch()            # rays (and recycled output blocks) were last touched on torch's current stream
+        self._check(self._lib.bihrt_intersect_k(self._ctx, _ptr(rays8), C.c_int64(n), C.c_int32(k), C.c_uint32(flags),
+                                                C.byref(rec), _ptr(res.get("count")), _ptr(res.get("total"))))
         if on_dev:
             self.torch_wait()            # device outputs are written asynchronously on the context's stream
         return res

@@ -623,6 +623,42 @@ int bihrt_intersect(bihrt_ctx* c, const bihrt_ray_interval* rays, int64_t n, uin
     return unstage_outputs(c, n, o);
 }
 
+// Multi-hit ray queries (include/bihrt.h): k_trace MODE 5, MODE 6 with two-sided triangles.  The record arrays have n*k
+// rows, count and total n entries; host ones are staged like every other output.
+int bihrt_intersect_k(bihrt_ctx* c, const bihrt_ray_interval* rays, int64_t n, int32_t k, uint32_t flags, const bihrt_hits* rec,
+                      int32_t* count, int32_t* total) {
+    ENTER(c);
+    if (flags & ~BIHRT_INTERSECT_TWO_SIDED) return bihrt_fail(c, BIHRT_ERR_INVALID, "unsupported flags 0x%x", flags & ~BIHRT_INTERSECT_TWO_SIDED);
+    if (!rec) return bihrt_fail(c, BIHRT_ERR_INVALID, "no output record");
+    if (k < 0 || k > BIHRT_INTERSECT_K_MAX) return bihrt_fail(c, BIHRT_ERR_INVALID, "k = %d outside 0 .. %d", k, BIHRT_INTERSECT_K_MAX);
+    if (n < 0 || (n > 0 && !rays)) return bihrt_fail(c, BIHRT_ERR_INVALID, "bad ray array");
+    if (n >= (1ll << 32) - (1ll << 24)) return bihrt_fail(c, BIHRT_ERR_INVALID, "too many rays in one call (32-bit work counter)");
+    if (!c->built) return bihrt_fail(c, BIHRT_ERR_STATE, "BIH not built");
+    { int st = check_status(c); if (st) return st; }
+    if (n == 0) return BIHRT_OK;
+    const bool rays_dev = is_device_ptr(rays);
+    if (rays_dev && ((uintptr_t)rays & 15u)) return bihrt_fail(c, BIHRT_ERR_INVALID, "device rays must be 16-byte aligned (two 128-bit loads per ray)");
+    enum { K_T, K_U, K_V, K_SLOT, K_PRIM, K_NG, K_COUNT, K_TOTAL, K_ARRAYS };
+    void* const want[K_ARRAYS] = { rec->t, rec->u, rec->v, rec->slot, rec->prim, rec->ng, count, total };
+    const size_t rows = (size_t)n * (size_t)k;
+    const size_t bytes[K_ARRAYS] = { 4 * rows, 4 * rows, 4 * rows, 4 * rows, 4 * rows, 12 * rows, 4 * (size_t)n, 4 * (size_t)n };
+    void* dev[K_ARRAYS]; void* host[K_ARRAYS]; uint8_t* front;
+    int rc = stage_arrays(c, rays_dev ? 0 : (size_t)n * sizeof(bihrt_ray_interval), K_ARRAYS, want, bytes, dev, host, &front);
+    if (rc) return rc;
+    TraceArgs a; base_args(c, a);
+    if (rays_dev) a.rays_iv = rays;
+    else {
+        BIHRT_CUDA(c, cudaMemcpyAsync(front, rays, (size_t)n * sizeof(bihrt_ray_interval), cudaMemcpyHostToDevice, c->stream));
+        a.rays_iv = (const bihrt_ray_interval*)front;
+    }
+    a.nrays = n; a.k = k;
+    a.out_t = (float*)dev[K_T]; a.out_u = (float*)dev[K_U]; a.out_v = (float*)dev[K_V];
+    a.out_slot = (int32_t*)dev[K_SLOT]; a.out_prim = (int32_t*)dev[K_PRIM]; a.out_ng = (float*)dev[K_NG];
+    a.out_count = (int32_t*)dev[K_COUNT]; a.out_total = (int32_t*)dev[K_TOTAL];
+    if ((rc = bihrt_trace_launch(c, a, (flags & BIHRT_INTERSECT_TWO_SIDED) ? 6 : 5, false))) return rc;
+    return unstage_arrays(c, K_ARRAYS, dev, host, bytes);
+}
+
 // Closest-point queries with per-point radii and full records (include/bihrt.h): k_closest, csrc/closest.cu.
 int bihrt_closest_point(bihrt_ctx* c, const bihrt_point_query* pts, int64_t n, const bihrt_closest* out) {
     ENTER(c);

@@ -206,8 +206,11 @@ struct TraceArgs {
     // camera modes, set by bihrt_trace_launch: tiles per row and 0xFFFFFFFF / tile_cols, so that a warp finds its unit's
     // tile row with a multiply-high (and one correction) instead of a divide
     uint32_t tile_cols, tile_cols_rcp;
+    // MODE 5 and 6 (bihrt_intersect_k): k rows per ray in the record arrays above (rows i*k + j, ng 3 floats per row), and
+    // count / total per ray (NULL = not wanted).  A non-NULL out_total makes the walk cut at the interval's upper end only.
+    int32_t k; int32_t* out_count; int32_t* out_total;
 };
-int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a, int mode /*0 rays,1 render fb,2 render hits,3 ray queries,4 two-sided ray queries*/, bool counted);
+int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a, int mode /*0 rays,1 render fb,2 render hits,3 ray queries,4 two-sided ray queries,5 multi-hit ray queries,6 two-sided multi-hit ray queries*/, bool counted);
 int bihrt_resolve_launch(bihrt_ctx* c, uint32_t* fb, int npix, int spp);
 int bihrt_tile_order_launch(bihrt_ctx* c, uint32_t* cost, uint32_t* order, uint32_t ntiles, bool full_sort);
 // closest.cu: bihrt_closest_point (outputs NULL = not wanted)

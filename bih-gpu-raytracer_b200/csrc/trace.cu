@@ -98,16 +98,47 @@ __device__ __forceinline__ float mt_v(float dx, float dy, float dz, float e1x, f
     return __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(dx, qx), __fmul_rn(dy, qy)), __fmul_rn(dz, qz)), inv);
 }
 
+// Multi-hit ray queries (MODE 5 and 6): the lane's sorted list of up to k keys t_bits << 32 | slot in local memory (every
+// accepted t is > 0, so the keys order exactly as (t, slot) does), the keys held and the accepted triangles met.
+struct KList { unsigned long long* keys; int cnt; uint32_t tot; };
+
+// hit record of a row of the multi-hit ray queries (MODE 5 and 6): MODE 3's epilogue, the same operations in the same order.
+// (MODE 3 keeps its inline copy: routed through this function, ptxas scheduled its ng products differently.)  The triangle
+// again (48 bytes read by the walk, likely in L1); with `rec`, u and v by the walk's arithmetic on the ray still in shared
+// memory and ng = e1 x e2 (products rounded, no FMA).
+__device__ __forceinline__ void hit_record(const BihTri* tri, const float* my_ray, bool rec, int32_t& prim, float& u, float& v,
+                                           float& gx, float& gy, float& gz) {
+    const float4* tq = reinterpret_cast<const float4*>(tri);
+    const float4 q0 = __ldg(tq), q1 = __ldg(tq + 1), q2 = __ldg(tq + 2);
+    prim = (int32_t)__float_as_uint(q2.y);
+    if (rec) {
+        const float e1x = q0.w, e1y = q1.x, e1z = q1.y, e2x = q1.z, e2y = q1.w, e2z = q2.x;
+        const float2 dxy = *reinterpret_cast<const float2*>(my_ray + 6);
+        const float dx = dxy.x, dy = dxy.y, dz = my_ray[8];
+        float px, py, pz, tx, ty, tz, qx, qy, qz;
+        const float inv = __frcp_rn(mt_det(dx, dy, dz, e1x, e1y, e1z, e2x, e2y, e2z, px, py, pz));
+        u = mt_u(my_ray[0], my_ray[2], my_ray[4], q0, px, py, pz, inv, tx, ty, tz);
+        v = mt_v(dx, dy, dz, e1x, e1y, e1z, tx, ty, tz, inv, qx, qy, qz);
+        gx = __fsub_rn(__fmul_rn(e1y, e2z), __fmul_rn(e1z, e2y));
+        gy = __fsub_rn(__fmul_rn(e1z, e2x), __fmul_rn(e1x, e2z));
+        gz = __fsub_rn(__fmul_rn(e1x, e2y), __fmul_rn(e1y, e2x));
+    }
+}
+
 // FIRST: stop at the first accepted triangle (coverage queries)
 // RANGE: ray queries with an interval (MODE 3): a triangle is accepted for tlo < t < h.t, with tlo = max(tmin, 0) read from
 // word 9 of the lane's shared-memory ray record (only when a candidate is found: no register is held through the leaf)
 // TWO_SIDED: back faces too (MODE 4): Moller-Trumbore's non-culling branch, |det| >= 1e-6.  Everything after the det test is
 // the same arithmetic (1/det rounds symmetrically), so a front-face candidate is computed bit for bit as without it; a NaN
 // det still passes here and is rejected by the t compare.
-template <bool COUNTED, bool FIRST, bool RANGE = false, bool TWO_SIDED = false>
+// MULTI: the list variant (MODE 5 and 6, with RANGE).  h.t is the cut: the interval's upper end until k keys are held (and
+// always when `prune` is false: the caller counts every accepted triangle), then the k-th key's t.  Below the upper end a
+// triangle is accepted (tot counts it); at exactly the k-th t it still enters when its key is below the k-th one, so the
+// cut is closed for ties, as the node tests are (pMin <= min(pMax, h.t)).
+template <bool COUNTED, bool FIRST, bool RANGE = false, bool TWO_SIDED = false, bool MULTI = false>
 __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, float ox, float oy, float oz,
                                           float dx, float dy, float dz, Hit& h, uint32_t& ntris, uint32_t& wleaf,
-                                          const float* tlo_p = nullptr) {
+                                          const float* tlo_p = nullptr, KList* kl = nullptr, int k = 0, bool prune = false) {
     const float4* p = reinterpret_cast<const float4*>(first_tri);
     for (;;) {
         const float4 q0 = __ldg(p), q1 = __ldg(p + 1), q2 = __ldg(p + 2);
@@ -124,7 +155,24 @@ __device__ __forceinline__ void test_leaf(const char* __restrict__ first_tri, fl
                 const float v = mt_v(dx, dy, dz, e1x, e1y, e1z, tx, ty, tz, inv, qx, qy, qz);
                 if (!(v < 0.f || __fadd_rn(u, v) > 1.f)) {
                     const float t = __fmul_rn(__fadd_rn(__fadd_rn(__fmul_rn(e2x, qx), __fmul_rn(e2y, qy)), __fmul_rn(e2z, qz)), inv);
-                    if (t > (RANGE ? *tlo_p : 0.f) && t < h.t) {                              // :218-221, slot = sorted index
+                    if constexpr (MULTI) {
+                        const bool full = prune && kl->cnt == k;       // h.t is the k-th t, not the upper end
+                        if (t > *tlo_p && (t < h.t || (full && t == h.t))) {
+                            kl->tot++;
+                            const unsigned long long key = (unsigned long long)__float_as_uint(t) << 32 | __float_as_uint(q2.w);
+                            if (k > 0 && (kl->cnt < k || key < kl->keys[k - 1])) {
+                                // insertion from the free place (the last one when full: the k-th key drops out)
+                                int j = kl->cnt < k ? kl->cnt++ : k - 1;
+                                for (; j > 0; j--) {
+                                    const unsigned long long e = kl->keys[j - 1];
+                                    if (e < key) break;
+                                    kl->keys[j] = e;
+                                }
+                                kl->keys[j] = key;
+                                if (prune && kl->cnt == k) h.t = __uint_as_float((uint32_t)(kl->keys[k - 1] >> 32));
+                            }
+                        }
+                    } else if (t > (RANGE ? *tlo_p : 0.f) && t < h.t) {                       // :218-221, slot = sorted index
                         h.t = t; h.slot = (int)__float_as_uint(q2.w);
                         if (FIRST) break;
                     }
@@ -166,8 +214,10 @@ __device__ __forceinline__ uint32_t unit_first_pixel(const TraceArgs& a, uint32_
 // ------------------------------------------------------------------------------------------
 // MODE 0: ray list -> (t, slot, prim);  1: camera -> packed framebuffer;  2: camera -> per-sample hits;
 // 3: ray list with per-ray intervals [tmin, tmax] -> hit records (t, u, v, slot, prim, ng): bihrt_intersect;
-// 4: MODE 3 with two-sided triangles (BIHRT_INTERSECT_TWO_SIDED): only the leaf's det test differs.
-// Work item = one ray (MODE 0/3/4) or one pixel with its spp samples (MODE 1/2).
+// 4: MODE 3 with two-sided triangles (BIHRT_INTERSECT_TWO_SIDED): only the leaf's det test differs;
+// 5, 6: multi-hit ray queries (bihrt_intersect_k), one- and two-sided: MODE 3 / 4 with test_leaf's list variant in place of
+// the closest hit and h.t as the list's cut; the epilogue writes k rows, the count and the total.
+// Work item = one ray (MODE 0/3/4/5/6) or one pixel with its spp samples (MODE 1/2).
 // MODE 3 walks exactly like MODE 0 with a narrower root interval: pMin = max(rMin, tlo) and pMax = min(sMax, h.t), where
 // h.t starts at min(tmax, FLT_MAX) (so the item in hand is valid, as for the occlusion query) and tlo = max(tmin, 0) sits in
 // word 9 of the ray record, where the triangle test reads it.  u, v and ng are not carried through the walk (the kernel is
@@ -182,9 +232,10 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
     constexpr int STACK_DEPTH = Q ? STACK_DEPTH_QUALITY : STACK_DEPTH_PARITY;
     constexpr bool COVER = MODE == 1;                                  // a sample ends at its first hit
     constexpr bool OCTS = MODE == 1;                                   // node phase specialised on the warp's ray octant
-    constexpr bool LIST = MODE == 0 || MODE == 3 || MODE == 4;         // work items are rays of a list
-    constexpr bool RANGE = MODE == 3 || MODE == 4;                     // rays carry [tmin, tmax]; hit records out
-    constexpr bool TWO_SIDED = MODE == 4;                              // back faces accepted too
+    constexpr bool MULTI = MODE == 5 || MODE == 6;                     // the k nearest hits of the interval
+    constexpr bool LIST = MODE == 0 || MODE == 3 || MODE == 4 || MULTI;   // work items are rays of a list
+    constexpr bool RANGE = MODE == 3 || MODE == 4 || MULTI;            // rays carry [tmin, tmax]; hit records out
+    constexpr bool TWO_SIDED = MODE == 4 || MODE == 6;                 // back faces accepted too
     // per-axis ray constants (origin, 1/dir), one row of 3 float2 per thread: 24-byte stride keeps a
     // half-warp's 64-bit accesses on distinct banks when the lanes agree on the axis
     // per-thread ray record in shared memory, 10 words: (ox, 1/dx) (oy, 1/dy) (oz, 1/dz) dx dy dz, and word 9: tlo (MODE 3 and 4) or
@@ -280,6 +331,8 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
     uint32_t cur = NONE;                       // item being walked: node index, leaf|slot, or NONE
     float rMin = 0.f, pMin = 0.f, pMax = 0.f;
     Hit h; h.t = FLT_MAX; h.slot = -1;
+    unsigned long long klist[MULTI ? BIHRT_INTERSECT_K_MAX : 1];
+    KList kl = { klist, 0, 0u };               // MULTI: the ray's list (h.t is its cut)
     bool tracing = false;                      // a ray is in flight (its result has not been recorded)
     uint4 stack[STACK_DEPTH];
     int sp = 0;
@@ -328,7 +381,29 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                 if (cur == NONE) {
                     if (tracing) {                               // record the ray that just ended
                         tracing = false;
-                        if (RANGE) {
+                        if (MULTI) {
+                            const bool rec = a.out_u || a.out_v || a.out_ng;
+                            // the rows: each kept triangle's record as MODE 3 computes it, the miss record after them
+                            for (int j = 0; j < a.k; j++) {
+                                float t = FLT_MAX, u = 0.f, v = 0.f, gx = 0.f, gy = 0.f, gz = 0.f;
+                                int32_t slot = -1, prim = -1;
+                                if (j < kl.cnt) {
+                                    const unsigned long long key = klist[j];
+                                    t = __uint_as_float((uint32_t)(key >> 32));
+                                    slot = (int32_t)(uint32_t)key;
+                                    if (rec || a.out_prim) hit_record(tris + slot, my_ray, rec, prim, u, v, gx, gy, gz);
+                                }
+                                const uint64_t row = item * (uint64_t)a.k + (uint64_t)j;
+                                if (a.out_t) a.out_t[row] = t;
+                                if (a.out_slot) a.out_slot[row] = slot;
+                                if (a.out_prim) a.out_prim[row] = prim;
+                                if (a.out_u) a.out_u[row] = u;
+                                if (a.out_v) a.out_v[row] = v;
+                                if (a.out_ng) { float* g = a.out_ng + 3 * row; g[0] = gx; g[1] = gy; g[2] = gz; }
+                            }
+                            if (a.out_count) a.out_count[item] = kl.cnt;
+                            if (a.out_total) a.out_total[item] = (int32_t)kl.tot;
+                        } else if (RANGE) {
                             // hit record epilogue: the hit triangle again (48 bytes just read by the walk, likely in L1), u and v
                             // by the walk's arithmetic on the ray still in shared memory, ng = e1 x e2 (products rounded, no FMA)
                             const bool hit = h.slot >= 0;
@@ -542,6 +617,10 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
                     tlo = fmaxf(r0.w, 0.f);
                     live = r0.w == r0.w && tlo < r1.w;
                     thi = fminf(r1.w, FLT_MAX);
+                    if (MULTI) {                          // k == 0 without the total asks for nothing: no walk
+                        live = live && (a.k > 0 || a.out_total);
+                        kl.cnt = 0; kl.tot = 0;
+                    }
                 } else if (MODE == 0) {
                     const float* p = reinterpret_cast<const float*>(a.rays + item);
                     ox = __ldg(p); oy = __ldg(p + 1); oz = __ldg(p + 2); dx = __ldg(p + 3); dy = __ldg(p + 4); dz = __ldg(p + 5);
@@ -779,7 +858,8 @@ __global__ void __launch_bounds__(TRACE_THREADS, TRACE_MIN_BLOCKS) k_trace(Trace
             const char* tp;
             asm("mad.wide.u32 %0, %1, 12, %2;" : "=l"(tp) : "r"(cur & 0x7FFFFFFCu), "l"(tris_b));
             const float2 dxy = *reinterpret_cast<const float2*>(my_ray + 6);
-            test_leaf<COUNTED, COVER, RANGE, TWO_SIDED>(tp, my_ray[0], my_ray[2], my_ray[4], dxy.x, dxy.y, my_ray[8], h, ntris, wleaf, my_ray + 9);
+            test_leaf<COUNTED, COVER, RANGE, TWO_SIDED, MULTI>(tp, my_ray[0], my_ray[2], my_ray[4], dxy.x, dxy.y, my_ray[8], h, ntris,
+                                                               wleaf, my_ray + 9, &kl, a.k, a.out_total == nullptr);
             // occluded / covered: nothing else to learn
             if (((LIST && a.any_hit) || COVER) && h.slot >= 0) { STACK_RESET(); cur = NONE; }
             else POP_VALID();
@@ -940,6 +1020,8 @@ static int launch_mode(bihrt_ctx* c, const TraceArgs& a, int mode, bool counted)
         case 5: return launch<2, true, Q>(c, a);
         case 6: return launch<3, false, Q>(c, a);
         case 8: return launch<4, false, Q>(c, a);
+        case 10: return launch<5, false, Q>(c, a);
+        case 12: return launch<6, false, Q>(c, a);
         default: return bihrt_fail(c, BIHRT_ERR_INVALID, "bad trace mode %d", mode);
     }
 }
@@ -948,7 +1030,7 @@ int bihrt_trace_launch(bihrt_ctx* c, const TraceArgs& a_in, int mode, bool count
     TraceArgs a = a_in;
     // per-SM queues pay off once a launch is long enough to amortise the end-of-kernel stealing
     // (measured: +7 % at 133 M rays, -9 % at 2 M rays on the 1 M-triangle scene)
-    const bool list = mode == 0 || mode == 3 || mode == 4;     // ray lists (3, 4: with intervals and hit records)
+    const bool list = mode == 0 || mode >= 3;     // ray lists (3, 4: with intervals and hit records; 5, 6: with k of them)
     const int64_t rays = list ? a.nrays : (int64_t)a.w * a.h * (a.s_end - a.s_begin) / (a.shard_count > 0 ? a.shard_count : 1) / (a.il_count > 0 ? a.il_count : 1);
     // ... and only when a warp spans many pixels: with a pixel's samples in consecutive lanes a warp is coherent on
     // its own and the queues only add stealing overhead (-5 % at 4K x 16 spp)

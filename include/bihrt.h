@@ -220,6 +220,46 @@ typedef struct bihrt_hits {
 #define BIHRT_INTERSECT_ANY 1u   /* occlusion: end at the first accepted triangle of the interval */
 #define BIHRT_INTERSECT_TWO_SIDED 4u   /* back faces count too (|det| >= 1e-6); flag values 0, 1, 4 and 5 are valid */
 BIHRT_API int bihrt_intersect(bihrt_ctx* ctx, const bihrt_ray_interval* rays, int64_t n, uint32_t flags, const bihrt_hits* out);
+/* ---- multi-hit ray queries: the k nearest accepted triangles of each ray's interval, front to back, and the number of all
+ *      of them (the ray's crossing count).
+ *      Acceptance is bihrt_intersect's: max(tmin, 0) < t < min(tmax, FLT_MAX), both strict, and the det test of the flags;
+ *      a ray with !(max(tmin, 0) < tmax), NaN bounds included, has no candidates and is not walked.
+ *      flags 0: one-sided; BIHRT_INTERSECT_TWO_SIDED: back faces count too.  BIHRT_INTERSECT_ANY and every other bit:
+ *        BIHRT_ERR_INVALID.
+ *      The walk is bihrt_intersect's (scene-box entry; on parity trees the strict plane test, the children boxes with their
+ *      margin and the far-leaf-first order, hence the same misses on axis-aligned flat geometry; on quality trees the closed
+ *      tests).  Only the cut differs: once k triangles are held it is the t of the k-th of them, before that -- and always when
+ *      total is asked for -- the interval's upper end.  The cut is CLOSED for ties: a node whose interval starts exactly at the
+ *      k-th t is still visited, and a triangle at exactly that t with a smaller slot still enters.
+ *      Result for ray i: the accepted triangles the walk reaches, ordered by (t, slot) ascending, ties to the smaller slot (the
+ *      key t_bits << 32 | slot orders them exactly: every accepted t is > 0).  The first min(k, that many) go to rows i*k + 0,
+ *      1, ... of the arrays of rec, each row a full bihrt_hits record (t, u, v, slot, prim, ng) computed after the walk from
+ *      its slot with the walk's own arithmetic, so t, u, v are bit for bit what bihrt_intersect reports for that triangle.
+ *      The rows after them hold the miss record (t = FLT_MAX, slot = prim = -1, u = v = 0, ng = 0).  count[i] is the number of
+ *      rows written; total[i] the number of ALL accepted triangles the walk reaches over the whole interval (with
+ *      BIHRT_INTERSECT_TWO_SIDED on a closed mesh its parity is an inside test).  Consequences:
+ *        - k == 1: t, u, v and ng of the row are bihrt_intersect's record; slot and prim may differ only between triangles
+ *          at exactly the same t, where this call takes the smaller slot;
+ *        - quality-mode trees: the rows equal brute force over the interval, except the classes bihrt_intersect documents
+ *          (DESIGN.md section 2, and the two-sided coplanar-leaves note above);
+ *        - the rows at k are the first k rows at any larger k;
+ *        - where total <= k, the distinct t of the rows are exactly the sequence the peeling loop (bihrt_intersect again with
+ *          tmin = the last t) visits -- and unlike peeling the rows keep triangles that share a t.  With
+ *          BIHRT_INTERSECT_TWO_SIDED this holds up to the coplanar-leaves class above, on both tree kinds: where coincident
+ *          faces of different leaves are hit at t an ulp apart, a peeling step (a closest-hit walk from a raised tmin) may
+ *          skip one of them that the rows hold (DESIGN.md section 11);
+ *        - refit trees: as the other ray queries, see bihrt_refit.
+ *      Cost: without total the walk prunes at the k-th t, like bihrt_intersect at k = 1.  With total it visits every leaf the
+ *      interval crosses, so the cost grows with the ray's depth complexity.
+ *      k: 0 .. BIHRT_INTERSECT_K_MAX.  k == 0 writes no rows: with total the call is a pure crossing count, without it the call
+ *      only fills count with 0.
+ *      rec: arrays of n*k entries (ng: 3*n*k floats), any of them NULL; count, total: n entries, either NULL.  Each one host or
+ *      device.  rays, staging, synchronisation, watchdog and replica behaviour as bihrt_intersect.
+ *      Errors: those of bihrt_intersect, and BIHRT_ERR_INVALID for k < 0, k > BIHRT_INTERSECT_K_MAX, rec == NULL or
+ *      BIHRT_INTERSECT_ANY; BIHRT_ERR_NOMEM when the staging buffer of host outputs cannot be allocated. ------------------ */
+#define BIHRT_INTERSECT_K_MAX 64
+BIHRT_API int bihrt_intersect_k(bihrt_ctx* ctx, const bihrt_ray_interval* rays, int64_t n, int32_t k, uint32_t flags,
+                                const bihrt_hits* rec, int32_t* count, int32_t* total);
 /* ---- closest-point queries: the triangle nearest to a point within the point's own search radius, full records.
  *      Distance of point p to a triangle: one IEEE binary32 function, every product, sum and quotient rounded, no FMA,
  *      computed from the triangle record's v0, e1 = v1 - v0, e2 = v2 - v0 (fl(v1 - v0), fl(v2 - v0), as bihrt_intersect
